@@ -2,11 +2,13 @@
 """GP-blur fwd+bwd throughput (windows/s) on B200 - the metric of BASELINE.json.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                  [--sweep] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic forecast windows per GPU:
 whitened-SVGP predictive (mean, variance, fused Philox sample) of every GP call of the workload, the
 ELBO on the decoder-side call, and the full hand-written backward (dX + every GP parameter gradient);
-for N > 1 the flat GP-gradient bucket is all-reduced over NCCL inside the step.
+for N > 1 the flat GP-gradient bucket is all-reduced over NCCL inside the step.  The inputs and
+parameters are seeded, so runs with the same arguments see the same inputs.
 
 Workloads (BASELINE.json `configs`; per-GPU batch is fixed => weak scaling):
   c2      configs[1]: the two GP-blur calls of the traffic-shape train step, enc [256,192,64] and
@@ -17,11 +19,27 @@ Workloads (BASELINE.json `configs`; per-GPU batch is fixed => weak scaling):
   c4      configs[3]: two-layer DeepGP, B=2048, L=24, D=64, M=256, hidden width H=10
   c5_mM   configs[4]: B=8192, L=24, D=64, M in {64,128,256,512,1024}
 
-The JSON line carries `value` (inputs resident in HBM), `e2e` (host buffers, H2D/D2H inside the timed
-region, through the public module API), `roofline` of the dominant kernel (per-stage CUDA-event times
-measured live by the library's profile hooks) and `cpu_baseline` (the oracle's reference-order
-restatement of the gpytorch path on the host cores: gpytorch itself is not installable here).
-`--impl reference` times that CPU path alone.
+The run prints ONE JSON result line for --workload on stdout, and the breakdown (roofline,
+roofline_per_point_kernel, stage_ms_per_step and what --sweep adds) as one JSON line on stderr.
+  value     K = --steps timed steps on inputs resident in HBM: per-step CUDA events (max over ranks),
+            a 256 MiB L2 flush (write) and 3 rotating input sets between timed steps.
+  e2e       the same steps through the public module API from pinned host buffers: step i + 1's
+            inputs travel on a copy stream while step i computes; the per-window ELBO goes back into
+            pinned memory and the host reads EVERY step's result one step behind the launches, the
+            last one before the clock stops.
+  cpu_baseline  the oracle's reference-order restatement of the gpytorch path on the host cores
+            (gpytorch itself when it can be imported).  `--impl reference` times that CPU path alone.
+  roofline  the dominant kernel, and roofline_per_point_kernel the dominant per-point kernel
+            (per-stage CUDA-event times from the library's profile hooks).  "achieved" counts
+            ALGORITHMIC bytes or flops; the tensor peak is the TF32 dense rate, 1/2 of the bf16 peak
+            (a 3xTF32 kernel issues 3 MMAs per product, so its ceiling is frac = 1/3; M <= 32 runs
+            FP32 FFMA, ~74 TFLOP/s).  The once-per-update M x M stages (mm_fwd / mm_bwd / sg_reduce)
+            are latency-bound fp64 work with no per-window traffic.  "traffic" is the measured DRAM
+            bytes per launch recorded in profiles/ncu_traffic.json for that workload and kernel.
+--sweep adds `workloads` (the other BASELINE.json configurations, measured the same way in the same
+process) and `next_rows` (the kernels on either side of the GP blur, each beside the torch-eager
+sequence it replaces).
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed (dump_outputs).
 """
 from __future__ import annotations
 
@@ -36,6 +54,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark writes nothing into the tree it runs from
 
 import torch  # noqa: E402
 
@@ -57,6 +76,9 @@ DEFAULT_WORKLOAD = "c2"
 METRIC = "gp_blur_fwd_bwd_windows_per_sec"
 UNIT = "windows/s"
 L2_FLUSH_BYTES = 256 << 20
+DUMP_LIMIT_BYTES = 64 << 20
+# printed on stderr: the result line on stdout stays short enough to be read back from the end of the output
+DETAIL_KEYS = ("roofline", "roofline_per_point_kernel", "stage_ms_per_step", "workloads", "next_rows")
 
 
 def load_peaks():
@@ -215,9 +237,9 @@ def cpu_reference_step_fn_two_layer(wl, B_cpu, seed=1234):
 
 
 def gpytorch_step_fn(wl, B_cpu, seed=1234):
-    """The reference's OWN classes on real gpytorch (BASELINE.md section 2) - only when gpytorch can be imported (it is
-    not in this image's wheelhouse) and the reference tree is reachable (baseline/_ref or /root/reference)."""
-    for extra in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    """The reference's OWN classes on real gpytorch (BASELINE.md section 2) - only when gpytorch can be imported and
+    the reference tree is installed under baseline/_ref."""
+    for extra in (os.path.join(ROOT, "baseline", "_ref"),):
         if os.path.isdir(extra) and extra not in sys.path:
             sys.path.append(extra)
     import gpytorch                                    # noqa: F401  (ImportError -> caller falls back to the port)
@@ -331,6 +353,25 @@ def exercise_init(layer, seed):
         vs.variational_params_initialized.fill_(1)
 
 
+def dump_outputs(dirname, outputs, model):
+    """Writes what one step hands its caller as DIR/<name>.npy (float32): the per-call mean / sample and dX
+    (mean_<c>, sample_<c>, dx_<c>, c = index of the GP call), the per-window ELBO and every parameter gradient
+    (grad_<parameter name>).  When together they exceed DUMP_LIMIT_BYTES, every array larger than an equal share
+    of the limit is replaced by the same seeded sample of its flattened elements (sorted indices) in every run."""
+    import numpy as np
+    arrays = dict(outputs)
+    arrays.update({"grad_" + n: p.grad for n, p in model.named_parameters() if p.grad is not None})
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES and a.nbytes > share:
+            keep = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def make_model(wl, device, seed=1234):
     from fine_grained_gaussian_process_forcasting_b200.DeepGP import DeepGPp, DeepGP2
     from fine_grained_gaussian_process_forcasting_b200 import gpcompat
@@ -346,8 +387,8 @@ def make_model(wl, device, seed=1234):
 
 
 def run_ours(args, wl, name):
-    """The driver's line: the default workload in full, plus (unless --single) a `workloads` dict with the other
-    BASELINE.json configurations measured the same way in the same process (c3 strong-scaled: B = 1024 global)."""
+    """The result line: --workload in full, plus (with --sweep) a `workloads` dict with the other BASELINE.json
+    configurations measured the same way in the same process (c3 strong-scaled: B = 1024 global) and `next_rows`."""
     from fine_grained_gaussian_process_forcasting_b200 import _cabi
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -364,7 +405,7 @@ def run_ours(args, wl, name):
     _cabi.lib()
     ctx = dict(world=world, rank=rank, local_rank=local_rank, device=device, dist=dist)
     line = measure(args, wl, name, ctx, primary=True)
-    if not args.single:
+    if args.sweep:
         extra = {}
         for other in EXTRA_WORKLOADS:
             if other == name:
@@ -382,6 +423,8 @@ def run_ours(args, wl, name):
             except Exception as e:      # the headline line must survive a failure of the side measurements
                 line["next_rows"] = {"error": repr(e)}
     if rank == 0:
+        detail = {k: line.pop(k) for k in DETAIL_KEYS if k in line}
+        print(json.dumps(detail), file=sys.stderr, flush=True)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
@@ -430,10 +473,11 @@ def measure(args, wl, name, ctx, primary=True):
     call_streams = CallStreams(device, len(calls)) if (args.call_streams and len(calls) > 1 and not fused) else None
 
     def step_body(xin, yin):
-        """forward (mean, variance, fused sample, ELBO) + backward (dX, every GP parameter gradient)"""
+        """forward (mean, variance, fused sample, ELBO) + backward (dX, every GP parameter gradient); returns what
+        the caller receives besides the parameter gradients, by name (dump_outputs), the ELBO under "elbo"."""
         bucket.zero()
         outs, grads = [], []
-        elbo = None
+        res = {}
         if fused:
             # ONE fused evaluation for all the activations of the step (one launch per kernel, one leaf for dX)
             from fine_grained_gaussian_process_forcasting_b200 import ops as _ops
@@ -442,26 +486,31 @@ def measure(args, wl, name, ctx, primary=True):
             for c, o in enumerate(segs):
                 outs += [o.mean, o.sample]
                 grads += [gms[c], gss[c]]
-            elbo = segs[-1].elbo
-            outs.append(elbo)
+                res[f"mean_{c}"], res[f"sample_{c}"] = o.mean, o.sample
+            res["elbo"] = segs[-1].elbo
+            outs.append(res["elbo"])
             grads.append(g_elbo)
             torch.autograd.backward(outs, grads)
             if world > 1 and allreduce_in_step[0]:
                 bucket.all_reduce(average=True)
-            return elbo
+            res.update((f"dx_{c}", g_) for c, g_ in enumerate(seg_views(xf.grad)))
+            return res
         if call_streams is not None:
             for ly in layers:                             # the shared stage is built once, on the main stream
                 ly._kl_only()
+        leaves = []
         for c, L in enumerate(calls):
             x = xin[c].detach().requires_grad_(True)      # fresh leaf: dX flows back to the forecaster
+            leaves.append(x)
             last = c == len(calls) - 1
             fn = (lambda x=x, last=last: model.blur(x, yin if last else None, num_data=D))
             out = call_streams.run(c, fn) if call_streams is not None else fn()
             outs += [out.mean, out.sample]
             grads += [gms[c], gss[c]]
+            res[f"mean_{c}"], res[f"sample_{c}"] = out.mean, out.sample
             if last:
-                elbo = out.elbo
-                outs.append(elbo)
+                res["elbo"] = out.elbo
+                outs.append(out.elbo)
                 grads.append(g_elbo)
         if call_streams is not None:
             call_streams.join()
@@ -470,7 +519,8 @@ def measure(args, wl, name, ctx, primary=True):
             call_streams.join()
         if world > 1 and allreduce_in_step[0]:
             bucket.all_reduce(average=True)               # NCCL AVG on the flat bucket: part of the captured step
-        return elbo
+        res.update((f"dx_{c}", x.grad) for c, x in enumerate(leaves))
+        return res
 
     allreduce_in_step = [not args.allreduce_after_replay]
 
@@ -532,14 +582,14 @@ def measure(args, wl, name, ctx, primary=True):
     def run_step(i, xin, yin):
         """one step on inputs already in HBM; returns the per-window ELBO"""
         if graphed is None:
-            return eager_step(i, xin, yin)
+            return eager_step(i, xin, yin)["elbo"]
         for dst, src in zip(g_inputs, list(xin) + [yin]):
             if dst.data_ptr() != src.data_ptr():
                 dst.copy_(src, non_blocking=True)
-        (elbo,) = graphed.replay()
+        (res,) = graphed.replay()
         if world > 1 and not allreduce_in_step[0]:
             bucket.all_reduce(average=True)
-        return elbo
+        return res["elbo"]
 
     for i in range(3):
         run_step(i, xs[i % nbuf], ys[i % nbuf])
@@ -559,11 +609,11 @@ def measure(args, wl, name, ctx, primary=True):
         flush.zero_()                                   # L2 flush between timed iterations (outside the events)
         evs[i][0].record()
         if graphed is not None:
-            graphed.replay()
+            (last,) = graphed.replay()
             if world > 1 and not allreduce_in_step[0]:
                 bucket.all_reduce(average=True)
         else:
-            eager_step(i, xs[i % nbuf], ys[i % nbuf])
+            last = eager_step(i, xs[i % nbuf], ys[i % nbuf])
         evs[i][1].record()
     sync_all()
     t_wall = time.perf_counter() - t_wall0
@@ -576,6 +626,8 @@ def measure(args, wl, name, ctx, primary=True):
     ms_total = float(t.item())
     ms_per_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and primary and rank == 0:     # before anything below runs the step again
+        dump_outputs(args.dump_outputs, last, model)
 
     # ---- timed region 2: end to end through the module API with host buffers ----
     if graphed is not None:
@@ -747,20 +799,13 @@ def measure(args, wl, name, ctx, primary=True):
               if by > 0 and intensity < tf32_peak * 1e12 / (peaks["hbm_gbs"] * 1e9):
                   roof = {"bound": "hbm", "achieved": by / per_launch_s / 1e9, "peak": peaks["hbm_gbs"], "unit": "GB/s"}
               else:
-                  roof = {"bound": "tensor", "achieved": fl / per_launch_s / 1e12, "peak": tf32_peak, "unit": "TFLOP/s",
-                          "peak_note": "TF32 dense rate = 1/2 of the measured cuBLAS bf16 burst peak; 'achieved' counts "
-                                       "ALGORITHMIC flops (a 3xTF32 kernel issues 3 MMAs per product, so its "
-                                       "ceiling is frac = 1/3; M <= 32 runs FP32 FFMA, peak ~74 TFLOP/s)"}
+                  roof = {"bound": "tensor", "achieved": fl / per_launch_s / 1e12, "peak": tf32_peak, "unit": "TFLOP/s"}
               roof["frac"] = roof["achieved"] / roof["peak"]
               if roof["bound"] == "tensor" and M > 32 and dom in point_stages:
                   roof["frac_of_3xtf32_ceiling"] = 3.0 * roof["frac"]
               if M <= 32 and dom in point_stages:     # FP32-FFMA path: CUDA-core bound long before HBM
                   roof["ffma_tflops_achieved"] = fl / per_launch_s / 1e12
                   roof["ffma_frac_of_74_tflops"] = roof["ffma_tflops_achieved"] / 74.0
-              if dom in ("mm_fwd", "mm_bwd", "sg_reduce"):
-                  roof["note"] = ("once-per-parameter-update M x M stage (fp64 Cholesky / inverse / Cholesky backward on "
-                                  "CUDA cores): serial panel factorisations + grid barriers, latency-bound; no "
-                                  "per-window traffic - see roofline_per_point_kernel for the throughput kernels")
               # measured DRAM traffic of that kernel (ncu --set full capture of this same command, per launch)
               roof["traffic"] = None
               try:
@@ -768,7 +813,6 @@ def measure(args, wl, name, ctx, primary=True):
                   ent = tj.get(name, {}).get(dom)
                   if ent:
                       roof["traffic"] = ent["bytes_per_launch"]
-                      roof["traffic_source"] = "profiles/ncu_traffic.json (dram__bytes_read+write per launch, ncu --set full)"
               except Exception:
                   pass
               roof["algorithmic_bytes_per_launch"] = by
@@ -785,20 +829,15 @@ def measure(args, wl, name, ctx, primary=True):
             "warmup": max(3, args.warmup), "ms_per_step": ms_per_step, "higher_is_better": True,
             "scaling": "strong" if wl.get("strong") else "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-            "config": {"workload": name, "desc": wl["desc"], "B_per_gpu": B, "B_global": B * world, "L": calls, "D": D, "M": M,
-                       "parallelism": f"dp{world}", "l2": f"flush ({L2_FLUSH_BYTES >> 20} MiB write) between timed steps "
-                       "+ 3 rotating input sets", "timing": "per-step CUDA events, max over ranks",
+            "config": {"workload": name, "B_per_gpu": B, "B_global": B * world, "L": calls, "D": D, "M": M,
+                       "parallelism": f"dp{world}",
                        "launch": graph_note,
                        "call_streams": call_streams is not None,
                        "calls_fused": fused,
                        "allreduce": (None if world == 1 else "one-shot kernel over NVLink peer memory (CUDA IPC), rank-ordered sum"
                                      if peer_allreduce else "NCCL all-reduce (AVG)"),
                        "regime": "R-exercise (SURVEY 8d)"},
-            "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "pipeline": "pinned host inputs -> copy stream (step i + 1 in flight during step i) -> device "
-                                "hand-over -> step -> D2H of the per-window ELBO into pinned memory; the host waits "
-                                "for and reads EVERY step's result, one step behind the launches (step i - 1 while "
-                                "step i runs, double-buffered), the last one before the clock stops"},
+            "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
             "gpu_launches": int(launches),
             "clocks": clocks,
             "roofline": roofs.get("roofline"),
@@ -1003,10 +1042,15 @@ def main():
                     help="evaluate the GP once per activation (blur) instead of once per step (blur_segments)")
     ap.add_argument("--eager", action="store_true", help="launch every kernel from Python instead of replaying the "
                     "step as a CUDA graph")
-    ap.add_argument("--single", action="store_true", help="measure only --workload (no `workloads` dict)")
+    ap.add_argument("--sweep", action="store_true", help="also measure the other BASELINE.json workloads (`workloads`) "
+                    "and the kernels on either side of the GP blur (`next_rows`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step "
+                    "computed as DIR/<name>.npy (float32, at most 64 MiB in all)")
     ap.add_argument("--check", action="store_true", help="N > 1: verify the all-reduced gradient bucket against a "
                     "single-rank run on the concatenated batch (adds `allreduce_check` to the line)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl, args.workload)

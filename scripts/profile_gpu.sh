@@ -3,7 +3,7 @@
 #   scripts/profile_gpu.sh <workload> <kernel-regex> [tag] [skip] [count]
 set -u
 W=${1:-c2}; K=${2:-tc2_|tc_reduce|mm_|stage_grad}; TAG=${3:-$W}; SKIP=${4:-8}; CNT=${5:-4}
-CMD="python bench.py --single --workload $W --steps 3 --warmup 3 --no-cpu-baseline"
+CMD="python bench.py --workload $W --steps 3 --warmup 3 --no-cpu-baseline"
 mkdir -p gpurun_out
 $CMD > gpurun_out/plain_$TAG.log 2>&1 || { echo "plain run failed"; tail -5 gpurun_out/plain_$TAG.log; exit 1; }
 tail -c 600 gpurun_out/plain_$TAG.log; echo

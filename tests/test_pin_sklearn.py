@@ -1,4 +1,4 @@
-"""An EXTERNAL anchor for the GP oracle (gpytorch itself is not installable here, tests/test_pin_gpytorch.py skips):
+"""An EXTERNAL anchor for the GP oracle (the suite does not run gpytorch itself):
 scikit-learn's exact GP regression, an independent implementation of the same kernel algebra.
 
 * Whitened SVGP predictive.  With the inducing points as "training inputs", whitened variational mean m = L^-1 y_z and
