@@ -676,6 +676,7 @@ int gpblur_debug_fetch(int which, long long N, int D, int M, const void* ws, voi
     case 3: off = L.A; bytes = (size_t)(L.MP >= 128 ? round_up_ll(N, 128) : N) * L.MP * 4; break;   // tile-major if MP >= 128
     case 4: off = L.stamps; bytes = kStampSlots * 8; break;
     case 5: off = L.W; bytes = (size_t)(L.MP >= 128 ? round_up_ll(N, 128) : N) * L.MP * 4; break;   // W = kbar o k (after a backward)
+    case 6: off = L.gsc; bytes = (size_t)2 * (N > 0 ? N : 1) * 4; break;   // folded g_mu, g_var (after a backward)
     default: return GPBLUR_EINVAL;
   }
   if (out_bytes < bytes) return GPBLUR_EWORKSPACE;

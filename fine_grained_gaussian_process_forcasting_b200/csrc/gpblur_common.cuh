@@ -47,7 +47,8 @@ struct WsLayout {
   long long N;
   int D, DP, M, MP;
   int training;
-  int splitsS, splitsZ;     // split-K factors of the Gram / W^T X reductions
+  int splitsS, splitsZ;     // split-K factors of the Gram (its diagonal bands on the tensor-core path) / W^T X
+  int splitsO;              // tensor-core path: split-K factor of the off-diagonal Gram units (0: none, MP <= 256)
   int nvec;                 // number of per-CTA vector partials (persistent backward CTAs)
   int vec_len;              // floats per vector partial
   // byte offsets
@@ -134,6 +135,31 @@ __host__ __device__ inline size_t tc_tiled_index(long long n, int m, int MP) {
   return ((((size_t)(n >> 7) * (size_t)(MP >> 2) + (size_t)(m >> 2)) << 7) + (size_t)(n & 127)) * 4 + (size_t)(m & 3);
 }
 
+// Gram partials of the tensor-core path: only the lower triangle of 128 x 128 blocks is computed and stored, packed,
+// block (bi, bj), bi >= bj, at block index bi (bi + 1) / 2 + bj, each block row-major.  S is symmetric: an element
+// of a block above the diagonal is the element of the mirrored block.  The Gram kernel writes through
+// tc_gram_index, stage_grad_reduce reads through its inverse tc_gram_element.
+__host__ __device__ inline size_t tc_gram_index(int i, int j) {
+  if ((i >> 7) < (j >> 7)) { const int t = i; i = j; j = t; }
+  const int bi = i >> 7, bj = j >> 7;
+  return ((size_t)(bi * (bi + 1) / 2 + bj) << 14) + ((size_t)(i & 127) << 7) + (size_t)(j & 127);
+}
+// inverse of tc_gram_index on the stored (lower) blocks: packed float index -> (i, j)
+__host__ __device__ inline void tc_gram_element(size_t idx, int* i, int* j) {
+  const int b = (int)(idx >> 14);
+  int bi = 0;
+  while ((bi + 1) * (bi + 2) / 2 <= b) ++bi;
+  *i = bi * 128 + (int)((idx >> 7) & 127);
+  *j = (b - bi * (bi + 1) / 2) * 128 + (int)(idx & 127);
+}
+__host__ __device__ inline size_t tc_gram_floats(int MP) { const size_t nb = MP / 128; return nb * (nb + 1) / 2 * 16384; }
+// the Gram units are 256-wide column bands (128 at MP = 128): a block inside the diagonal band belongs to that
+// band's diagonal unit, every other block to an off-diagonal unit (their split counts differ)
+__host__ __device__ inline bool tc_gram_diag_block(int MP, int bi, int bj) {
+  const int bw = MP >= 256 ? 2 : 1;
+  return bi / bw == bj / bw;
+}
+
 inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 
 inline int choose_splits(long long N, int ntiles) {
@@ -147,6 +173,10 @@ inline int choose_splits(long long N, int ntiles) {
   if (s > kMaxSplits) s = kMaxSplits;
   return (int)s;
 }
+
+// per-row cost of a W^T X unit per 128 rows of W, relative to one 128 x 128 Gram block, for the split choice below
+// (measured at c2 on B200: 0.6 / 1.0 / 1.5 gave 0.362 / 0.351 / 0.359 ms per step)
+constexpr double kWxCost = 1.0;
 
 inline WsLayout make_layout(long long N, int D, int M, int training) {
   WsLayout w;
@@ -193,21 +223,26 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
   const int nt = w.MP / tp;
   w.splitsS = choose_splits(N, nt * (nt + 1) / 2);
   w.splitsZ = choose_splits(N, nt);
+  w.splitsO = 0;
   if (w.MP >= 128) {
-    // tensor-core reductions: Gram = (MP / 128) row tiles x (MP / 256) column tiles x splitsS CTAs, W^T X =
-    // (MP / 128) row tiles x splitsZ CTAs: about one wave of 148 SMs each, >= 128 rows per split
-    const int qt = w.MP >= 256 ? w.MP / 256 : 1;
+    // tensor-core reductions, ONE launch of about one wave of 148 SMs (gpblur_tc_reduce.cu): per band of BW = 256
+    // inducing points (128 at MP = 128) one diagonal Gram unit (its 3 lower-triangle 128 x 128 blocks) and one W^T X
+    // unit, plus a (row tile, column band) unit of 2 blocks per row tile and band below the diagonal.  The split
+    // counts follow the per-row cost of a unit, in 128 x 128 Gram blocks: diagonal 3 (1 at MP = 128), off-diagonal 2,
+    // W^T X kWxCost per band, so that all CTAs of the wave finish together.  Splits are >= 128 rows deep.
+    const int nb = w.MP / tc_bw(w.MP);
+    const double cd = w.MP >= 256 ? 3.0 : 1.0, co = 2.0, cz = kWxCost * (w.MP >= 256 ? 2 : 1);
+    const double units = nb * cd + (double)nb * (nb - 1) * co + nb * cz;
+    const double share = units / 148.0;   // cost per CTA
     const long long maxs = (N + 127) / 128;
-    // the Gram kernel skips the [128 x 256] tiles strictly above the diagonal: only the rest needs SMs
-    int gram_tiles = 0;
-    for (int pt = 0; pt < w.MP / 128; ++pt)
-      for (int q = 0; q < qt; ++q)
-        if (q * 256 <= pt * 128 + 127) ++gram_tiles;
-    long long sS = 148 / gram_tiles, sZ = 148 / (w.MP / 128);
-    if (sS > maxs) sS = maxs;
-    if (sZ > maxs) sZ = maxs;
-    w.splitsS = (int)(sS < 1 ? 1 : sS);
-    w.splitsZ = (int)(sZ < 1 ? 1 : sZ);
+    auto fit = [&](double c) {
+      long long s = (long long)(c / share);
+      if (s > maxs) s = maxs;
+      return (int)(s < 1 ? 1 : s);
+    };
+    w.splitsS = fit(cd);
+    w.splitsO = nb > 1 ? fit(co) : 0;
+    w.splitsZ = fit(cz);
   }
   w.nvec = kMaxPersist;
   w.vec_len = w.MP + 2 * w.DP + VS_COUNT;
@@ -218,7 +253,9 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
     const size_t Nt = w.MP >= 128 ? (size_t)round_up_ll(N, 128) : (size_t)N;
     w.A = take(Nt * MP * 4);
     w.W = take(Nt * MP * 4);
-    w.Spart = take((size_t)w.splitsS * MP * MP * 4);
+    // [MP x MP] per split: the FFMA kernels (forced for MP >= 128 by GPBLUR_TC=-1) store full partials, the
+    // tensor-core Gram writes only the first tc_gram_floats(MP) of each
+    w.Spart = take((size_t)(w.splitsS > w.splitsO ? w.splitsS : w.splitsO) * MP * MP * 4);
     w.upart = take((size_t)w.splitsS * MP * 4);
     w.WXpart = take((size_t)w.splitsZ * MP * DP * 4);
     w.vecpart = take((size_t)w.nvec * w.vec_len * 4);

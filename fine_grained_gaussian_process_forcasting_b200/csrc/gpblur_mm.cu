@@ -1282,13 +1282,14 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   const float* vecpart = ws_cptr<float>(a.ws, L.vecpart);
   const float* cpart = ws_cptr<float>(a.ws, L.cpart);
   const int tp = MP < 128 ? MP : 128;   // tile size used by the Gram reduction (lower tile triangle valid)
-  double* g_u = a.sgrad;
-  double* g_vec = g_u + MP;
-  double* g_S = g_vec + L.vec_len;
-  double* g_WX = g_S + (size_t)MP * MP;
-  const size_t n_u = MP, n_vec = L.vec_len, n_S = (size_t)MP * MP, n_WX = (size_t)MP * DP;
+  const bool tc = a.ncpart > 0;
+  // S region: the FFMA Gram holds only the lower tile triangle (tile size tp) of full [MP x MP] partials, read in
+  // output order (mirrored tiles transposed); the tensor-core Gram packed lower-triangle 128 x 128 blocks, read in
+  // packed order (coalesced) and written to (i, j) and, outside the diagonal blocks, to its mirror (j, i)
+  const size_t n_u = MP, n_vec = L.vec_len, n_S = tc ? tc_gram_floats(MP) : (size_t)MP * MP, n_WX = (size_t)MP * DP;
   const size_t total = n_u + n_vec + n_S + n_WX;
-  // A CTA owns 32 consecutive output elements per iteration (lanes, coalesced); warp g sums partials g, g + 8, ...
+  const size_t s_out = n_u + n_vec;   // first S element of the stage gradient
+  // A CTA owns 32 consecutive input elements per iteration (lanes, coalesced); warp g sums partials g, g + 8, ...
   // and the 8 warp sums are folded in fixed order through shared memory (bit-deterministic), which keeps 8x more
   // loads in flight than one thread per element.
   __shared__ double red[8][32];
@@ -1296,34 +1297,48 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   const size_t nchunks = (total + 31) / 32;
   for (size_t ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
     const size_t e = ch * 32 + lane;
+    size_t dst = e, mirror = 0;   // output element(s); mirror 0: none
+    if (e >= s_out + n_S) dst = e - n_S + (size_t)MP * MP;
     double s = 0.0;
-    if (e < total && L.N > 0) {
+    if (e >= s_out && e < s_out + n_S) {
+      const size_t idx = e - s_out;
+      int i, j;
+      const float* src;
+      size_t pstride;
+      int nsp = L.splitsS;
+      if (tc) {
+        tc_gram_element(idx, &i, &j);
+        src = Spart + idx;
+        pstride = tc_gram_floats(MP);
+        if (!tc_gram_diag_block(MP, i >> 7, j >> 7)) nsp = L.splitsO;
+        if ((i >> 7) != (j >> 7)) mirror = s_out + (size_t)j * MP + i;
+      } else {
+        i = (int)(idx / MP); j = (int)(idx - (size_t)i * MP);
+        const bool lower = i / tp >= j / tp;
+        src = Spart + (size_t)(lower ? i : j) * MP + (lower ? j : i);
+        pstride = (size_t)MP * MP;
+      }
+      dst = s_out + (size_t)i * MP + j;
+      if (L.N > 0) {
+        // loads batched 4 deep before the (ordered) adds: independent requests in flight
+        int sp = g;
+        for (; sp + 24 < nsp; sp += 32) {
+          const float v0 = src[(size_t)sp * pstride], v1 = src[(size_t)(sp + 8) * pstride];
+          const float v2 = src[(size_t)(sp + 16) * pstride], v3 = src[(size_t)(sp + 24) * pstride];
+          s += (double)v0; s += (double)v1; s += (double)v2; s += (double)v3;
+        }
+        for (; sp < nsp; sp += 8) s += (double)src[(size_t)sp * pstride];
+      }
+    } else if (e < total && L.N > 0) {
       if (e < n_u) {
         for (int sp = g; sp < L.splitsS; sp += 8) s += (double)upart[(size_t)sp * MP + e];
       } else if (e < n_u + n_vec) {
         const size_t k = e - n_u;
         for (int c = g; c < a.nvec_used; c += 8) s += (double)vecpart[(size_t)c * L.vec_len + k];
-        if (a.ncpart > 0 && k < (size_t)MP)
+        if (tc && k < (size_t)MP)
           for (int c = g; c < a.ncpart; c += 8) s += (double)cpart[(size_t)c * MP + k];
-      } else if (e < n_u + n_vec + n_S) {
-        const size_t idx = e - n_u - n_vec;
-        const int i = (int)(idx / MP), j = (int)(idx - (size_t)i * MP);
-        // the FFMA Gram holds only the lower tile triangle (tile size tp); the tensor-core Gram (ncpart > 0)
-        // computes the [128 x 256] tiles (i / 128, j / 256) that touch the lower triangle: mirror the rest
-        const bool lower = a.ncpart > 0 ? ((j / 256) * 256 <= (i / 128) * 128 + 127) : (i / tp >= j / tp);
-        const int si = lower ? i : j, sj = lower ? j : i;
-        // loads batched 4 deep before the (ordered) adds: independent requests in flight
-        const float* src = Spart + (size_t)si * MP + sj;
-        const size_t pstride = (size_t)MP * MP;
-        int sp = g;
-        for (; sp + 24 < L.splitsS; sp += 32) {
-          const float v0 = src[(size_t)sp * pstride], v1 = src[(size_t)(sp + 8) * pstride];
-          const float v2 = src[(size_t)(sp + 16) * pstride], v3 = src[(size_t)(sp + 24) * pstride];
-          s += (double)v0; s += (double)v1; s += (double)v2; s += (double)v3;
-        }
-        for (; sp < L.splitsS; sp += 8) s += (double)src[(size_t)sp * pstride];
       } else {
-        const size_t idx = e - n_u - n_vec - n_S;
+        const size_t idx = e - s_out - n_S;
         for (int sp = g; sp < L.splitsZ; sp += 8) s += (double)WXpart[(size_t)sp * MP * DP + idx];
       }
     }
@@ -1334,10 +1349,10 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
       double t = 0.0;
 #pragma unroll
       for (int w = 0; w < 8; ++w) t += red[w][lane];
-      a.sgrad[e] = t;
+      a.sgrad[dst] = t;
+      if (mirror) a.sgrad[mirror] = t;
     }
   }
-  (void)g_u; (void)g_vec; (void)g_S; (void)g_WX;
 }
 
 template <int RT>
@@ -1917,7 +1932,7 @@ int launch_mm_backward(const gpblur_svgp_params& p, const WsLayout& L, void* sta
 
 int stage_grad_reduce_impl(const WsLayout& L, const void* ws, double* sgrad, int nvec_used, int ncpart,
                            cudaStream_t st) {
-  const size_t total = stage_grad_doubles(L.MP, L.DP);
+  const size_t total = stage_grad_doubles(L.MP, L.DP);   // at most the elements the kernel reads
   int grid = (int)((total + 31) / 32);
   if (grid > 16 * 148) grid = 16 * 148;
   SgReduceArgs args{L, ws, sgrad, nvec_used, ncpart};

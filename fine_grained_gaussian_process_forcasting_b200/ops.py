@@ -276,7 +276,8 @@ def rbf_covariance(x1: Tensor, x2: Tensor, raw_lengthscale: Tensor, raw_outputsc
 
 
 def debug_fetch(which: int, N: int, D: int, M: int, ws: Tensor) -> Tensor:
-    """Test probe: 0 = L, 1 = Linv, 2 = Kzz + jitter (float64 [Mp, Mp]); 3 = A (float32 [N, Mp])."""
+    """Test probe: 0 = L, 1 = Linv, 2 = Kzz + jitter (float64 [Mp, Mp]); 3 = A, 5 = W (float32 [N, Mp]); 6 = the
+    folded upstream gradients g_mu, g_var of the last backward (float32 [2, N])."""
     mp = C.c_int(0)
     Mp = 32 if M <= 32 else 128 if M <= 128 else (M + 255) // 256 * 256
     if which == 4:
@@ -284,6 +285,8 @@ def debug_fetch(which: int, N: int, D: int, M: int, ws: Tensor) -> Tensor:
     elif which in (3, 5):
         Nt = (N + 127) // 128 * 128 if Mp >= 128 else N     # tensor-core path: whole 128-point tiles, tile-major
         out = torch.empty(Nt, Mp, device=ws.device, dtype=torch.float32)
+    elif which == 6:
+        out = torch.empty(2, max(N, 1), device=ws.device, dtype=torch.float32)
     else:
         out = torch.empty(Mp, Mp, device=ws.device, dtype=torch.float64)
     with torch.cuda.device(ws.device):

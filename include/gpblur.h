@@ -239,7 +239,8 @@ int gpblur_rbf_covariance_backward(const float* x1, const float* x2, long long n
 
 /* Debug / test probes into the workspace of the last forward on (ws): copies device-to-device.
  * which: 0 = L (fp64 [Mp,Mp]), 1 = Linv (fp64 [Mp,Mp]), 2 = Kzz+jitter (fp64 [Mp,Mp]),
- *        3 = A (fp32 [N,Mp]), 4 = phase timestamps of the M x M kernels (uint64 ns [32]).
+ *        3 = A (fp32 [N,Mp]), 4 = phase timestamps of the M x M kernels (uint64 ns [32]),
+ *        5 = W (fp32 [N,Mp], after a backward), 6 = folded upstream gradients g_mu, g_var (fp32 [2,N], after a backward).
  *        Returns the padded inducing count Mp via *mp. */
 int gpblur_debug_fetch(int which, long long N, int D, int M, const void* ws, void* out,
                        size_t out_bytes, int* mp, void* stream);
