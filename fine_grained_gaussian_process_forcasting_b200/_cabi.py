@@ -16,6 +16,9 @@ LIB_PATH = _PKG / "libgpblur.so"
 GPBLUR_MAX_D = 128
 GPBLUR_MAX_M = 1024
 
+# covariance functions (GPBLUR_KERNEL_*): name used by ops.py -> kind
+KERNEL_KINDS = {"rbf": 0, "matern12": 1, "matern32": 2, "matern52": 3}
+
 ERRORS = {
     -1: "GPBLUR_EINVAL (bad shape / null pointer / misaligned workspace)",
     -2: "GPBLUR_EWORKSPACE (workspace too small)",
@@ -82,6 +85,26 @@ SIGNATURES = {
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
         C.c_void_p]),
+    "gpblur_svgp_param_stage_kind": (C.c_int, [
+        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+        C.c_size_t, C.c_void_p]),
+    "gpblur_svgp_param_stage_backward_kind": (C.c_int, [
+        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+        C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gpblur_svgp_point_forward_shared_kind": (C.c_int, [
+        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+        C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gpblur_svgp_point_backward_segments_kind": (C.c_int, [
+        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+        C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+        C.c_size_t, C.c_void_p]),
+    "gpblur_covariance": (C.c_int, [
+        C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+        C.c_void_p, C.c_void_p]),
+    "gpblur_covariance_backward_scratch_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong, C.c_int, C.c_int]),
+    "gpblur_covariance_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int,
+                                             C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_step_scratch_floats": (C.c_size_t, [C.c_int]),
     "gpblur_blur_apply_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int,
                                             C.c_void_p, C.c_void_p]),

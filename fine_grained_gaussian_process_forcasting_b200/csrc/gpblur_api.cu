@@ -268,7 +268,8 @@ __global__ void rsample_bwd_kernel(const float* __restrict__ var, const float* _
   g_var[i] = g * philox_normal(seed, offset + (uint64_t)i, stream_id) * 0.5f * rsqrtf(var[i]);
 }
 
-// dense ScaleKernel(RBF): 16 x 16 output tile per CTA, direct differences
+// dense ScaleKernel(RBF | Matern): 16 x 16 output tile per CTA, direct differences
+template <int KIND>
 __global__ void rbf_cov_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n1,
                                long long n2, int D, const float* __restrict__ raw_ell, int ard,
                                const float* __restrict__ raw_os, float* __restrict__ out) {
@@ -304,7 +305,13 @@ __global__ void rbf_cov_kernel(const float* __restrict__ x1, const float* __rest
   if (i < n1 && j < n2) {
     const float r = raw_os[0];
     const float os = r > 20.f ? r : log1pf(expf(r));
-    out[(size_t)i * n2 + j] = os * expf(-0.5f * acc);
+    if constexpr (KIND == GPBLUR_KERNEL_RBF) {
+      out[(size_t)i * n2 + j] = os * expf(-0.5f * acc);
+    } else {
+      float k, g;
+      matern_kg<KIND>(acc, os, k, g);
+      out[(size_t)i * n2 + j] = k;
+    }
   }
 }
 
@@ -406,6 +413,31 @@ int gpblur_svgp_param_stage_shared_sms(const gpblur_svgp_params* p, int D, int M
   return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream, extra_jitter, max_ctas);
 }
 
+int gpblur_svgp_param_stage_kind(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter,
+                                 int max_ctas, float* kl, int* info, void* stage, size_t stage_bytes, void* stream) {
+  int rc = validate(p, 0, D, M);
+  if (rc) return rc;
+  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
+  if (!stage || (reinterpret_cast<uintptr_t>(stage) & 255) || !(extra_jitter >= 0.0) || max_ctas < 0) return GPBLUR_EINVAL;
+  WsLayout L = make_layout(0, D, M, 0);
+  L.kind = kind;
+  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
+  return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream, extra_jitter, max_ctas);
+}
+
+int gpblur_svgp_param_stage_backward_kind(const gpblur_svgp_params* p, int D, int M, int kind,
+                                          const double* stage_grad, const float* g_kl, float* grad_bucket,
+                                          int accumulate, int max_ctas, void* stage, size_t stage_bytes, void* stream) {
+  int rc = validate(p, 0, D, M);
+  if (rc) return rc;
+  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
+  if (!stage_grad || !grad_bucket || !stage || (reinterpret_cast<uintptr_t>(stage) & 255) || max_ctas < 0) return GPBLUR_EINVAL;
+  WsLayout L = make_layout(0, D, M, 0);
+  L.kind = kind;
+  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
+  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream, accumulate ? 1 : 0, max_ctas);
+}
+
 int gpblur_svgp_param_stage_backward_shared_sms(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
                                                 const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
                                                 void* stage, size_t stage_bytes, void* stream) {
@@ -453,16 +485,17 @@ int gpblur_svgp_forward_cached(const gpblur_svgp_params* p, const float* x, long
                                    training, ws, ws_bytes, stream);
 }
 
-int gpblur_svgp_point_backward(const float* x, long long N, int D, int M, const float* g_mean, const float* g_var,
-                               const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
-                               uint32_t stream_id, const unsigned long long* offset_dev, float* dx,
+static int point_backward_kind(const float* x, long long N, int D, int M, int kind, const float* g_mean,
+                               const float* g_var, const float* g_sample, const float* var, uint64_t seed,
+                               uint64_t offset, uint32_t stream_id, const unsigned long long* offset_dev, float* dx,
                                double* stage_grad, void* ws, size_t ws_bytes, void* stream) {
   OffsetDevScope ods(offset_dev);
-  if (N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
+  if (N < 0 || D < 1 || M < 1 || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
   if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
   if (!stage_grad || !ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
   if (N > 0 && (!x || !var)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(N, D, M, 1);
+  WsLayout L = make_layout(N, D, M, 1);
+  L.kind = kind;
   if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = GPBLUR_OK;
@@ -478,16 +511,34 @@ int gpblur_svgp_point_backward(const float* x, long long N, int D, int M, const 
   return launch_stage_grad_reduce(L, ws, stage_grad, st);
 }
 
+int gpblur_svgp_point_backward(const float* x, long long N, int D, int M, const float* g_mean, const float* g_var,
+                               const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
+                               uint32_t stream_id, const unsigned long long* offset_dev, float* dx,
+                               double* stage_grad, void* ws, size_t ws_bytes, void* stream) {
+  return point_backward_kind(x, N, D, M, GPBLUR_KERNEL_RBF, g_mean, g_var, g_sample, var, seed, offset, stream_id,
+                             offset_dev, dx, stage_grad, ws, ws_bytes, stream);
+}
+
 int gpblur_svgp_point_forward_shared(const void* param_stage, const float* x, long long N, int D, int M, float* mean,
                                      float* var, float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
                                      const unsigned long long* offset_dev, int training, void* ws, size_t ws_bytes,
                                      void* stream) {
+  return gpblur_svgp_point_forward_shared_kind(param_stage, x, N, D, M, GPBLUR_KERNEL_RBF, mean, var, sample, seed,
+                                               offset, stream_id, offset_dev, training, ws, ws_bytes, stream);
+}
+
+int gpblur_svgp_point_forward_shared_kind(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                                          float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
+                                          uint32_t stream_id, const unsigned long long* offset_dev, int training,
+                                          void* ws, size_t ws_bytes, void* stream) {
   OffsetDevScope ods(offset_dev);
   if (!param_stage || (reinterpret_cast<uintptr_t>(param_stage) & 255) || N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
+  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
   if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
   if (N > 0 && (!x || !mean || !var)) return GPBLUR_EINVAL;
   if (!ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(N, D, M, training ? 1 : 0);
+  WsLayout L = make_layout(N, D, M, training ? 1 : 0);
+  L.kind = kind;
   if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
   if (N == 0) return GPBLUR_OK;
   ParamStageScope pss(param_stage);
@@ -503,6 +554,30 @@ int gpblur_svgp_point_backward_shared(const void* param_stage, const float* x, l
   ParamStageScope pss(param_stage);
   return gpblur_svgp_point_backward(x, N, D, M, g_mean, g_var, g_sample, var, seed, offset, stream_id, offset_dev, dx,
                                     stage_grad, ws, ws_bytes, stream);
+}
+
+int gpblur_svgp_point_backward_segments_kind(const void* param_stage, const float* x, long long N, int D, int M,
+                                             int kind, int nseg, const long long* seg_start,
+                                             const float* const* g_mean, const float* const* g_var,
+                                             const float* const* g_sample, const float* var, uint64_t seed,
+                                             uint64_t offset, uint32_t stream_id,
+                                             const unsigned long long* offset_dev, float* dx, double* stage_grad,
+                                             void* ws, size_t ws_bytes, void* stream) {
+  if (nseg < 1 || nseg > kMaxSegments || !seg_start || seg_start[0] != 0) return GPBLUR_EINVAL;
+  if (param_stage && (reinterpret_cast<uintptr_t>(param_stage) & 255)) return GPBLUR_EINVAL;
+  SegGrads sg{};
+  sg.nseg = nseg;
+  for (int i = 0; i < nseg; ++i) {
+    if (seg_start[i] < 0 || seg_start[i] > N || (i > 0 && seg_start[i] < seg_start[i - 1])) return GPBLUR_EINVAL;
+    sg.start[i] = seg_start[i];
+    sg.gm[i] = g_mean ? g_mean[i] : nullptr;
+    sg.gv[i] = g_var ? g_var[i] : nullptr;
+    sg.gs[i] = g_sample ? g_sample[i] : nullptr;
+  }
+  SegGradsScope sgs(sg);
+  ParamStageScope pss(param_stage);
+  return point_backward_kind(x, N, D, M, kind, nullptr, nullptr, nullptr, var, seed, offset, stream_id, offset_dev, dx,
+                             stage_grad, ws, ws_bytes, stream);
 }
 
 int gpblur_svgp_point_backward_segments(const void* param_stage, const float* x, long long N, int D, int M, int nseg,
@@ -652,12 +727,29 @@ int gpblur_rsample_backward(const float* var, const float* g_out, long long n, u
 int gpblur_rbf_covariance(const float* x1, const float* x2, long long n1, long long n2, int D,
                           const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out,
                           void* stream) {
-  if (n1 < 0 || n2 < 0 || D < 1 || !raw_lengthscale || !raw_outputscale) return GPBLUR_EINVAL;
+  return gpblur_covariance(x1, x2, n1, n2, D, GPBLUR_KERNEL_RBF, raw_lengthscale, ard, raw_outputscale, out, stream);
+}
+
+int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                      const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream) {
+  if (n1 < 0 || n2 < 0 || D < 1 || !raw_lengthscale || !raw_outputscale || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
   if (n1 == 0 || n2 == 0) return GPBLUR_OK;
   if (!x1 || !x2 || !out) return GPBLUR_EINVAL;
   dim3 grid((unsigned)((n2 + 15) / 16), (unsigned)((n1 + 15) / 16));
-  rbf_cov_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x1, x2, n1, n2, D, raw_lengthscale, ard,
-                                                         raw_outputscale, out);
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (kind) {
+    case GPBLUR_KERNEL_MATERN12:
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      break;
+    case GPBLUR_KERNEL_MATERN32:
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      break;
+    case GPBLUR_KERNEL_MATERN52:
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      break;
+    default:
+      rbf_cov_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+  }
   note_launch();
   return check_launch("rbf_cov");
 }

@@ -21,7 +21,63 @@ constexpr int kMaxSplits = 148;          // split-K factor cap of the N-reductio
 enum { H_OS = 0, H_JIT = 1, H_CWB = 2, H_KL = 3, H_COUNT = 8 };
 constexpr int kStampSlots = 32;   // phase timestamps (globaltimer ns) of the M x M kernels: [0,16) forward, [16,32) backward
 // per-CTA vector partial layout of the backward point kernel: [colsum MP | q DP | wbar DP | scalars 4]
-enum { VS_GMU = 0, VS_RSUM = 1, VS_GVAR = 2, VS_COUNT = 4 };
+// VS_KBK = sum kbar o k: the outputscale gradient of the Matern kinds (for RBF, W = kbar o k and VS_RSUM is that sum)
+enum { VS_GMU = 0, VS_RSUM = 1, VS_GVAR = 2, VS_KBK = 3, VS_COUNT = 4 };
+
+// ---- covariance functions (GPBLUR_KERNEL_*, include/gpblur.h) ----------------------------------------------------
+// k = os f(r) with r = sqrt(max(d2, 1e-30)), and g = -2 os df/d(d2) = -os f'(r) / r: every distance gradient is the RBF
+// one with W = kbar o g in place of kbar o k (for RBF g = k).  g = 0 where the clamp is active (d2 <= 1e-30).  Every
+// kernel site evaluates the Matern kinds through these functions; the RBF sites keep their own exp.
+__host__ __device__ constexpr bool kernel_kind_valid(int kind) {
+  return kind >= GPBLUR_KERNEL_RBF && kind <= GPBLUR_KERNEL_MATERN52;
+}
+__device__ __forceinline__ float ex2_fast(float v) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(v));
+  return y;
+}
+// fp32, the kind a template argument so that the coefficients are immediates
+template <int KIND>
+__device__ __forceinline__ void matern_kg(float d2, float os, float& k, float& g) {
+  static_assert(KIND == GPBLUR_KERNEL_MATERN12 || KIND == GPBLUR_KERNEL_MATERN32 || KIND == GPBLUR_KERNEL_MATERN52,
+                "Matern kinds only");
+  const float dc = fmaxf(d2, 1e-30f);
+  const float ir = rsqrtf(dc), r = dc * ir;
+  const bool live = d2 > 1e-30f;
+  if constexpr (KIND == GPBLUR_KERNEL_MATERN12) {
+    const float e = os * ex2_fast(-1.4426950408889634f * r);
+    k = e;
+    g = live ? e * ir : 0.f;
+  } else if constexpr (KIND == GPBLUR_KERNEL_MATERN32) {
+    const float s = 1.7320508075688772f * r, e = os * ex2_fast(-1.4426950408889634f * s);
+    k = fmaf(s, e, e);
+    g = live ? 3.0f * e : 0.f;
+  } else {
+    const float s = 2.2360679774997896f * r, e = os * ex2_fast(-1.4426950408889634f * s);
+    const float p = 1.0f + s;
+    k = fmaf(s * s * (1.0f / 3.0f), e, p * e);
+    g = live ? (5.0f / 3.0f) * p * e : 0.f;
+  }
+}
+// fp64 (the M x M stage): any kind
+__device__ __forceinline__ void kernel_kg64(int kind, double d2, double os, double& k, double& g) {
+  if (kind == GPBLUR_KERNEL_RBF) { k = os * exp(-0.5 * d2); g = k; return; }
+  const double r = sqrt(fmax(d2, 1e-30));
+  const bool live = d2 > 1e-30;
+  if (kind == GPBLUR_KERNEL_MATERN12) {
+    const double e = os * exp(-r);
+    k = e;
+    g = live ? e / r : 0.0;
+  } else if (kind == GPBLUR_KERNEL_MATERN32) {
+    const double s = 1.7320508075688772 * r, e = os * exp(-s);
+    k = (1.0 + s) * e;
+    g = live ? 3.0 * e : 0.0;
+  } else {
+    const double s = 2.2360679774997896 * r, e = os * exp(-s);
+    k = (1.0 + s + s * s / 3.0) * e;
+    g = live ? (5.0 / 3.0) * (1.0 + s) * e : 0.0;
+  }
+}
 
 __host__ __device__ inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
 __host__ __device__ inline long long round_up_ll(long long a, long long b) { return (a + b - 1) / b * b; }
@@ -60,6 +116,8 @@ struct WsLayout {
   size_t v64, t64;                 // fp64 scratch of the M x M backward (part of the parameter stage)
   size_t A, W, Spart, upart, WXpart, vecpart, gsc, rrow, cpart, sgrad;
   size_t total;
+  size_t D2zz64;            // fp64 inducing-pair distances d2 of the Kzz build (Matern kinds: read by the backward)
+  int kind;                 // covariance function (GPBLUR_KERNEL_*); make_layout leaves RBF, the *_kind entry points set it
 };
 
 // ---- UMMA slab images of the constant operands (tensor-core path) -------------------------------------------
@@ -180,7 +238,7 @@ constexpr double kWxCost = 1.0;
 
 inline WsLayout make_layout(long long N, int D, int M, int training) {
   WsLayout w;
-  w.N = N; w.D = D; w.M = M; w.training = training;
+  w.N = N; w.D = D; w.M = M; w.training = training; w.kind = GPBLUR_KERNEL_RBF;
   w.DP = padded_d(D); w.MP = padded_m(M);
   const size_t MP = w.MP, DP = w.DP;
   size_t o = 0;
@@ -248,6 +306,7 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
   w.vec_len = w.MP + 2 * w.DP + VS_COUNT;
   w.v64 = take((size_t)(3 * MP + w.vec_len) * 8);
   w.t64 = take((size_t)MP * DP * 8);
+  w.D2zz64 = take(MP * MP * 8);      // last region of the parameter stage: the offsets before it do not depend on it
   if (training) {
     // the tensor-core kernels keep A and W TILE-major (see tc_tiled_index): whole 128-point tiles
     const size_t Nt = w.MP >= 128 ? (size_t)round_up_ll(N, 128) : (size_t)N;

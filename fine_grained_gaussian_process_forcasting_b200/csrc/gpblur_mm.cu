@@ -448,6 +448,8 @@ struct MmFwdArgs {
   unsigned* flags;       // two zeroed words: diagonal blocks published, worker arrivals (phase 2)
 };
 
+// MAT: a Matern kind (L.kind); the RBF instantiation carries none of the Matern code
+template <bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
   cg::grid_group grid = cg::this_grid();
   unsigned bar_target = 0;
@@ -484,6 +486,7 @@ __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
   double* Li64 = ws_ptr<double>(a.ws, L.Linv64);
   double* T64 = ws_ptr<double>(a.ws, L.T64);
   double* W64 = ws_ptr<double>(a.ws, L.U64);   // forward only: trailing matrix of the Cholesky (the backward reuses it)
+  double* D2 = ws_ptr<double>(a.ws, L.D2zz64);
   float* LinvT32 = ws_ptr<float>(a.ws, L.LinvT32);
   float* LC32 = ws_ptr<float>(a.ws, L.LC32);
   float* Linv32 = ws_ptr<float>(a.ws, L.Linv32);
@@ -556,8 +559,19 @@ __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
       for (int i = 0; i < 4; ++i) {
         const int gi = bi * TB + ty + 8 * i, gj = bj * TB + tx;
         double kv;
-        if (gi < M && gj < M) kv = os * exp(-0.5 * acc[i]) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
-        else kv = (gi == gj) ? 1.0 : 0.0;
+        if (gi < M && gj < M) {
+          if constexpr (!MAT) {
+            kv = os * exp(-0.5 * acc[i]) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
+          } else {
+            double kk, g;
+            kernel_kg64(L.kind, acc[i], os, kk, g);
+            kv = kk + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
+            D2[(size_t)gi * MP + gj] = acc[i];
+            D2[(size_t)gj * MP + gi] = acc[i];
+          }
+        } else {
+          kv = (gi == gj) ? 1.0 : 0.0;
+        }
         K64[(size_t)gi * MP + gj] = kv;
         K64[(size_t)gj * MP + gi] = kv;
         W64[(size_t)gi * MP + gj] = kv;                       // working copy (lower block triangle) of the factorisation
@@ -1071,6 +1085,7 @@ constexpr int kSmallZs = TB * (GPBLUR_MAX_D + 1);     // doubles: scaled inducin
 constexpr size_t kSmallFwdSmem = (size_t)(kSmallZs + 2 * TB * TLD + 2 * TB + GPBLUR_MAX_D) * sizeof(double) +
                                  (size_t)(2 * GPBLUR_MAX_D + 2 * TB) * sizeof(float);
 
+template <bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_small_forward_kernel(MmFwdArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* Zs = reinterpret_cast<double*>(smem_raw);          // [32][DP + 1]  Z / ell (raw, not centred: differences)
@@ -1168,8 +1183,18 @@ __global__ void __launch_bounds__(kThreads) mm_small_forward_kernel(MmFwdArgs a)
         acc = fma(df, df, acc);
       }
       double kv;
-      if (gi < M && gj < M) kv = os * exp(-0.5 * acc) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
-      else kv = (gi == gj) ? 1.0 : 0.0;
+      if (gi < M && gj < M) {
+        if constexpr (!MAT) {
+          kv = os * exp(-0.5 * acc) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
+        } else {
+          double kk, g;
+          kernel_kg64(L.kind, acc, os, kk, g);
+          kv = kk + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
+          ws_ptr<double>(a.ws, L.D2zz64)[(size_t)gi * MP + gj] = acc;
+        }
+      } else {
+        kv = (gi == gj) ? 1.0 : 0.0;
+      }
       K64[(size_t)gi * MP + gj] = kv;
       Ks[gi * TLD + gj] = kv;
     }
@@ -1355,7 +1380,7 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   }
 }
 
-template <int RT>
+template <int RT, bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   constexpr int NH = TB / RT;   // row parts of a 32 x 32 tile
   constexpr int NR = RT / 8;    // rows per thread
@@ -1390,8 +1415,9 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   const double* vec64 = a.sgrad + MP;
   const double* S64 = vec64 + L.vec_len;
   const double* WX64 = S64 + (size_t)MP * MP;
-  // fp64 vector scratch: [unused MP | unused vec_len | diag(S) MP | rz MP]
+  // fp64 vector scratch: [row sums of sym(Kb) o (Kzz - jitter I) MP (Matern kinds) | unused vec_len | diag(S) MP | rz MP]
   double* v64 = ws_ptr<double>(a.ws, L.v64);
+  double* kbk64 = v64;
   double* rz64 = v64 + 2 * MP + L.vec_len;
   double* t64 = ws_ptr<double>(a.ws, L.t64);   // [MP, DP] per-(i, d) terms of d lengthscale
 
@@ -1477,7 +1503,30 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   const double zz_jitter = ws_cptr<double>(a.ws, L.hyp64)[H_JIT];
   // ---------------- phase 5: Wzz = sym(Kb) o (Kzz - jitter I) -> U64 ----------------
   // (building Wzz on the fly while phase 6 stages its A operand was tried: the transposed read made it 2x slower)
-  {
+  // Matern kinds: Wzz = sym(Kb) o g(d2) from the distances the forward kept; the outputscale term
+  // sum sym(Kb) o (Kzz - jitter I) is no longer sum Wzz: its row sums go to kbk64 (one warp per row, fixed order)
+  if constexpr (MAT) {
+    const double os = hyp64[H_OS];
+    const double* D2 = ws_cptr<double>(a.ws, L.D2zz64);
+    for (int i = blockIdx.x * 8 + warp; i < MP; i += G * 8) {
+      double rs = 0.0;
+      for (int j = lane; j < MP; j += 32) {
+        const size_t idx = (size_t)i * MP + j;
+        double v = 0.0;
+        if (i < M && j < M) {
+          const double kb = 0.5 * (T64[idx] + T64[(size_t)j * MP + i]);
+          double kk, g;
+          kernel_kg64(L.kind, D2[idx], os, kk, g);
+          v = kb * g;
+          rs += kb * (K64[idx] - (i == j ? zz_jitter : 0.0));
+        }
+        U64[idx] = v;
+      }
+      rs = warp_sum(rs);
+      if (lane == 0) kbk64[i] = rs;
+    }
+    GPBLUR_GRID_SYNC();
+  } else {
     for (int idx = gtid; idx < MP * MP; idx += gsize) {
       const int i = idx / MP, j = idx - i * MP;
       double v = 0.0;
@@ -1600,11 +1649,14 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
       GPBLUR_PUT(&b_s[m], (float)(2.0 * ss * S64[(size_t)m * MP + m] + gkl * (ss - 1.0 / ss)));
     }
     if (warp == 0) {
+      // sum sym(Kb) o (Kzz - jitter I) + sum kbar o k: for RBF both are the sums of the W matrices
+      constexpr bool rbf = !MAT;
+      const double* rows = rbf ? rz64 : kbk64;
       double s = 0.0;
-      for (int i = lane; i < M; i += 32) s += rz64[i];
+      for (int i = lane; i < M; i += 32) s += rows[i];
       s = warp_sum(s);
       if (lane == 0) {
-        const double dos = (s + sc[VS_RSUM]) / os + sc[VS_GVAR];
+        const double dos = (s + sc[rbf ? VS_RSUM : VS_KBK]) / os + sc[VS_GVAR];
         GPBLUR_PUT(&b_os[0], (float)(dos * sigmoid64((double)a.p.raw_outputscale[0])));
         GPBLUR_PUT(&b_b[0], (float)sc[VS_GMU]);
       }
@@ -1621,6 +1673,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
 // (general kernel at M = 32: 23 us in-kernel, 45 us with the cooperative launch around it).
 constexpr size_t kSmallBwdSmem = (size_t)(6 * TB * TLD + 2 * TB * (GPBLUR_MAX_D + 1) + 6 * TB + GPBLUR_MAX_D + 8) * sizeof(double);
 
+template <bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* Ss = reinterpret_cast<double*>(smem_raw);   // [32][33] S (stage gradient), later Wzz
@@ -1734,13 +1787,31 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   }
   __syncthreads();
   // ---- phase 5: Wzz = sym(Kbar) o (Kzz - jitter I) -> Ss ; row sums ----
+  // (Matern kinds: Wzz = sym(Kbar) o g(d2); the products sym(Kbar) o (Kzz - jitter I) of the outputscale term are
+  //  parked in Us, free since phase 4, and summed into kbk)
+  constexpr bool rbf = !MAT;
+  double kbk = 0.0;
   {
     const double zz_jitter = hyp64[H_JIT];
+    const double os = hyp64[H_OS];
+    const double* D2 = ws_cptr<double>(a.ws, L.D2zz64);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int r = warp + 8 * i;
       double v = 0.0;
-      if (r < M && lane < M) v = 0.5 * (Ts[r * TLD + lane] + Ts[lane * TLD + r]) * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
+      if (rbf) {
+        if (r < M && lane < M) v = 0.5 * (Ts[r * TLD + lane] + Ts[lane * TLD + r]) * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
+      } else {
+        double u = 0.0;
+        if (r < M && lane < M) {
+          const double kb = 0.5 * (Ts[r * TLD + lane] + Ts[lane * TLD + r]);
+          double kk, g;
+          kernel_kg64(L.kind, D2[(size_t)r * MP + lane], os, kk, g);
+          v = kb * g;
+          u = kb * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
+        }
+        Us[r * TLD + lane] = u;
+      }
       Ss[r * TLD + lane] = v;
     }
   }
@@ -1749,6 +1820,10 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     double rz = 0.0;
     for (int j = 0; j < TB; ++j) rz += Ss[tid * TLD + j];
     rz_s[tid] = rz;
+  }
+  if (!rbf && warp == 7) {
+    for (int r = 0; r < M; ++r) kbk += Us[r * TLD + lane];
+    kbk = warp_sum(kbk);
   }
   __syncthreads();
   // (diag(S) of the stage gradient is needed in phase 7 and Ss now holds Wzz: it is re-read from global memory there)
@@ -1808,9 +1883,9 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     }
     if (warp == 7) {
       double s = lane < M ? rz_s[lane] : 0.0;
-      s = warp_sum(s);
+      s = rbf ? warp_sum(s) : kbk;
       if (lane == 0) {
-        const double dos = (s + sc[VS_RSUM]) / os + sc[VS_GVAR];
+        const double dos = (s + sc[rbf ? VS_RSUM : VS_KBK]) / os + sc[VS_GVAR];
         GPBLUR_PUT(&b_os[0], (float)(dos * sigmoid64((double)a.p.raw_outputscale[0])));
         GPBLUR_PUT(&b_b[0], (float)sc[VS_GMU]);
       }
@@ -1844,14 +1919,18 @@ int coop_grid(const void* func, int want, size_t smem) {
 int launch_mm_forward(const gpblur_svgp_params& p, const WsLayout& L, void* ws, float* kl, int* info,
                       cudaStream_t st, double extra_jitter, int max_ctas) {
   const size_t smem = sizeof(Tile) * 11 + kGemmScratchDoubles * sizeof(double);
+  const bool mat = L.kind != GPBLUR_KERNEL_RBF;
+  const void* fwd = mat ? (const void*)mm_forward_kernel<true> : (const void*)mm_forward_kernel<false>;
   // per-DEVICE attribute: set on every launch (cheap) instead of a process-wide flag
-  cudaFuncSetAttribute(mm_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaFuncSetAttribute(fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   const int nb = L.MP / TB;
   if (nb == 1) {   // M <= 32: one CTA, no grid barrier, plain launch
-    cudaFuncSetAttribute(mm_small_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallFwdSmem);
+    const void* small = mat ? (const void*)mm_small_forward_kernel<true> : (const void*)mm_small_forward_kernel<false>;
+    cudaFuncSetAttribute(small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallFwdSmem);
     MmFwdArgs args{p, L, ws, kl, info, extra_jitter, nullptr, -1, nullptr};
     ProfScope ps(ST_MM_FWD, st);
-    mm_small_forward_kernel<<<1, kThreads, kSmallFwdSmem, st>>>(args);
+    void* kargs[] = {&args};
+    cudaLaunchKernel(small, dim3(1), dim3(kThreads), kargs, kSmallFwdSmem, st);
     note_launch();
     return check_launch("mm_small_forward");
   }
@@ -1866,7 +1945,7 @@ int launch_mm_forward(const gpblur_svgp_params& p, const WsLayout& L, void* ws, 
   if (max_ctas > 0 && want > max_ctas) want = max_ctas;
   if (want < 8) want = 8;
   if (want > 148) want = 148;
-  const int grid = coop_grid((const void*)mm_forward_kernel, want, smem);
+  const int grid = coop_grid(fwd, want, smem);
 #ifdef GPBLUR_TRACE   // developer builds only (scripts/mm_only.py, mm_step_probe.py): the kernel returns after a phase
   static const int dbg_stop = [] { const char* e = getenv("GPBLUR_MM_STOP"); return e ? atoi(e) : -1; }();
 #else
@@ -1878,12 +1957,13 @@ int launch_mm_forward(const gpblur_svgp_params& p, const WsLayout& L, void* ws, 
   if (!mm_cooperative()) {
     args.bar = sync_words;
     cudaMemsetAsync(sync_words, 0, sizeof(unsigned), st);
-    mm_forward_kernel<<<grid, kThreads, smem, st>>>(args);
+    void* kargs[] = {&args};
+    cudaLaunchKernel(fwd, dim3(grid), dim3(kThreads), kargs, smem, st);
     note_launch();
     return check_launch("mm_forward");
   }
   void* kargs[] = {&args};
-  cudaError_t e = cudaLaunchCooperativeKernel((const void*)mm_forward_kernel, dim3(grid), dim3(kThreads),
+  cudaError_t e = cudaLaunchCooperativeKernel(fwd, dim3(grid), dim3(kThreads),
                                               kargs, smem, st);
   note_launch();
   if (e != cudaSuccess) return check_launch("mm_forward");
@@ -1893,11 +1973,14 @@ int launch_mm_forward(const gpblur_svgp_params& p, const WsLayout& L, void* ws, 
 int launch_mm_backward(const gpblur_svgp_params& p, const WsLayout& L, void* stage, const double* sgrad,
                        const float* g_kl, float* grad_bucket, cudaStream_t st, int accumulate, int max_ctas) {
   const int nb = L.MP / TB;
+  const bool mat = L.kind != GPBLUR_KERNEL_RBF;
   if (nb == 1) {   // M <= 32: one CTA, everything in shared memory, plain launch
-    cudaFuncSetAttribute(mm_small_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallBwdSmem);
+    const void* small = mat ? (const void*)mm_small_backward_kernel<true> : (const void*)mm_small_backward_kernel<false>;
+    cudaFuncSetAttribute(small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmallBwdSmem);
     MmBwdArgs args{p, L, stage, sgrad, g_kl, grad_bucket, accumulate, nullptr};
     ProfScope ps(ST_MM_BWD, st);
-    mm_small_backward_kernel<<<1, kThreads, kSmallBwdSmem, st>>>(args);
+    void* kargs[] = {&args};
+    cudaLaunchKernel(small, dim3(1), dim3(kThreads), kargs, kSmallBwdSmem, st);
     note_launch();
     return check_launch("mm_small_backward");
   }
@@ -1905,7 +1988,8 @@ int launch_mm_backward(const gpblur_svgp_params& p, const WsLayout& L, void* sta
   // barriers instead of grid barriers, was tried: 29 us against 21 us on 8 CTAs - the elementwise phases want the threads)
   const bool half = 2 * nb * nb <= 2 * 148;
   const size_t smem = half ? wide_bytes<16>() : wide_bytes<32>();
-  const void* func = half ? (const void*)mm_backward_kernel<16> : (const void*)mm_backward_kernel<32>;
+  const void* func = mat ? (half ? (const void*)mm_backward_kernel<16, true> : (const void*)mm_backward_kernel<32, true>)
+                         : (half ? (const void*)mm_backward_kernel<16, false> : (const void*)mm_backward_kernel<32, false>);
   cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
   int want = (half ? 2 : 1) * nb * nb;
   const int dwant = (L.MP * L.DP + kThreads - 1) / kThreads;

@@ -4,7 +4,7 @@
 //   g_mu, g_var  <- upstream (mean, variance, reparameterised sample folded, variance clamp respected)
 //   k            <- recomputed from X and the staged Z~ tiles (stage A, as in the forward)
 //   kbar[n, :]   = g_mu[n] beta + 2 g_var[n] (diag(c) Linv)^T a[n, :]        block-triangular GEMM on saved A
-//   W            = kbar o k ;  r[n] = sum_m W ;  colsum[m] = sum_n W
+//   W            = kbar o k ;  r[n] = sum_m W ;  colsum[m] = sum_n W     (Matern kinds: W = kbar o g)
 //   dx[n, :]     = ( W Z~ - r x~ ) / ell + g_mu w                             GEMM on the resident W chunk
 // W is also written to HBM once: the N-reduction GEMMs (gpblur_reduce.cu) turn it into dZ / d lengthscale.
 // Per-CTA vector partials (colsum, q = sum r x~^2, wbar, scalar sums) are reduced by the M x M stage.
@@ -24,7 +24,9 @@ struct BwdSmem {
   }
 };
 
-template <class Cfg, int DP>
+// KIND (GPBLUR_KERNEL_*): for the Matern kinds the recomputed chunk holds d2 instead of k, and step (c) forms
+// W = kbar o g and the sum of kbar o k (vector partial slot VS_KBK) from it
+template <class Cfg, int DP, int KIND>
 __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_kernel(PointBwdArgs a) {
   constexpr int PT = Cfg::PT, CT = Cfg::CT, CW = Cfg::CW, TN = Cfg::TN, TXN = Cfg::TXN, TYN = Cfg::TYN;
   using S = BwdSmem<Cfg, DP>;
@@ -79,6 +81,7 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
   for (int i = tid; i < MP; i += kThreads) colsum_s[i] = 0.f;
   for (int i = tid; i < DP; i += kThreads) { q_s[i] = 0.f; t1_s[i] = 0.f; }
   if (tid < 16) sc_s[tid] = 0.f;
+  float kbk_acc = 0.f;                            // Matern kinds: this thread's share of sum kbar o k
 
   for (int tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
     const long long n0 = (long long)tile * TN;
@@ -142,7 +145,8 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
           for (int f = 0; f < CT; ++f) {
             const int m = jc + Cfg::col(tx, f);
             const float d2 = fmaxf(xn + zn[m] - 2.0f * acc[e][f], 0.f);
-            kv[f] = (m < M) ? os * expf(-0.5f * d2) : 0.f;
+            if constexpr (KIND == GPBLUR_KERNEL_RBF) kv[f] = (m < M) ? os * expf(-0.5f * d2) : 0.f;
+            else kv[f] = (m < M) ? d2 : 1e30f;   // padded columns: k = g = 0
           }
           *reinterpret_cast<float4*>(Ws + (size_t)n * ldw + tx * 4) = make_float4(kv[0], kv[1], kv[2], kv[3]);
           if (CT == 8)
@@ -195,7 +199,14 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
 #pragma unroll
           for (int f = 0; f < CT; ++f) {
             const float kb = fmaf(gv2, acc[e][f], gm * bet[f]);
-            w[f] = kb * kk[f];
+            if constexpr (KIND == GPBLUR_KERNEL_RBF) {
+              w[f] = kb * kk[f];
+            } else {
+              float kv, g;
+              matern_kg<KIND>(kk[f], os, kv, g);
+              w[f] = kb * g;
+              kbk_acc = fmaf(kb, kv, kbk_acc);
+            }
             rsum_p[e] += w[f];
             cpart[f] += w[f];
           }
@@ -336,6 +347,17 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
     }
   }  // tiles
 
+  if constexpr (KIND != GPBLUR_KERNEL_RBF) {                // fixed order: lanes, then warps
+    __syncthreads();
+    const float s = warp_sum(kbk_acc);
+    if (lane == 0) dpart[warp] = s;
+    __syncthreads();
+    if (tid == 0) {
+      float t = 0.f;
+      for (int w8 = 0; w8 < kThreads / 32; ++w8) t += dpart[w8];
+      sc_s[VS_KBK] = t;
+    }
+  }
   __syncthreads();
   float* vp = vecpart + (size_t)blockIdx.x * L.vec_len;
   for (int i = tid; i < MP; i += kThreads) vp[i] = colsum_s[i];
@@ -362,17 +384,33 @@ inline int bwd_persistent_grid(const WsLayout& L, int TN) {
   return (int)(nt < kMaxPersist ? (nt < 1 ? 1 : nt) : kMaxPersist);
 }
 
-template <class Cfg, int DP>
-int launch_bwd_cfg(const PointBwdArgs& a0, cudaStream_t st) {
+template <class Cfg, int DP, int KIND>
+int launch_bwd_kind(const PointBwdArgs& a0, cudaStream_t st) {
   PointBwdArgs a = a0;
   const size_t smem = sizeof(float) * BwdSmem<Cfg, DP>::floats(a.L.MP);
-  cudaFuncSetAttribute(point_bwd_kernel<Cfg, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
+  cudaFuncSetAttribute(point_bwd_kernel<Cfg, DP, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
   a.ntiles = (int)((a.L.N + Cfg::TN - 1) / Cfg::TN);
   const int grid = bwd_persistent_grid(a.L, Cfg::TN);
   ProfScope ps(ST_POINT_BWD, st);
-  point_bwd_kernel<Cfg, DP><<<grid, kThreads, smem, st>>>(a);
+  point_bwd_kernel<Cfg, DP, KIND><<<grid, kThreads, smem, st>>>(a);
   note_launch();
   return check_launch("point_bwd");
+}
+
+template <class Cfg, int DP>
+int launch_bwd_cfg(const PointBwdArgs& a, cudaStream_t st) {
+  // the Matern kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
+  if constexpr (Cfg::CW != 32) {
+    if (a.L.kind != GPBLUR_KERNEL_RBF) return GPBLUR_EUNSUPPORTED;
+    return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_RBF>(a, st);
+  } else {
+    switch (a.L.kind) {
+      case GPBLUR_KERNEL_MATERN12: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN12>(a, st);
+      case GPBLUR_KERNEL_MATERN32: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN32>(a, st);
+      case GPBLUR_KERNEL_MATERN52: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN52>(a, st);
+      default: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_RBF>(a, st);
+    }
+  }
 }
 
 template <int DP>

@@ -3,6 +3,7 @@
 // kernels; /root/reference/denoising_model/DeepGP.py:56-73,94-99 via VariationalStrategy.forward):
 //
 //   stage A  k[n, m]  = os * exp(-1/2 |x~_n - z~_m|^2)          norm expansion, FP32 FFMA, Z~ tiles staged
+//            (Matern kinds: os f(r) of the same d2, gpblur_common.cuh: matern_kg)
 //   stage B  a[n, :]  = Linv k[n, :]                             block-triangular GEMM, K resident in smem
 //   epilogue mean = a.m + x.w + b ; var = max(os + jitter + sum (s^2-1) a^2, 1e-6) ;
 //            sample = mean + sqrt(var) * PhiloxNormal(seed, offset + n)
@@ -13,7 +14,7 @@ namespace gpblur {
 
 namespace {
 
-template <class Cfg>
+template <class Cfg, int KIND>
 __global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kernel(PointFwdArgs a) {
   constexpr int PT = Cfg::PT, CT = Cfg::CT, CW = Cfg::CW, TN = Cfg::TN;
   extern __shared__ __align__(16) float smem[];
@@ -80,7 +81,13 @@ __global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kern
         for (int f = 0; f < CT; ++f) {
           const int m = mc + Cfg::col(tx, f);
           const float d2 = fmaxf(xn + zn[m] - 2.0f * acc[e][f], 0.f);
-          kv[f] = (m < M) ? os * expf(-0.5f * d2) : 0.f;
+          if constexpr (KIND == GPBLUR_KERNEL_RBF) {
+            kv[f] = (m < M) ? os * expf(-0.5f * d2) : 0.f;
+          } else {
+            float g;
+            matern_kg<KIND>(d2, os, kv[f], g);
+            if (m >= M) kv[f] = 0.f;
+          }
         }
         *reinterpret_cast<float4*>(Ks + (size_t)n * ldk + mc + tx * 4) = make_float4(kv[0], kv[1], kv[2], kv[3]);
         if (CT == 8)
@@ -161,22 +168,38 @@ size_t fwd_smem_bytes(const WsLayout& L) {
                           4 * Cfg::TN);
 }
 
-template <class Cfg>
-int launch_fwd_cfg(const PointFwdArgs& a0, cudaStream_t st) {
+template <class Cfg, int KIND>
+int launch_fwd_kind(const PointFwdArgs& a0, cudaStream_t st) {
   PointFwdArgs a = a0;
   const size_t smem = fwd_smem_bytes<Cfg>(a.L);
-  cudaFuncSetAttribute(point_fwd_kernel<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
+  cudaFuncSetAttribute(point_fwd_kernel<Cfg, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
   a.ntiles = (int)((a.L.N + Cfg::TN - 1) / Cfg::TN);
   int occ = 1;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, point_fwd_kernel<Cfg>, kThreads, smem);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, point_fwd_kernel<Cfg, KIND>, kThreads, smem);
   if (occ < 1) occ = 1;
   int grid = occ * num_sms();
   if (grid > a.ntiles) grid = a.ntiles;
   if (grid < 1) grid = 1;
   ProfScope ps(ST_POINT_FWD, st);
-  point_fwd_kernel<Cfg><<<grid, kThreads, smem, st>>>(a);
+  point_fwd_kernel<Cfg, KIND><<<grid, kThreads, smem, st>>>(a);
   note_launch();
   return check_launch("point_fwd");
+}
+
+template <class Cfg>
+int launch_fwd_cfg(const PointFwdArgs& a, cudaStream_t st) {
+  // the Matern kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
+  if constexpr (Cfg::CW != 32) {
+    if (a.L.kind != GPBLUR_KERNEL_RBF) return GPBLUR_EUNSUPPORTED;
+    return launch_fwd_kind<Cfg, GPBLUR_KERNEL_RBF>(a, st);
+  } else {
+    switch (a.L.kind) {
+      case GPBLUR_KERNEL_MATERN12: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN12>(a, st);
+      case GPBLUR_KERNEL_MATERN32: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN32>(a, st);
+      case GPBLUR_KERNEL_MATERN52: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN52>(a, st);
+      default: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_RBF>(a, st);
+    }
+  }
 }
 
 constexpr size_t kSmemCap = 220 * 1024;

@@ -5,6 +5,8 @@
 //   g_x1[i, d] = -sum_j W_ij (x1_id - x2_jd) / l_d^2          g_x2[j, d] = +sum_i W_ij (x1_id - x2_jd) / l_d^2
 //   g_l_d      =  sum_ij W_ij (x1_id - x2_jd)^2 / l_d^3        g_os = sum_ij W_ij / os
 // and the chain rule through softplus (sigmoid of the raw value); an isotropic kernel sums g_l over d.
+// Matern kinds: W = G o g (gpblur_common.cuh: matern_kg) in the distance gradients, and g_os = sum_ij G_ij K_ij / os
+// from a second matrix Wk = G o K.
 // Three launches: W (tile kernel, as the forward) -> row pass (g_x1, per-row lengthscale / W sums) and column pass
 // (g_x2) -> one CTA adds the per-row sums in row order (bit-deterministic).  O(n1 n2 D) work, exact-GP sizes.
 #include "gpblur_common.cuh"
@@ -17,9 +19,10 @@ __device__ __forceinline__ float softplus_f(float r) { return r > 20.f ? r : log
 __device__ __forceinline__ float sigmoid_f(float r) { return 1.0f / (1.0f + expf(-r)); }
 
 // W[i, j] = G[i, j] * os * exp(-1/2 sum_d ((x1_id - x2_jd) / l_d)^2): 16 x 16 tile per CTA, direct differences
+template <int KIND>
 __global__ void rbf_w_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n1, long long n2, int D,
                              const float* __restrict__ raw_ell, int ard, const float* __restrict__ raw_os,
-                             const float* __restrict__ g_out, float* __restrict__ W) {
+                             const float* __restrict__ g_out, float* __restrict__ W, float* __restrict__ Wk) {
   __shared__ float a[16][33], b[16][33], ie[32];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const long long i0 = (long long)blockIdx.y * 16, j0 = (long long)blockIdx.x * 16;
@@ -43,14 +46,25 @@ __global__ void rbf_w_kernel(const float* __restrict__ x1, const float* __restri
     }
   }
   const long long i = i0 + ty, j = j0 + tx;
-  if (i < n1 && j < n2) W[(size_t)i * n2 + j] = g_out[(size_t)i * n2 + j] * softplus_f(raw_os[0]) * expf(-0.5f * acc);
+  if (i < n1 && j < n2) {
+    if constexpr (KIND == GPBLUR_KERNEL_RBF) {
+      W[(size_t)i * n2 + j] = g_out[(size_t)i * n2 + j] * softplus_f(raw_os[0]) * expf(-0.5f * acc);
+    } else {
+      float k, g;
+      matern_kg<KIND>(acc, softplus_f(raw_os[0]), k, g);
+      const float go = g_out[(size_t)i * n2 + j];
+      W[(size_t)i * n2 + j] = go * g;
+      Wk[(size_t)i * n2 + j] = go * k;
+    }
+  }
 }
 
 // one CTA per row i of x1: threads = dimensions (d < D <= 128), loop over j.
-//   g_x1[i, d] ; rowstat[i, d] = sum_j W_ij (x1_id - x2_jd)^2 ; rowstat[i, D] = sum_j W_ij   (double)
+//   g_x1[i, d] ; rowstat[i, d] = sum_j W_ij (x1_id - x2_jd)^2 ; rowstat[i, D] = sum_j Wos_ij   (double)
+//   (Wos: W for RBF, Wk for the Matern kinds)
 __global__ void rbf_row_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n2, int D,
                                const float* __restrict__ raw_ell, int ard, const float* __restrict__ W,
-                               float* __restrict__ g_x1, double* __restrict__ rowstat) {
+                               const float* __restrict__ Wos, float* __restrict__ g_x1, double* __restrict__ rowstat) {
   const long long i = blockIdx.x;
   const int d = threadIdx.x;
   const float* wr = W + (size_t)i * n2;
@@ -66,8 +80,9 @@ __global__ void rbf_row_kernel(const float* __restrict__ x1, const float* __rest
     if (g_x1) g_x1[(size_t)i * D + d] = (float)(-s1 / ((double)ell * ell));
     rowstat[(size_t)i * (D + 1) + d] = s2;
   } else if (d == D) {
+    const float* wo = Wos + (size_t)i * n2;
     double s = 0.0;
-    for (long long j = 0; j < n2; ++j) s += (double)wr[j];
+    for (long long j = 0; j < n2; ++j) s += (double)wo[j];
     rowstat[(size_t)i * (D + 1) + D] = s;
   }
 }
@@ -119,9 +134,54 @@ __global__ void rbf_finish_kernel(const double* __restrict__ rowstat, long long 
 
 using namespace gpblur;
 
+extern "C" size_t gpblur_covariance_backward_scratch_bytes(long long n1, long long n2, int D, int kind) {
+  if (n1 < 0 || n2 < 0 || D < 1 || !kernel_kind_valid(kind)) return 0;
+  const size_t wb = align_up((size_t)n1 * (size_t)n2 * 4);
+  return (kind == GPBLUR_KERNEL_RBF ? wb : 2 * wb) + (size_t)n1 * (size_t)(D + 1) * 8;
+}
+
 extern "C" size_t gpblur_rbf_covariance_backward_scratch_bytes(long long n1, long long n2, int D) {
-  if (n1 < 0 || n2 < 0 || D < 1) return 0;
-  return align_up((size_t)n1 * (size_t)n2 * 4) + (size_t)n1 * (size_t)(D + 1) * 8;
+  return gpblur_covariance_backward_scratch_bytes(n1, n2, D, GPBLUR_KERNEL_RBF);
+}
+
+extern "C" int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                                          const float* raw_lengthscale, int ard, const float* raw_outputscale,
+                                          const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
+                                          float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream) {
+  if (n1 < 1 || n2 < 1 || D < 1 || D > GPBLUR_MAX_D || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
+  if (!x1 || !x2 || !raw_lengthscale || !raw_outputscale || !g_out || !g_raw_lengthscale || !g_raw_outputscale || !scratch)
+    return GPBLUR_EINVAL;
+  if ((reinterpret_cast<uintptr_t>(scratch) & 255) ||
+      scratch_bytes < gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind))
+    return GPBLUR_EWORKSPACE;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const size_t wb = align_up((size_t)n1 * (size_t)n2 * 4);
+  const bool rbf = kind == GPBLUR_KERNEL_RBF;
+  float* W = static_cast<float*>(scratch);
+  float* Wk = rbf ? W : reinterpret_cast<float*>(static_cast<char*>(scratch) + wb);
+  double* rowstat = reinterpret_cast<double*>(static_cast<char*>(scratch) + (rbf ? wb : 2 * wb));
+  const int threads = round_up(D + 1, 32);
+  ProfScope ps(ST_OTHER, st);
+  dim3 grid((unsigned)((n2 + 15) / 16), (unsigned)((n1 + 15) / 16));
+  switch (kind) {
+    case GPBLUR_KERNEL_MATERN12:
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      break;
+    case GPBLUR_KERNEL_MATERN32:
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      break;
+    case GPBLUR_KERNEL_MATERN52:
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      break;
+    default:
+      rbf_w_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+  }
+  rbf_row_kernel<<<(unsigned)n1, threads, 0, st>>>(x1, x2, n2, D, raw_lengthscale, ard, W, Wk, g_x1, rowstat);
+  if (g_x2) rbf_col_kernel<<<(unsigned)n2, threads, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, W, g_x2);
+  rbf_finish_kernel<<<1, threads, 0, st>>>(rowstat, n1, D, raw_lengthscale, ard, raw_outputscale, g_raw_lengthscale,
+                                           g_raw_outputscale);
+  note_launch(g_x2 ? 4 : 3);
+  return check_launch("rbf_cov_backward");
 }
 
 extern "C" int gpblur_rbf_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D,
@@ -129,22 +189,6 @@ extern "C" int gpblur_rbf_covariance_backward(const float* x1, const float* x2, 
                                               const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
                                               float* g_raw_outputscale, void* scratch, size_t scratch_bytes,
                                               void* stream) {
-  if (n1 < 1 || n2 < 1 || D < 1 || D > GPBLUR_MAX_D) return GPBLUR_EINVAL;
-  if (!x1 || !x2 || !raw_lengthscale || !raw_outputscale || !g_out || !g_raw_lengthscale || !g_raw_outputscale || !scratch)
-    return GPBLUR_EINVAL;
-  if ((reinterpret_cast<uintptr_t>(scratch) & 255) || scratch_bytes < gpblur_rbf_covariance_backward_scratch_bytes(n1, n2, D))
-    return GPBLUR_EWORKSPACE;
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  float* W = static_cast<float*>(scratch);
-  double* rowstat = reinterpret_cast<double*>(static_cast<char*>(scratch) + align_up((size_t)n1 * (size_t)n2 * 4));
-  const int threads = round_up(D + 1, 32);
-  ProfScope ps(ST_OTHER, st);
-  dim3 grid((unsigned)((n2 + 15) / 16), (unsigned)((n1 + 15) / 16));
-  rbf_w_kernel<<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W);
-  rbf_row_kernel<<<(unsigned)n1, threads, 0, st>>>(x1, x2, n2, D, raw_lengthscale, ard, W, g_x1, rowstat);
-  if (g_x2) rbf_col_kernel<<<(unsigned)n2, threads, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, W, g_x2);
-  rbf_finish_kernel<<<1, threads, 0, st>>>(rowstat, n1, D, raw_lengthscale, ard, raw_outputscale, g_raw_lengthscale,
-                                           g_raw_outputscale);
-  note_launch(g_x2 ? 4 : 3);
-  return check_launch("rbf_cov_backward");
+  return gpblur_covariance_backward(x1, x2, n1, n2, D, GPBLUR_KERNEL_RBF, raw_lengthscale, ard, raw_outputscale, g_out,
+                                    g_x1, g_x2, g_raw_lengthscale, g_raw_outputscale, scratch, scratch_bytes, stream);
 }

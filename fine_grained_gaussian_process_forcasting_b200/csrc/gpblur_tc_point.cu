@@ -370,7 +370,15 @@ constexpr int kMaxFwdSlabs = 20 * 8;   // MP = 1024: 20 passes x (4 d-slabs + 4 
 // parity = A stage), so the latency chain of a slab (TMEM load -> exp -> stage acquire -> tcgen05.st -> arrive) has
 // two slab times; warp 16 issues.  Accumulator chunk c is read out (mean / variance partials, A saved for the
 // backward) by group c & 1 as soon as the issuer's commit on chunk[c] says that its last slab has retired.
-template <int BQ, int BWO, int NSTB>
+// Matern epilogue of a cross-covariance element.  t = min(log2e (S + xnc' + znc'), log2 os) = log2 os - 1/2 log2e d2
+// is the RBF exponent (RBF: k = 2^t).  The Matern kinds recover d2 = 2 ln2 (log2 os - t) >= 0 and evaluate k = os f and
+// g through matern_kg; a padded column (znc = -1e30) gives d2 ~ 1e30 and exactly k = g = 0.
+template <int KIND>
+__device__ __forceinline__ void tc_kg(float t, float l2os, float os, float& k, float& g) {
+  matern_kg<KIND>((l2os - t) * 1.3862943611198906f, os, k, g);
+}
+
+template <int BQ, int BWO, int NSTB, int KIND>
 __global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) Bars bars;
@@ -627,10 +635,18 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) {
 #pragma unroll
               for (int j = 0; j < 16; j += 4) {
                 const float4 z4 = ldg4(znq + col0 + j);
-                v[j + 0] = tc::ex2_approx(fminf(fmaf(v[j + 0], 1.4426950408889634f, xnc + z4.x), l2os));
-                v[j + 1] = tc::ex2_approx(fminf(fmaf(v[j + 1], 1.4426950408889634f, xnc + z4.y), l2os));
-                v[j + 2] = tc::ex2_approx(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os));
-                v[j + 3] = tc::ex2_approx(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os));
+                if constexpr (KIND == GPBLUR_KERNEL_RBF) {
+                  v[j + 0] = tc::ex2_approx(fminf(fmaf(v[j + 0], 1.4426950408889634f, xnc + z4.x), l2os));
+                  v[j + 1] = tc::ex2_approx(fminf(fmaf(v[j + 1], 1.4426950408889634f, xnc + z4.y), l2os));
+                  v[j + 2] = tc::ex2_approx(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os));
+                  v[j + 3] = tc::ex2_approx(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os));
+                } else {
+                  float g;
+                  tc_kg<KIND>(fminf(fmaf(v[j + 0], 1.4426950408889634f, xnc + z4.x), l2os), l2os, os, v[j + 0], g);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 1], 1.4426950408889634f, xnc + z4.y), l2os), l2os, os, v[j + 1], g);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os), l2os, os, v[j + 2], g);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os), l2os, os, v[j + 3], g);
+                }
               }
               if (ptr) ptr[2] = clock64() + (long long)(v[0] == 12345.f);
               // s_full (a commit: every earlier MMA has retired) already covers the stages of the first two slabs
@@ -771,7 +787,7 @@ __device__ __forceinline__ int warp_reduce16_index(int lane) {
   return ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1);
 }
 
-template <int BT, int DXW, int NSTA, int NSTB>
+template <int BT, int DXW, int NSTA, int NSTB, int KIND>
 __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) BwdBars bb;
@@ -933,7 +949,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
       }
     } else {
       // =================== row owners ===================
-      const float l2os = log2f(hyp[H_OS]);
+      const float os = hyp[H_OS], l2os = log2f(os);
       const uint32_t tmem_s = tmem_base + lane_base + S_COL, tmem_t = tmem_base + lane_base + T_COL;
       const uint32_t tmem_dx = tmem_base + lane_base + DX_COL;
       const int et = tid - kGroup;                        // thread index within the group
@@ -946,6 +962,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
 #pragma unroll
       for (int i = 0; i < NPIECE; ++i) { qacc[i] = 0.f; tacc[i] = 0.f; }
       float s_gm = 0.f, s_r = 0.f, s_gv = 0.f;           // scalar sums (k-half 0 threads)
+      float s_kbk = 0.f;                                  // sum kbar o k of the Matern kinds (every thread)
       uint32_t cnt = 0;                                   // W slabs produced so far (private stage NSTA - 1)
       // x rows of a tile go global -> shared memory with cp.async (coalesced: 16 bytes per thread and request, no
       // registers), one tile ahead: issued after the previous tile's dx epilogue, awaited at the tile head
@@ -1033,17 +1050,33 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
             const float* zp = znc_s + p * BT + col;
             const float* bp = beta_s + p * BT + col;
             const float gv2 = 2.0f * gv;
+            if constexpr (KIND == GPBLUR_KERNEL_RBF) {
 #pragma unroll
-            for (int i = 0; i < 16; i += 4) {
-              const float4 z4 = *reinterpret_cast<const float4*>(zp + i), b4 = *reinterpret_cast<const float4*>(bp + i);
-              const float k0 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 0]), 1.4426950408889634f, xnc + z4.x), l2os));
-              const float k1 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 1]), 1.4426950408889634f, xnc + z4.y), l2os));
-              const float k2 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 2]), 1.4426950408889634f, xnc + z4.z), l2os));
-              const float k3 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 3]), 1.4426950408889634f, xnc + z4.w), l2os));
-              w[i + 0] = fmaf(gv2, __uint_as_float(tr[i + 0]), gm * b4.x) * k0;
-              w[i + 1] = fmaf(gv2, __uint_as_float(tr[i + 1]), gm * b4.y) * k1;
-              w[i + 2] = fmaf(gv2, __uint_as_float(tr[i + 2]), gm * b4.z) * k2;
-              w[i + 3] = fmaf(gv2, __uint_as_float(tr[i + 3]), gm * b4.w) * k3;
+              for (int i = 0; i < 16; i += 4) {
+                const float4 z4 = *reinterpret_cast<const float4*>(zp + i), b4 = *reinterpret_cast<const float4*>(bp + i);
+                const float k0 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 0]), 1.4426950408889634f, xnc + z4.x), l2os));
+                const float k1 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 1]), 1.4426950408889634f, xnc + z4.y), l2os));
+                const float k2 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 2]), 1.4426950408889634f, xnc + z4.z), l2os));
+                const float k3 = tc::ex2_approx(fminf(fmaf(__uint_as_float(kr[i + 3]), 1.4426950408889634f, xnc + z4.w), l2os));
+                w[i + 0] = fmaf(gv2, __uint_as_float(tr[i + 0]), gm * b4.x) * k0;
+                w[i + 1] = fmaf(gv2, __uint_as_float(tr[i + 1]), gm * b4.y) * k1;
+                w[i + 2] = fmaf(gv2, __uint_as_float(tr[i + 2]), gm * b4.z) * k2;
+                w[i + 3] = fmaf(gv2, __uint_as_float(tr[i + 3]), gm * b4.w) * k3;
+              }
+            } else {
+#pragma unroll
+              for (int i = 0; i < 16; i += 4) {
+                const float4 z4 = *reinterpret_cast<const float4*>(zp + i), b4 = *reinterpret_cast<const float4*>(bp + i);
+                const float zz[4] = {z4.x, z4.y, z4.z, z4.w}, bb4[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                  float k, g;
+                  tc_kg<KIND>(fminf(fmaf(__uint_as_float(kr[i + e]), 1.4426950408889634f, xnc + zz[e]), l2os), l2os, os, k, g);
+                  const float kb = fmaf(gv2, __uint_as_float(tr[i + e]), gm * bb4[e]);
+                  w[i + e] = kb * g;
+                  s_kbk = fmaf(kb, k, s_kbk);
+                }
+              }
             }
 #pragma unroll
             for (int i = 0; i < 16; ++i) rsum += w[i];
@@ -1133,7 +1166,8 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
       }
       {
         const float sg = warp_sum(s_gm), sr = warp_sum(s_r), sv = warp_sum(s_gv);
-        if (lane == 0) { sc_s[ew][VS_GMU] = sg; sc_s[ew][VS_RSUM] = sr; sc_s[ew][VS_GVAR] = sv; sc_s[ew][3] = 0.f; }
+        const float sk = KIND == GPBLUR_KERNEL_RBF ? 0.f : warp_sum(s_kbk);
+        if (lane == 0) { sc_s[ew][VS_GMU] = sg; sc_s[ew][VS_RSUM] = sr; sc_s[ew][VS_GVAR] = sv; sc_s[ew][VS_KBK] = sk; }
       }
       asm volatile("bar.sync 2, 256;" ::: "memory");
       float* vp = vecpart + (size_t)blockIdx.x * L.vec_len;
@@ -1153,6 +1187,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
       if (et < VS_COUNT) {
         float sum = 0.f;
         if (et < 3) for (int w = 0; w < 4; ++w) sum += sc_s[w][et];
+        else if (KIND != GPBLUR_KERNEL_RBF) for (int w = 0; w < 8; ++w) sum += sc_s[w][et];   // VS_KBK: both k-halves
         vp[MP + 2 * DP + et] = sum;
       }
     }
@@ -1174,21 +1209,41 @@ void set_smem(K kernel, size_t bytes) {
   cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
+template <int BQ, int BWO, int NSTB, int KIND>
+void launch_fwd_kind(const Tc2Args& a, int grid, cudaStream_t st) {
+  const size_t smem = (size_t)NSTB * BWO * 256 + (size_t)(3 * a.L.MP + 3 * a.L.DP) * sizeof(float);
+  set_smem(tc2_fwd_kernel<BQ, BWO, NSTB, KIND>, smem);
+  tc2_fwd_kernel<BQ, BWO, NSTB, KIND><<<grid, kCtaThreads, smem, st>>>(a);
+}
+
 template <int BQ, int BWO, int NSTB>
 int launch_fwd(const Tc2Args& a, int grid, cudaStream_t st) {
-  const size_t smem = (size_t)NSTB * BWO * 256 + (size_t)(3 * a.L.MP + 3 * a.L.DP) * sizeof(float);
-  set_smem(tc2_fwd_kernel<BQ, BWO, NSTB>, smem);
-  tc2_fwd_kernel<BQ, BWO, NSTB><<<grid, kCtaThreads, smem, st>>>(a);
+  switch (a.L.kind) {
+    case GPBLUR_KERNEL_MATERN12: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN12>(a, grid, st); break;
+    case GPBLUR_KERNEL_MATERN32: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN32>(a, grid, st); break;
+    case GPBLUR_KERNEL_MATERN52: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN52>(a, grid, st); break;
+    default: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_RBF>(a, grid, st);
+  }
   return 0;
+}
+
+template <int BT, int DXW, int NSTA, int NSTB, int KIND>
+void launch_bwd_kind(const Tc2Args& a, int grid, cudaStream_t st) {
+  constexpr size_t brows = BT > DXW ? BT : DXW;
+  const size_t smem = (size_t)NSTB * brows * 256 +
+                      (size_t)(2 * a.L.MP + 3 * DXW + TNP * (DXW + 4) + 8 * 32 * 20) * sizeof(float);
+  set_smem(tc2_bwd_kernel<BT, DXW, NSTA, NSTB, KIND>, smem);
+  tc2_bwd_kernel<BT, DXW, NSTA, NSTB, KIND><<<grid, kCtaThreads, smem, st>>>(a);
 }
 
 template <int BT, int DXW, int NSTA, int NSTB>
 int launch_bwd(const Tc2Args& a, int grid, cudaStream_t st) {
-  constexpr size_t brows = BT > DXW ? BT : DXW;
-  const size_t smem = (size_t)NSTB * brows * 256 +
-                      (size_t)(2 * a.L.MP + 3 * DXW + TNP * (DXW + 4) + 8 * 32 * 20) * sizeof(float);
-  set_smem(tc2_bwd_kernel<BT, DXW, NSTA, NSTB>, smem);
-  tc2_bwd_kernel<BT, DXW, NSTA, NSTB><<<grid, kCtaThreads, smem, st>>>(a);
+  switch (a.L.kind) {
+    case GPBLUR_KERNEL_MATERN12: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN12>(a, grid, st); break;
+    case GPBLUR_KERNEL_MATERN32: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN32>(a, grid, st); break;
+    case GPBLUR_KERNEL_MATERN52: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN52>(a, grid, st); break;
+    default: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_RBF>(a, grid, st);
+  }
   return 0;
 }
 

@@ -175,12 +175,19 @@ class RBFKernel(Kernel):
 
 
 class MaternKernel(Kernel):
-    """Imported (unused) by the reference at DeepGP.py:7; the CUDA path implements RBF only."""
+    """gpytorch's MaternKernel (imported by the reference at DeepGP.py:7): nu in {0.5, 1.5, 2.5}, evaluated by the same
+    CUDA kernels as RBFKernel (include/gpblur.h: GPBLUR_KERNEL_MATERN*)."""
     has_lengthscale = True
 
     def __init__(self, nu=2.5, **kwargs):
+        if nu not in {0.5, 1.5, 2.5}:
+            raise RuntimeError("nu expected to be 0.5, 1.5, or 2.5")
         super().__init__(**kwargs)
         self.nu = nu
+
+    @property
+    def kernel_name(self):
+        return {0.5: "matern12", 1.5: "matern32", 2.5: "matern52"}[self.nu]
 
 
 class ScaleKernel(Kernel):
@@ -197,27 +204,35 @@ class ScaleKernel(Kernel):
         return self.raw_outputscale_constraint.transform(self.raw_outputscale)
 
     def forward(self, x1, x2=None):
-        """Dense ScaleKernel(RBF) covariance by the CUDA kernel, differentiable w.r.t. the inputs and both raw
-        hyper-parameters (hand-written backward: gpblur_rbf_covariance_backward)."""
+        """Dense ScaleKernel(RBF | Matern) covariance by the CUDA kernel, differentiable w.r.t. the inputs and both raw
+        hyper-parameters (hand-written backward: gpblur_covariance_backward)."""
         x2 = x1 if x2 is None else x2
         bk = self.base_kernel
-        if not isinstance(bk, RBFKernel) or len(self.batch_shape):
-            raise NotImplementedError("dense covariance: un-batched ScaleKernel(RBFKernel) only")
+        if not isinstance(bk, (RBFKernel, MaternKernel)) or len(self.batch_shape):
+            raise NotImplementedError("dense covariance: un-batched ScaleKernel(RBFKernel | MaternKernel) only")
+        kernel = _base_kernel_name(bk)
         lead = x1.shape[:-2]
         x1f = x1.reshape(-1, x1.shape[-2], x1.shape[-1])
         x2f = x2.reshape(-1, x2.shape[-2], x2.shape[-1])
         same = x2 is x1
-        outs = [ops.rbf_covariance(a, a if same else b, bk.raw_lengthscale, self.raw_outputscale, bk.ard_num_dims is not None)
+        outs = [ops.rbf_covariance(a, a if same else b, bk.raw_lengthscale, self.raw_outputscale, bk.ard_num_dims is not None,
+                                   kernel=kernel)
                 for a, b in zip(x1f, x2f)]
         return torch.stack(outs).reshape(*lead, x1.shape[-2], x2.shape[-2])
 
 
+def _base_kernel_name(base_kernel):
+    return "rbf" if isinstance(base_kernel, RBFKernel) else base_kernel.kernel_name
+
+
 def _kernel_raw_params(covar_module):
-    """(raw_lengthscale, raw_outputscale, ard) of a ScaleKernel(RBFKernel) - anything else is unsupported."""
-    if not isinstance(covar_module, ScaleKernel) or not isinstance(covar_module.base_kernel, RBFKernel):
-        raise NotImplementedError("the CUDA GP path implements ScaleKernel(RBFKernel(ard_num_dims=D)) "
+    """(raw_lengthscale, raw_outputscale, kernel name) of a ScaleKernel(RBFKernel | MaternKernel) - anything else is
+    unsupported.  The name is what ops.svgp_predict takes as `kernel`."""
+    if not isinstance(covar_module, ScaleKernel) or not isinstance(covar_module.base_kernel, (RBFKernel, MaternKernel)):
+        raise NotImplementedError("the CUDA GP path implements ScaleKernel(RBFKernel | MaternKernel(ard_num_dims=D)) "
                                   "(DeepGP.py:46-49); got %r" % type(covar_module).__name__)
-    return covar_module.base_kernel.raw_lengthscale, covar_module.raw_outputscale
+    bk = covar_module.base_kernel
+    return bk.raw_lengthscale, covar_module.raw_outputscale, _base_kernel_name(bk)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -507,7 +522,7 @@ class DeepGPLayer(ApproximateGP):
         its batched parameters ([H, M, D] inducing points ...) and is evaluated by ONE batched op."""
         vs = self.variational_strategy
         vd = vs._variational_distribution
-        raw_ell, raw_os = _kernel_raw_params(self.covar_module)
+        raw_ell, raw_os, _ = _kernel_raw_params(self.covar_module)
         Z, m, s = vs.inducing_points, vd.variational_mean, vd._variational_stddev
         mm = self.mean_module
         if isinstance(mm, LinearMean):
@@ -518,12 +533,16 @@ class DeepGPLayer(ApproximateGP):
             raise NotImplementedError("mean module %r" % type(mm).__name__)
         return Z, raw_ell, raw_os, m, s, w, b
 
+    def _kernel(self):
+        return _kernel_raw_params(self.covar_module)[2]
+
     def _stage_cache(self):
         return self._stage_caches.setdefault(None, {}) if self.share_param_stage else None
 
     def _kl_only(self):
         _, kl, _, _ = ops.svgp_param_stage(*self._layer_params(), stage_cache=self._stage_cache(),
-                                           check=bool(check_cholesky.value()), grad_sink=self._grad_sink)
+                                           check=bool(check_cholesky.value()), grad_sink=self._grad_sink,
+                                           kernel=self._kernel())
         return kl.sum() if kl.dim() else kl
 
     def __call__(self, inputs, are_samples=False, **kwargs):
@@ -549,7 +568,7 @@ class DeepGPLayer(ApproximateGP):
                                                        stage_cache=self._stage_cache(),
                                                        offset_dev=self.rng_offset_dev, h_stride=self._rng_h_stride,
                                                        check=bool(check_cholesky.value()),
-                                                       grad_sink=self._grad_sink)
+                                                       grad_sink=self._grad_sink, kernel=self._kernel())
         self.last_info = info
         if H is None:
             cls = MultivariateNormal
@@ -580,7 +599,8 @@ class DeepGPLayer(ApproximateGP):
         segs, kl, info = ops.svgp_predict_segments(x_flat, seg_shapes, *self._layer_params(), seed, off, stream,
                                                    want_sample=self.fused_sample, stage_cache=self._stage_cache(),
                                                    offset_dev=self.rng_offset_dev,
-                                                   check=bool(check_cholesky.value()), grad_sink=self._grad_sink)
+                                                   check=bool(check_cholesky.value()), grad_sink=self._grad_sink,
+                                                   kernel=self._kernel())
         self.last_info = info
         vs._cache_kl(kl)
         S = num_likelihood_samples.value()

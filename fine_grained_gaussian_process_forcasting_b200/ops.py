@@ -216,34 +216,42 @@ def philox_normal(seed: int, offset: int, n: int, stream_id: int = 0, device="cu
     return out
 
 
-def _rbf_covariance_raw(x1, x2, raw_lengthscale, raw_outputscale, ard: bool) -> Tensor:
+def kernel_kind(kernel: str) -> int:
+    """Covariance function name ("rbf", "matern12", "matern32", "matern52") -> GPBLUR_KERNEL_* kind."""
+    kind = _cabi.KERNEL_KINDS.get(kernel)
+    if kind is None:
+        raise ValueError(f"unknown covariance function {kernel!r}: expected one of {sorted(_cabi.KERNEL_KINDS)}")
+    return kind
+
+
+def _rbf_covariance_raw(x1, x2, raw_lengthscale, raw_outputscale, ard: bool, kind: int = 0) -> Tensor:
     n1, D = x1.shape
     n2 = x2.shape[0]
     out = torch.empty(n1, n2, device=x1.device, dtype=torch.float32)
     with torch.cuda.device(x1.device):
-        rc = _cabi.lib().gpblur_rbf_covariance(_ptr(x1), _ptr(x2), n1, n2, D, _ptr(raw_lengthscale),
-                                               int(ard), _ptr(raw_outputscale), _ptr(out), _stream())
-    _cabi.check(rc, "gpblur_rbf_covariance")
+        rc = _cabi.lib().gpblur_covariance(_ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(raw_lengthscale),
+                                           int(ard), _ptr(raw_outputscale), _ptr(out), _stream())
+    _cabi.check(rc, "gpblur_covariance")
     return out
 
 
 class _RbfCovFunction(torch.autograd.Function):
-    """Dense ScaleKernel(RBF) covariance with its hand-written backward (gpblur_rbf_covariance_backward): gradients of
-    the inputs, the raw lengthscale(s) and the raw outputscale."""
+    """Dense ScaleKernel(RBF | Matern) covariance with its hand-written backward (gpblur_covariance_backward):
+    gradients of the inputs, the raw lengthscale(s) and the raw outputscale."""
 
     @staticmethod
-    def forward(ctx, x1, x2, raw_lengthscale, raw_outputscale, ard):
+    def forward(ctx, x1, x2, raw_lengthscale, raw_outputscale, ard, kind=0):
         same = x2 is x1
         x1c, ellc, osc = _f32c(x1), _f32c(raw_lengthscale).reshape(-1), _f32c(raw_outputscale).reshape(-1)
         x2c = x1c if same else _f32c(x2)
         ctx.save_for_backward(x1c, x2c, ellc, osc)
-        ctx.meta = (bool(ard), same, raw_lengthscale.shape, raw_outputscale.shape)
-        return _rbf_covariance_raw(x1c, x2c, ellc, osc, ard)
+        ctx.meta = (bool(ard), same, raw_lengthscale.shape, raw_outputscale.shape, int(kind))
+        return _rbf_covariance_raw(x1c, x2c, ellc, osc, ard, kind)
 
     @staticmethod
     def backward(ctx, g_out):
         x1, x2, ell, os_ = ctx.saved_tensors
-        ard, same, ell_shape, os_shape = ctx.meta
+        ard, same, ell_shape, os_shape, kind = ctx.meta
         n1, D = x1.shape
         n2 = x2.shape[0]
         dev = x1.device
@@ -253,26 +261,28 @@ class _RbfCovFunction(torch.autograd.Function):
         g_x2 = torch.empty(n2, D, device=dev, dtype=torch.float32) if want_x2 else None
         g_ell = torch.empty(D if ard else 1, device=dev, dtype=torch.float32)
         g_os = torch.empty(1, device=dev, dtype=torch.float32)
-        nbytes = int(_cabi.lib().gpblur_rbf_covariance_backward_scratch_bytes(n1, n2, D))
+        nbytes = int(_cabi.lib().gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind))
         scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
         with torch.cuda.device(dev):
-            rc = _cabi.lib().gpblur_rbf_covariance_backward(_ptr(x1), _ptr(x2), n1, n2, D, _ptr(ell), int(ard), _ptr(os_),
-                                                            _ptr(_f32c(g_out)), _ptr(g_x1), _ptr(g_x2), _ptr(g_ell),
-                                                            _ptr(g_os), _ptr(scratch), nbytes, _stream())
-        _cabi.check(rc, "gpblur_rbf_covariance_backward")
+            rc = _cabi.lib().gpblur_covariance_backward(_ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(ell), int(ard),
+                                                        _ptr(os_), _ptr(_f32c(g_out)), _ptr(g_x1), _ptr(g_x2),
+                                                        _ptr(g_ell), _ptr(g_os), _ptr(scratch), nbytes, _stream())
+        _cabi.check(rc, "gpblur_covariance_backward")
         if same:                       # K(x, x): the one tensor is both arguments
             gx = g_x1 + g_x2 if (need[0] or need[1]) else None
-            return gx if need[0] else None, None, g_ell.reshape(ell_shape), g_os.reshape(os_shape), None
+            return gx if need[0] else None, None, g_ell.reshape(ell_shape), g_os.reshape(os_shape), None, None
         return (g_x1 if need[0] else None, g_x2 if need[1] else None, g_ell.reshape(ell_shape), g_os.reshape(os_shape),
-                None)
+                None, None)
 
 
-def rbf_covariance(x1: Tensor, x2: Tensor, raw_lengthscale: Tensor, raw_outputscale: Tensor, ard: bool) -> Tensor:
-    """os * exp(-1/2 |(x1 - x2) / l|^2) [n1, n2]; differentiable w.r.t. x1, x2 and both raw hyper-parameters."""
+def rbf_covariance(x1: Tensor, x2: Tensor, raw_lengthscale: Tensor, raw_outputscale: Tensor, ard: bool,
+                   kernel: str = "rbf") -> Tensor:
+    """os * f(|(x1 - x2) / l|) [n1, n2] (f: exp(-d^2 / 2) for "rbf", the Matern functions of include/gpblur.h for
+    "matern12" / "matern32" / "matern52"); differentiable w.r.t. x1, x2 and both raw hyper-parameters."""
     _need_cuda(x1, x2, raw_lengthscale, raw_outputscale)
     if raw_lengthscale.numel() != (x1.shape[-1] if ard else 1):
         raise ValueError("rbf_covariance: raw_lengthscale must hold D values (ard) or one")
-    return _RbfCovFunction.apply(x1, x2, raw_lengthscale, raw_outputscale, bool(ard))
+    return _RbfCovFunction.apply(x1, x2, raw_lengthscale, raw_outputscale, bool(ard), kernel_kind(kernel))
 
 
 def debug_fetch(which: int, N: int, D: int, M: int, ws: Tensor) -> Tensor:
@@ -307,11 +317,13 @@ def stage_grad_doubles(D: int, M: int) -> int:
     return int(_cabi.lib().gpblur_svgp_stage_grad_doubles(D, M))
 
 
-def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: float = 0.0, max_ctas: int = 0):
+def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: float = 0.0, max_ctas: int = 0,
+                    kind: int = 0):
     """Once-per-parameter-update M x M stage: -> (stage uint8 [param_stage_bytes], kl [1], info [1] int32).
     `out` = preallocated (stage, kl, info) (the call then only launches on the current stream).
     `extra_jitter` is added to the diagonal of Kzz on top of the variational jitter (psd_safe_cholesky retries).
-    `max_ctas` > 0 bounds the cooperative grid (stages of a multi-output layer running side by side, see _Fork)."""
+    `max_ctas` > 0 bounds the cooperative grid (stages of a multi-output layer running side by side, see _Fork).
+    `kind`: covariance function (kernel_kind); the point and backward calls on this stage must pass the same."""
     _need_cuda(Z, raw_ell, raw_os, m, s, w, b)
     M, D = Z.shape
     dev = Z.device
@@ -327,7 +339,10 @@ def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: floa
         stage, kl, info = out
     p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
     with torch.cuda.device(dev):
-        if max_ctas:
+        if kind:
+            rc = _cabi.lib().gpblur_svgp_param_stage_kind(C.byref(p), D, M, int(kind), float(extra_jitter), int(max_ctas),
+                                                          _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
+        elif max_ctas:
             rc = _cabi.lib().gpblur_svgp_param_stage_shared_sms(C.byref(p), D, M, float(extra_jitter), int(max_ctas),
                                                                 _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
         elif extra_jitter:
@@ -342,7 +357,7 @@ def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: floa
 
 def point_forward_raw(stage: Tensor, x: Tensor, M: int, seed: int, offset: int, stream_id: int, want_sample: bool,
                       training: bool, out: Optional[Tensor] = None, offset_dev: Optional[Tensor] = None,
-                      ws: Optional[Tensor] = None):
+                      ws: Optional[Tensor] = None, kind: int = 0):
     """x [N, D] + parameter stage -> (mean [N], var [N], sample [N] | None, workspace uint8).
     `out`: preallocated float32 [(3 | 2) * N] receiving mean | var | sample."""
     _need_cuda(x, stage)
@@ -356,17 +371,19 @@ def point_forward_raw(stage: Tensor, x: Tensor, M: int, seed: int, offset: int, 
         ws = torch.empty(workspace_bytes(N, D, M, training), device=dev, dtype=torch.uint8)
     with torch.cuda.device(dev):
         # "_shared": the kernels read the stage in place (no device-to-device copy of it into `ws`)
-        rc = _cabi.lib().gpblur_svgp_point_forward_shared(
-            _ptr(stage), _ptr(x), N, D, M, _ptr(mean), _ptr(var), _ptr(sample),
-            seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev),
-            int(training), _ptr(ws), ws.numel(), _stream())
+        tail = (_ptr(mean), _ptr(var), _ptr(sample), seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF,
+                stream_id & 0xFFFFFFFF, _ptr(offset_dev), int(training), _ptr(ws), ws.numel(), _stream())
+        if kind:
+            rc = _cabi.lib().gpblur_svgp_point_forward_shared_kind(_ptr(stage), _ptr(x), N, D, M, int(kind), *tail)
+        else:
+            rc = _cabi.lib().gpblur_svgp_point_forward_shared(_ptr(stage), _ptr(x), N, D, M, *tail)
     _cabi.check(rc, "gpblur_svgp_point_forward_shared")
     return mean, var, sample, ws
 
 
 def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, offset, stream_id, ws,
                        need_dx: bool = True, dx: Optional[Tensor] = None, sgrad: Optional[Tensor] = None,
-                       offset_dev: Optional[Tensor] = None, stage: Optional[Tensor] = None):
+                       offset_dev: Optional[Tensor] = None, stage: Optional[Tensor] = None, kind: int = 0):
     """-> (dx [N, D] | None, stage_grad float64 [stage_grad_doubles(D, M)]).
     `stage`: the parameter stage the matching point_forward_raw call read (None: the stage was built in `ws` itself by
     svgp_forward_raw)."""
@@ -377,6 +394,16 @@ def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, of
         dx = torch.empty(N, D, device=dev, dtype=torch.float32)
     if sgrad is None:
         sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
+    if kind:               # the kind-taking point backward is the segments form: one segment
+        keep = [None if t is None else _f32c(t) for t in (g_mean, g_var, g_sample)]
+        ptrs = [(C.c_void_p * 1)(_ptr(t)) for t in keep]
+        with torch.cuda.device(dev):
+            rc = _cabi.lib().gpblur_svgp_point_backward_segments_kind(
+                _ptr(stage), _ptr(x), N, D, M, int(kind), 1, (C.c_longlong * 1)(0), *ptrs, _ptr(var),
+                seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev),
+                _ptr(dx if need_dx else None), _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
+        _cabi.check(rc, "gpblur_svgp_point_backward_segments_kind")
+        return (dx if need_dx else None), sgrad
     with torch.cuda.device(dev):
         args = (_ptr(x), N, D, M, _ptr(g_mean), _ptr(g_var), _ptr(g_sample), _ptr(var),
                 seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev),
@@ -391,7 +418,7 @@ def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, of
 
 def point_backward_segments_raw(x: Tensor, M: int, seg_sizes, g_means, g_vars, g_samples, var, seed, offset, stream_id,
                                 ws, need_dx: bool = True, offset_dev: Optional[Tensor] = None,
-                                stage: Optional[Tensor] = None):
+                                stage: Optional[Tensor] = None, kind: int = 0):
     """point_backward_raw with the upstream gradients given per segment of the point range (lists of tensors or None,
     one entry per segment, indexed from the start of the segment) -> (dx [N, D] | None, stage_grad)."""
     _need_cuda(x, ws, var)
@@ -412,16 +439,20 @@ def point_backward_segments_raw(x: Tensor, M: int, seg_sizes, g_means, g_vars, g
     dx = torch.empty(N, D, device=dev, dtype=torch.float32) if need_dx else None
     sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
     with torch.cuda.device(dev):
-        rc = _cabi.lib().gpblur_svgp_point_backward_segments(
-            _ptr(stage), _ptr(x), N, D, M, nseg, (C.c_longlong * nseg)(*starts), ptr_array(gm), ptr_array(gv),
-            ptr_array(gs), _ptr(var), seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF,
-            _ptr(offset_dev), _ptr(dx), _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
+        tail = (nseg, (C.c_longlong * nseg)(*starts), ptr_array(gm), ptr_array(gv), ptr_array(gs), _ptr(var),
+                seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev), _ptr(dx),
+                _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
+        if kind:
+            rc = _cabi.lib().gpblur_svgp_point_backward_segments_kind(_ptr(stage), _ptr(x), N, D, M, int(kind), *tail)
+        else:
+            rc = _cabi.lib().gpblur_svgp_point_backward_segments(_ptr(stage), _ptr(x), N, D, M, *tail)
     _cabi.check(rc, "gpblur_svgp_point_backward_segments")
     return dx, sgrad
 
 
 def param_stage_backward_raw(Z, raw_ell, raw_os, m, s, w, b, sgrad: Tensor, g_kl: Optional[Tensor], stage: Tensor,
-                             bucket: Optional[Tensor] = None, accumulate: bool = False, max_ctas: int = 0):
+                             bucket: Optional[Tensor] = None, accumulate: bool = False, max_ctas: int = 0,
+                             kind: int = 0):
     """Summed stage gradient (+ g_kl) -> flat parameter-gradient bucket [M*D + 2M + 2D + 2] (`accumulate`: added to
     `bucket` instead of overwriting it)."""
     _need_cuda(Z, sgrad, stage, g_kl)
@@ -430,7 +461,11 @@ def param_stage_backward_raw(Z, raw_ell, raw_os, m, s, w, b, sgrad: Tensor, g_kl
         bucket = torch.empty(grad_bucket_floats(D, M), device=Z.device, dtype=torch.float32)
     p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
     with torch.cuda.device(Z.device):
-        if max_ctas:
+        if kind:
+            rc = _cabi.lib().gpblur_svgp_param_stage_backward_kind(
+                C.byref(p), D, M, int(kind), _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas),
+                _ptr(stage), stage.numel(), _stream())
+        elif max_ctas:
             rc = _cabi.lib().gpblur_svgp_param_stage_backward_shared_sms(
                 C.byref(p), D, M, _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas), _ptr(stage),
                 stage.numel(), _stream())
@@ -550,7 +585,8 @@ class _ParamStageFunction(torch.autograd.Function):
                 fork.enter(h)
                 param_stage_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h], None if wc is None else wc[h % wc.shape[0]],
                                 bc[h % bc.shape[0]], out=(stage[h], kl[h:h + 1], info[h:h + 1]),
-                                extra_jitter=float(holder.get("extra_jitter", 0.0)), max_ctas=cap)
+                                extra_jitter=float(holder.get("extra_jitter", 0.0)), max_ctas=cap,
+                                kind=holder.get("kind", 0))
         finally:
             fork.join()
         holder["stage"] = stage
@@ -589,7 +625,8 @@ class _ParamStageFunction(torch.autograd.Function):
             # the caller's flat gradient buffer holds this layer's parameters contiguously in bucket order
             # (distributed.FlatGradBucket): the kernel accumulates straight into it, autograd gets no gradient to add
             param_stage_backward_raw(Zc[0], ellc[0], osc[0], mc[0], sc[0], wc[0], bc[0], sgrad[0],
-                                     None if gk is None else gk[0:1], stage[0], bucket=sink, accumulate=True)
+                                     None if gk is None else gk[0:1], stage[0], bucket=sink, accumulate=True,
+                                     kind=holder.get("kind", 0))
             holder["consumed"] = True
             return (None,) * 8
         bucket = torch.empty(H, nb, device=dev, dtype=torch.float32)
@@ -600,7 +637,8 @@ class _ParamStageFunction(torch.autograd.Function):
                 fork.enter(h)
                 param_stage_backward_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h],
                                          None if wc is None else wc[h % wc.shape[0]], bc[h % bc.shape[0]], sgrad[h],
-                                         None if gk is None else gk[h:h + 1], stage[h], bucket=bucket[h], max_ctas=cap)
+                                         None if gk is None else gk[h:h + 1], stage[h], bucket=bucket[h], max_ctas=cap,
+                                         kind=holder.get("kind", 0))
         finally:
             fork.join()
         holder["consumed"] = True        # the graph behind this token is gone: the next forward rebuilds the stage
@@ -654,12 +692,13 @@ class _PointFunction(torch.autograd.Function):
             for h in range(H):
                 fork.enter(h)
                 point_forward_raw(stage[h], x2, M, seed, offset + h * hs, stream_id, want_sample, training,
-                                  out=out[h], offset_dev=offset_dev, ws=wss[h])
+                                  out=out[h], offset_dev=offset_dev, ws=wss[h], kind=holder.get("kind", 0))
         finally:
             fork.join()
         if training:
             ctx.save_for_backward(x2, out, *wss)
             ctx.stage = stage                                  # read in place by the backward kernels
+            ctx.kind = holder.get("kind", 0)
         ctx.meta = (seed, offset, stream_id, M, shape, H, batched, nout, hs)
         ctx.offset_dev = offset_dev
         ctx.set_materialize_grads(False)
@@ -701,7 +740,7 @@ class _PointFunction(torch.autograd.Function):
                 point_backward_raw(x2, M, None if gm is None else gm[h], None if gv is None else gv[h],
                                    None if gs is None else gs[h], out[h, N:2 * N], seed, offset + h * hs, stream_id,
                                    wss[h], need_dx=need[0], dx=None if dx is None else dx[h], sgrad=sgrad[h],
-                                   offset_dev=ctx.offset_dev, stage=ctx.stage[h])
+                                   offset_dev=ctx.offset_dev, stage=ctx.stage[h], kind=ctx.kind)
         finally:
             fork.join()
         if dx is not None:
@@ -732,22 +771,26 @@ JITTER_RETRIES = (1e-6, 1e-5, 1e-4)
 def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outputscale: Tensor,
                      variational_mean: Tensor, variational_stddev: Tensor, mean_weights: Optional[Tensor],
                      mean_bias: Tensor, stage_cache: Optional[dict] = None, check: bool = False,
-                     grad_sink: Optional[Tensor] = None):
-    """-> (token, kl, info, holder).  With `stage_cache` (a dict owned by the caller, one per GP layer) consecutive
+                     grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
+    """-> (token, kl, info, holder).  `kernel`: covariance function ("rbf", "matern12", "matern32", "matern52"); it
+    is part of the stage-cache key and travels in `holder` to every call on the stage.  With `stage_cache` (a dict owned by the caller, one per GP layer) consecutive
     calls with unchanged parameter tensors (same `_version`) share one stage - and therefore one M x M backward -
     until a backward pass has consumed it.  Parameters with a leading H (inducing points [H, M, D]) describe the H
     independent GPs of a multi-output layer: kl is [H], token [H, G]."""
     params = (inducing_points, raw_lengthscale, raw_outputscale, variational_mean, variational_stddev, mean_weights,
               mean_bias)
     want_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in params)
+    kind = kernel_kind(kernel)
     key = None
     if stage_cache is not None:
-        key = _stage_key(*params)
+        key = _stage_key(*params) + (kind,)
         ent = stage_cache.get("entry")
         if ent is not None and stage_cache.get("key") == key and not ent[3]["consumed"] \
                 and ent[0].requires_grad == want_grad:
             return ent
     holder = {} if grad_sink is None else {"grad_sink": grad_sink}
+    if kind:
+        holder["kind"] = kind
     with torch.cuda.nvtx.range("gpblur.param_stage") if _NVTX else _null_ctx():
         token, kl, info = _ParamStageFunction.apply(*params, holder)
     # Cholesky status (LAPACK-style info, 0 = ok).  Reading it synchronises with the device, as gpytorch's
@@ -760,6 +803,8 @@ def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outpu
                 holder = {"extra_jitter": jit}
                 if grad_sink is not None:
                     holder["grad_sink"] = grad_sink
+                if kind:
+                    holder["kind"] = kind
                 token, kl, info = _ParamStageFunction.apply(*params, holder)
                 if int(info.max().item()) == 0:
                     warnings.warn(f"Kzz + 1e-4 I is not positive definite (pivot {k}): added jitter of {jit:.1e} to the "
@@ -780,15 +825,16 @@ def svgp_predict(x: Tensor, inducing_points: Tensor, raw_lengthscale: Tensor, ra
                  mean_bias: Tensor, seed: int = 0, offset: int = 0, stream_id: int = 0,
                  want_sample: bool = False, stage_cache: Optional[dict] = None,
                  offset_dev: Optional[Tensor] = None, h_stride: Optional[int] = None, check: bool = False,
-                 grad_sink: Optional[Tensor] = None):
+                 grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
     """x [..., D] -> (mean [...], var [...], sample [...] | None, kl [], info [1]); with inducing points [H, M, D]
     (multi-output layer) the outputs are [..., H], kl [H], info [H], and GP h draws its sample with Philox counters
     offset + h * h_stride + n (h_stride defaults to the N points of this call; batch-sharded callers pass the GLOBAL
     point count so that the counters do not depend on the number of ranks).  `stage_cache`: see svgp_param_stage.  `offset_dev`: optional int64 device scalar added to
-    `offset` when the kernels run (CUDA-graph replays draw fresh counters by bumping it between replays)."""
+    `offset` when the kernels run (CUDA-graph replays draw fresh counters by bumping it between replays).  `kernel`:
+    covariance function, see svgp_param_stage."""
     token, kl, info, holder = svgp_param_stage(inducing_points, raw_lengthscale, raw_outputscale, variational_mean,
                                                variational_stddev, mean_weights, mean_bias, stage_cache, check=check,
-                                               grad_sink=grad_sink)
+                                               grad_sink=grad_sink, kernel=kernel)
     if x.numel() == 0:
         shp = tuple(x.shape[:-1]) + ((token.shape[0],) if token.dim() == 2 else ())
         e = x.new_empty(shp, dtype=torch.float32)
@@ -835,10 +881,11 @@ class _PointSegFunction(torch.autograd.Function):
         stage = holder["stage"]
         ws = torch.empty(workspace_bytes(N, D, M, training), device=x2.device, dtype=torch.uint8)
         point_forward_raw(stage[0], x2, M, seed, offset, stream_id, want_sample, training, out=out,
-                          offset_dev=offset_dev, ws=ws)
+                          offset_dev=offset_dev, ws=ws, kind=holder.get("kind", 0))
         if training:
             ctx.save_for_backward(x2, out, ws)
             ctx.stage = stage
+            ctx.kind = holder.get("kind", 0)
         ctx.meta = (seed, offset, stream_id, M, tuple(x.shape), sizes, nout)
         ctx.offset_dev = offset_dev
         ctx.set_materialize_grads(False)
@@ -858,7 +905,8 @@ class _PointSegFunction(torch.autograd.Function):
         gms, gvs, gss = list(grads[0::3]), list(grads[1::3]), list(grads[2::3])
         with torch.cuda.nvtx.range("gpblur.point_backward") if _NVTX else _null_ctx():
             dx, sgrad = point_backward_segments_raw(x2, M, sizes, gms, gvs, gss, out[N:2 * N], seed, offset, stream_id, ws,
-                                                    need_dx=need[0], offset_dev=ctx.offset_dev, stage=ctx.stage[0])
+                                                    need_dx=need[0], offset_dev=ctx.offset_dev, stage=ctx.stage[0],
+                                                    kind=ctx.kind)
         return (dx.reshape(xshape) if dx is not None else None, sgrad if need[1] else None) + (None,) * 8
 
 
@@ -867,7 +915,7 @@ def svgp_predict_segments(x: Tensor, seg_shapes, inducing_points: Tensor, raw_le
                           mean_weights: Optional[Tensor], mean_bias: Tensor, seed: int = 0, offset: int = 0,
                           stream_id: int = 0, want_sample: bool = False, stage_cache: Optional[dict] = None,
                           offset_dev: Optional[Tensor] = None, check: bool = False,
-                          grad_sink: Optional[Tensor] = None):
+                          grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
     """svgp_predict for a single-output GP on x [N, D] = the concatenated points of several activations;
     ``seg_shapes`` (e.g. [(B, 192), (B, 24)]) are the output shapes of the segments, in order.
     -> ([(mean, var, sample | None) per segment], kl, info)."""
@@ -875,7 +923,7 @@ def svgp_predict_segments(x: Tensor, seg_shapes, inducing_points: Tensor, raw_le
         raise ValueError("svgp_predict_segments: single-output layers only")
     token, kl, info, holder = svgp_param_stage(inducing_points, raw_lengthscale, raw_outputscale, variational_mean,
                                                variational_stddev, mean_weights, mean_bias, stage_cache, check=check,
-                                               grad_sink=grad_sink)
+                                               grad_sink=grad_sink, kernel=kernel)
     with torch.cuda.nvtx.range("gpblur.point_forward") if _NVTX else _null_ctx():
         flat = _PointSegFunction.apply(x, token, holder, int(inducing_points.shape[-2]), int(seed), int(offset),
                                        int(stream_id), bool(want_sample), offset_dev,

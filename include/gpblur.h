@@ -36,6 +36,19 @@ extern "C" {
 #define GPBLUR_MAX_D 128
 #define GPBLUR_MAX_M 1024
 
+/* Covariance function of a layer (the `kind` argument of the *_kind entry points below).  With x~ = (x - c) / ell,
+ * d2 = |x~ - z~|^2 and r = sqrt(max(d2, 1e-30)) (gpytorch's covar_dist), k = os f:
+ *   RBF         f = exp(-d2 / 2)                         (every entry point without a kind argument)
+ *   MATERN12    f = exp(-r)                              (gpytorch MaternKernel(nu=0.5))
+ *   MATERN32    f = (1 + sqrt3 r) exp(-sqrt3 r)          (nu=1.5)
+ *   MATERN52    f = (1 + sqrt5 r + 5/3 r^2) exp(-sqrt5 r) (nu=2.5)
+ * A parameter stage must be consumed (point forward / backward, stage backward) with the kind it was built with;
+ * nothing on the device checks this. */
+#define GPBLUR_KERNEL_RBF 0
+#define GPBLUR_KERNEL_MATERN12 1
+#define GPBLUR_KERNEL_MATERN32 2
+#define GPBLUR_KERNEL_MATERN52 3
+
 /* Parameters of one whitened sparse variational GP layer.
  * Replaces the parameter set created by ToyDeepGPHiddenLayer.__init__
  * (/root/reference/denoising_model/DeepGP.py:15-49) for output_dims=None. */
@@ -175,6 +188,26 @@ int gpblur_svgp_param_stage_backward_shared_sms(const gpblur_svgp_params* p, int
                                                 const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
                                                 void* stage, size_t stage_bytes, void* stream);
 
+/* The entry points above with the covariance function as `kind` (GPBLUR_KERNEL_*; an unknown kind returns
+ * GPBLUR_EINVAL).  The plain entry points are these with GPBLUR_KERNEL_RBF.  `param_stage` of the point calls may be
+ * null when the stage lives in `ws` (as for gpblur_svgp_point_backward_segments). */
+int gpblur_svgp_param_stage_kind(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter,
+                                 int max_ctas, float* kl, int* info, void* stage, size_t stage_bytes, void* stream);
+int gpblur_svgp_param_stage_backward_kind(const gpblur_svgp_params* p, int D, int M, int kind,
+                                          const double* stage_grad, const float* g_kl, float* grad_bucket,
+                                          int accumulate, int max_ctas, void* stage, size_t stage_bytes, void* stream);
+int gpblur_svgp_point_forward_shared_kind(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                                          float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
+                                          uint32_t stream_id, const unsigned long long* offset_dev, int training,
+                                          void* ws, size_t ws_bytes, void* stream);
+int gpblur_svgp_point_backward_segments_kind(const void* param_stage, const float* x, long long N, int D, int M,
+                                             int kind, int nseg, const long long* seg_start,
+                                             const float* const* g_mean, const float* const* g_var,
+                                             const float* const* g_sample, const float* var, uint64_t seed,
+                                             uint64_t offset, uint32_t stream_id,
+                                             const unsigned long long* offset_dev, float* dx, double* stage_grad,
+                                             void* ws, size_t ws_bytes, void* stream);
+
 /* `stage` is the buffer filled by gpblur_svgp_param_stage; its fp64 scratch regions are overwritten. */
 int gpblur_svgp_param_stage_backward(const gpblur_svgp_params* p, int D, int M,
                                      const double* stage_grad, const float* g_kl,
@@ -236,6 +269,15 @@ int gpblur_rbf_covariance_backward(const float* x1, const float* x2, long long n
                                    const float* raw_lengthscale, int ard, const float* raw_outputscale,
                                    const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
                                    float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream);
+/* The dense covariance and its backward for any GPBLUR_KERNEL_* `kind` (the rbf entry points are these with
+ * GPBLUR_KERNEL_RBF).  The backward's scratch: gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind). */
+int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                      const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream);
+size_t gpblur_covariance_backward_scratch_bytes(long long n1, long long n2, int D, int kind);
+int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                               const float* raw_lengthscale, int ard, const float* raw_outputscale,
+                               const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
+                               float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream);
 
 /* Debug / test probes into the workspace of the last forward on (ws): copies device-to-device.
  * which: 0 = L (fp64 [Mp,Mp]), 1 = Linv (fp64 [Mp,Mp]), 2 = Kzz+jitter (fp64 [Mp,Mp]),
