@@ -49,55 +49,24 @@ SIGNATURES = {
         C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
         C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_svgp_param_stage_bytes": (C.c_size_t, [C.c_int, C.c_int]),
-    "gpblur_svgp_forward_cached": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_void_p, C.c_longlong, C.c_int, C.c_int,
-        C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
-        C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "gpblur_svgp_backward": (C.c_int, [
         C.POINTER(SvgpParams), C.c_void_p, C.c_longlong, C.c_int, C.c_int,
         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_svgp_stage_grad_doubles": (C.c_size_t, [C.c_int, C.c_int]),
     "gpblur_svgp_param_stage": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_param_stage_jitter": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-        C.c_void_p]),
-    "gpblur_svgp_param_stage_shared_sms": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-        C.c_void_p]),
-    "gpblur_svgp_param_stage_backward_shared_sms": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
-        C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_forward": (C.c_int, [
-        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-        C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_backward": (C.c_int, [
-        C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-        C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_forward_shared": (C.c_int, [
-        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-        C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_backward_shared": (C.c_int, [
-        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-        C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_backward_segments": (C.c_int, [
-        C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-        C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-        C.c_void_p]),
-    "gpblur_svgp_param_stage_kind": (C.c_int, [
         C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_param_stage_backward_kind": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
-        C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_forward_shared_kind": (C.c_int, [
+    "gpblur_svgp_point_forward": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
-    "gpblur_svgp_point_backward_segments_kind": (C.c_int, [
+    "gpblur_svgp_point_backward": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_size_t, C.c_void_p]),
+    "gpblur_svgp_param_stage_backward": (C.c_int, [
+        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+        C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_covariance": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
         C.c_void_p, C.c_void_p]),
@@ -134,22 +103,12 @@ SIGNATURES = {
                                                    C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                                    C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gpblur_rbf_covariance_backward_scratch_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong, C.c_int]),
-    "gpblur_rbf_covariance_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_void_p,
-                                                 C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                 C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_peer_comm_bytes": (C.c_size_t, [C.c_longlong]),
     "gpblur_peer_alloc": (C.c_int, [C.c_size_t, C.c_void_p, C.c_void_p]),
     "gpblur_peer_open": (C.c_int, [C.c_void_p, C.c_void_p]),
     "gpblur_peer_close": (C.c_int, [C.c_void_p]),
     "gpblur_peer_free": (C.c_int, [C.c_void_p]),
     "gpblur_peer_allreduce": (C.c_int, [C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_float, C.c_void_p]),
-    "gpblur_svgp_param_stage_backward": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-        C.c_void_p]),
-    "gpblur_svgp_param_stage_backward_acc": (C.c_int, [
-        C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t,
-        C.c_void_p]),
     "gpblur_elbo_forward": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float,
         C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]),
@@ -166,9 +125,6 @@ SIGNATURES = {
     "gpblur_rsample_backward": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_uint64, C.c_uint64, C.c_uint32,
         C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gpblur_rbf_covariance": (C.c_int, [
-        C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
-        C.c_void_p, C.c_void_p]),
     "gpblur_debug_fetch": (C.c_int, [
         C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
         C.POINTER(C.c_int), C.c_void_p]),

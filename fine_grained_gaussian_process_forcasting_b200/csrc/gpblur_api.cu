@@ -37,25 +37,6 @@ ProfScope::~ProfScope() {
   g_prof_recs.push_back(r);
 }
 
-static thread_local const unsigned long long* g_offset_dev = nullptr;
-const unsigned long long* current_offset_dev() { return g_offset_dev; }
-static thread_local const void* g_param_stage = nullptr;
-const void* current_param_stage() { return g_param_stage; }
-static thread_local SegGrads g_seg_grads = {};
-SegGrads current_seg_grads() { return g_seg_grads; }
-struct SegGradsScope {
-  explicit SegGradsScope(const SegGrads& s) { g_seg_grads = s; }
-  ~SegGradsScope() { g_seg_grads = SegGrads{}; }
-};
-struct ParamStageScope {
-  explicit ParamStageScope(const void* p) { g_param_stage = p; }
-  ~ParamStageScope() { g_param_stage = nullptr; }
-};
-struct OffsetDevScope {
-  explicit OffsetDevScope(const unsigned long long* p) { g_offset_dev = p; }
-  ~OffsetDevScope() { g_offset_dev = nullptr; }
-};
-
 static std::atomic<long long*> g_trace{nullptr};
 long long* debug_trace_buffer() { return g_trace.load(std::memory_order_relaxed); }
 
@@ -319,10 +300,12 @@ inline int ew_grid(long long n, int block) { return (int)((n + block - 1) / bloc
 
 }  // namespace
 
-int dispatch_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var, float* sample,
-                           uint64_t seed, uint64_t offset, uint32_t stream_id, cudaStream_t st) {
-  if (tc_point_supported(L)) return launch_tc_point_forward(L, ws, x, mean, var, sample, seed, offset, stream_id, st);
-  return launch_point_forward(L, ws, x, mean, var, sample, seed, offset, stream_id, st);
+int dispatch_point_forward(const WsLayout& L, const void* stage, void* ws, const float* x, float* mean, float* var,
+                           float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                           const unsigned long long* offset_dev, cudaStream_t st) {
+  if (tc_point_supported(L))
+    return launch_tc_point_forward(L, stage, ws, x, mean, var, sample, seed, offset, stream_id, offset_dev, st);
+  return launch_point_forward(L, stage, ws, x, mean, var, sample, seed, offset, stream_id, offset_dev, st);
 }
 
 int launch_stage_grad_reduce(const WsLayout& L, const void* ws, double* sgrad, cudaStream_t st) {
@@ -334,11 +317,6 @@ int launch_stage_grad_reduce(const WsLayout& L, const void* ws, double* sgrad, c
 
 using namespace gpblur;
 
-namespace gpblur {
-int dispatch_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var, float* sample,
-                           uint64_t seed, uint64_t offset, uint32_t stream_id, cudaStream_t st);
-}
-
 extern "C" {
 
 size_t gpblur_svgp_grad_bucket_floats(int D, int M) { return (size_t)M * D + 2 * (size_t)M + 2 * (size_t)D + 2; }
@@ -348,13 +326,44 @@ size_t gpblur_svgp_workspace_bytes(long long N, int D, int M, int training) {
   return make_layout(N, D, M, training).total;
 }
 
+static bool aligned256(const void* p) { return p && !(reinterpret_cast<uintptr_t>(p) & 255); }
+
+static int check_shape(long long N, int D, int M) {
+  if (N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
+  return (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) ? GPBLUR_EUNSUPPORTED : GPBLUR_OK;
+}
+
 static int validate(const gpblur_svgp_params* p, long long N, int D, int M) {
-  if (!p || N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
-  if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
+  if (!p) return GPBLUR_EINVAL;
+  const int rc = check_shape(N, D, M);
+  if (rc) return rc;
   if (!p->inducing_points || !p->raw_lengthscale || !p->raw_outputscale || !p->variational_mean ||
       !p->variational_stddev || !p->mean_bias)
     return GPBLUR_EINVAL;
   return GPBLUR_OK;
+}
+
+// Arguments of the M x M stage and of its backward: parameters, kind and the stage buffer.  Fills the stage layout.
+static int check_stage(const gpblur_svgp_params* p, int D, int M, int kind, const void* stage, size_t stage_bytes,
+                       WsLayout* L) {
+  const int rc = validate(p, 0, D, M);
+  if (rc) return rc;
+  if (!kernel_kind_valid(kind) || !aligned256(stage)) return GPBLUR_EINVAL;
+  *L = make_layout(0, D, M, 0);
+  L->kind = kind;
+  return stage_bytes < L->total ? GPBLUR_EWORKSPACE : GPBLUR_OK;
+}
+
+// Arguments of the point forward and backward: shape, kind, the stage they read and the workspace.  Fills the layout
+// of the call.
+static int check_point(const void* stage, long long N, int D, int M, int kind, int training, const void* ws,
+                       size_t ws_bytes, WsLayout* L) {
+  const int rc = check_shape(N, D, M);
+  if (rc) return rc;
+  if (!kernel_kind_valid(kind) || !aligned256(stage) || !aligned256(ws)) return GPBLUR_EINVAL;
+  *L = make_layout(N, D, M, training);
+  L->kind = kind;
+  return ws_bytes < L->total ? GPBLUR_EWORKSPACE : GPBLUR_OK;
 }
 
 int gpblur_svgp_forward(const gpblur_svgp_params* p, const float* x, long long N, int D, int M, float* mean,
@@ -363,14 +372,14 @@ int gpblur_svgp_forward(const gpblur_svgp_params* p, const float* x, long long N
   int rc = validate(p, N, D, M);
   if (rc) return rc;
   if (N > 0 && (!x || !mean || !var)) return GPBLUR_EINVAL;
-  if (!ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
+  if (!aligned256(ws)) return GPBLUR_EINVAL;
   const WsLayout L = make_layout(N, D, M, training ? 1 : 0);
   if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   rc = launch_mm_forward(*p, L, ws, kl, info, st);
   if (rc) return rc;
   if (N == 0) return GPBLUR_OK;
-  return dispatch_point_forward(L, ws, x, mean, var, sample, seed, offset, stream_id, st);
+  return dispatch_point_forward(L, ws, ws, x, mean, var, sample, seed, offset, stream_id, nullptr, st);
 }
 
 size_t gpblur_svgp_param_stage_bytes(int D, int M) {
@@ -383,249 +392,70 @@ size_t gpblur_svgp_stage_grad_doubles(int D, int M) {
   return stage_grad_doubles(padded_m(M), padded_d(D));
 }
 
-int gpblur_svgp_param_stage(const gpblur_svgp_params* p, int D, int M, float* kl, int* info, void* stage,
-                            size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
+int gpblur_svgp_param_stage(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter, int max_ctas,
+                            float* kl, int* info, void* stage, size_t stage_bytes, void* stream) {
+  WsLayout L;
+  const int rc = check_stage(p, D, M, kind, stage, stage_bytes, &L);
   if (rc) return rc;
-  if (!stage || (reinterpret_cast<uintptr_t>(stage) & 255)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream);
-}
-
-int gpblur_svgp_param_stage_jitter(const gpblur_svgp_params* p, int D, int M, double extra_jitter, float* kl, int* info,
-                                   void* stage, size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
-  if (rc) return rc;
-  if (!stage || (reinterpret_cast<uintptr_t>(stage) & 255) || !(extra_jitter >= 0.0)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream, extra_jitter);
-}
-
-int gpblur_svgp_param_stage_shared_sms(const gpblur_svgp_params* p, int D, int M, double extra_jitter, int max_ctas,
-                                       float* kl, int* info, void* stage, size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
-  if (rc) return rc;
-  if (!stage || (reinterpret_cast<uintptr_t>(stage) & 255) || !(extra_jitter >= 0.0) || max_ctas < 0) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
+  if (!(extra_jitter >= 0.0) || max_ctas < 0) return GPBLUR_EINVAL;
   return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream, extra_jitter, max_ctas);
 }
 
-int gpblur_svgp_param_stage_kind(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter,
-                                 int max_ctas, float* kl, int* info, void* stage, size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
+int gpblur_svgp_param_stage_backward(const gpblur_svgp_params* p, int D, int M, int kind, const double* stage_grad,
+                                     const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
+                                     void* stage, size_t stage_bytes, void* stream) {
+  WsLayout L;
+  const int rc = check_stage(p, D, M, kind, stage, stage_bytes, &L);
   if (rc) return rc;
-  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
-  if (!stage || (reinterpret_cast<uintptr_t>(stage) & 255) || !(extra_jitter >= 0.0) || max_ctas < 0) return GPBLUR_EINVAL;
-  WsLayout L = make_layout(0, D, M, 0);
-  L.kind = kind;
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_forward(*p, L, stage, kl, info, (cudaStream_t)stream, extra_jitter, max_ctas);
+  if (!stage_grad || !grad_bucket || max_ctas < 0) return GPBLUR_EINVAL;
+  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream, accumulate ? 1 : 0,
+                            max_ctas);
 }
 
-int gpblur_svgp_param_stage_backward_kind(const gpblur_svgp_params* p, int D, int M, int kind,
-                                          const double* stage_grad, const float* g_kl, float* grad_bucket,
-                                          int accumulate, int max_ctas, void* stage, size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
+int gpblur_svgp_point_forward(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                              float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
+                              uint32_t stream_id, const unsigned long long* offset_dev, int training, void* ws,
+                              size_t ws_bytes, void* stream) {
+  WsLayout L;
+  const int rc = check_point(param_stage, N, D, M, kind, training ? 1 : 0, ws, ws_bytes, &L);
   if (rc) return rc;
-  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
-  if (!stage_grad || !grad_bucket || !stage || (reinterpret_cast<uintptr_t>(stage) & 255) || max_ctas < 0) return GPBLUR_EINVAL;
-  WsLayout L = make_layout(0, D, M, 0);
-  L.kind = kind;
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream, accumulate ? 1 : 0, max_ctas);
+  if (N == 0) return GPBLUR_OK;
+  if (!x || !mean || !var) return GPBLUR_EINVAL;
+  return dispatch_point_forward(L, param_stage, ws, x, mean, var, sample, seed, offset, stream_id, offset_dev,
+                                (cudaStream_t)stream);
 }
 
-int gpblur_svgp_param_stage_backward_shared_sms(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
-                                                const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
-                                                void* stage, size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
+int gpblur_svgp_point_backward(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                               int nseg, const long long* seg_start, const float* const* g_mean,
+                               const float* const* g_var, const float* const* g_sample, const float* var,
+                               uint64_t seed, uint64_t offset, uint32_t stream_id, const unsigned long long* offset_dev,
+                               float* dx, double* stage_grad, void* ws, size_t ws_bytes, void* stream) {
+  const void* stage = param_stage ? param_stage : ws;
+  WsLayout L;
+  int rc = check_point(stage, N, D, M, kind, 1, ws, ws_bytes, &L);
   if (rc) return rc;
-  if (!stage_grad || !grad_bucket || !stage || (reinterpret_cast<uintptr_t>(stage) & 255) || max_ctas < 0) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream, accumulate ? 1 : 0, max_ctas);
-}
-
-int gpblur_svgp_point_forward(const void* param_stage, const float* x, long long N, int D, int M, float* mean,
-                              float* var, float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
-                              const unsigned long long* offset_dev, int training, void* ws, size_t ws_bytes,
-                              void* stream) {
-  OffsetDevScope ods(offset_dev);
-  if (!param_stage || N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
-  if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
-  if (N > 0 && (!x || !mean || !var)) return GPBLUR_EINVAL;
-  if (!ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(N, D, M, training ? 1 : 0);
-  if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
+  if (!stage_grad || (N > 0 && (!x || !var))) return GPBLUR_EINVAL;
+  if (nseg < 1 || nseg > kMaxSegments || !seg_start || seg_start[0] != 0) return GPBLUR_EINVAL;
+  SegGrads sg{};
+  sg.nseg = nseg;
+  for (int i = 0; i < nseg; ++i) {
+    if (seg_start[i] < 0 || seg_start[i] > N || (i > 0 && seg_start[i] < seg_start[i - 1])) return GPBLUR_EINVAL;
+    sg.start[i] = seg_start[i];
+    sg.gm[i] = g_mean ? g_mean[i] : nullptr;
+    sg.gv[i] = g_var ? g_var[i] : nullptr;
+    sg.gs[i] = g_sample ? g_sample[i] : nullptr;
+  }
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t pbytes = make_layout(0, D, M, 0).total;
-  if (param_stage != ws) cudaMemcpyAsync(ws, param_stage, pbytes, cudaMemcpyDeviceToDevice, st);
-  int rc = check_launch("param_stage_copy");
-  if (rc || N == 0) return rc;
-  return dispatch_point_forward(L, ws, x, mean, var, sample, seed, offset, stream_id, st);
-}
-
-int gpblur_svgp_forward_cached(const gpblur_svgp_params* p, const float* x, long long N, int D, int M, float* mean,
-                               float* var, float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
-                               float* kl, int* info, int training, void* ws, size_t ws_bytes,
-                               const void* param_stage, void* stream) {
-  if (!param_stage)
-    return gpblur_svgp_forward(p, x, N, D, M, mean, var, sample, seed, offset, stream_id, kl, info, training, ws,
-                               ws_bytes, stream);
-  int rc = validate(p, N, D, M);
-  if (rc) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  const WsLayout L0 = make_layout(0, D, M, 0);
-  if (kl) cudaMemcpyAsync(kl, ws_cptr<float>(param_stage, L0.hyp) + H_KL, sizeof(float), cudaMemcpyDeviceToDevice, st);
-  if (info) cudaMemsetAsync(info, 0, sizeof(int), st);
-  return gpblur_svgp_point_forward(param_stage, x, N, D, M, mean, var, sample, seed, offset, stream_id, nullptr,
-                                   training, ws, ws_bytes, stream);
-}
-
-static int point_backward_kind(const float* x, long long N, int D, int M, int kind, const float* g_mean,
-                               const float* g_var, const float* g_sample, const float* var, uint64_t seed,
-                               uint64_t offset, uint32_t stream_id, const unsigned long long* offset_dev, float* dx,
-                               double* stage_grad, void* ws, size_t ws_bytes, void* stream) {
-  OffsetDevScope ods(offset_dev);
-  if (N < 0 || D < 1 || M < 1 || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
-  if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
-  if (!stage_grad || !ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
-  if (N > 0 && (!x || !var)) return GPBLUR_EINVAL;
-  WsLayout L = make_layout(N, D, M, 1);
-  L.kind = kind;
-  if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = GPBLUR_OK;
   if (N > 0) {
     if (tc_point_supported(L))
-      rc = launch_tc_point_backward(L, ws, x, g_mean, g_var, g_sample, var, seed, offset, stream_id, dx, st);
+      rc = launch_tc_point_backward(L, stage, ws, x, sg, var, seed, offset, stream_id, offset_dev, dx, st);
     else
-      rc = launch_point_backward(L, ws, x, g_mean, g_var, g_sample, var, seed, offset, stream_id, dx, st);
+      rc = launch_point_backward(L, stage, ws, x, sg, var, seed, offset, stream_id, offset_dev, dx, st);
     if (rc) return rc;
     rc = launch_reductions(L, ws, x, st);
     if (rc) return rc;
   }
   return launch_stage_grad_reduce(L, ws, stage_grad, st);
-}
-
-int gpblur_svgp_point_backward(const float* x, long long N, int D, int M, const float* g_mean, const float* g_var,
-                               const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
-                               uint32_t stream_id, const unsigned long long* offset_dev, float* dx,
-                               double* stage_grad, void* ws, size_t ws_bytes, void* stream) {
-  return point_backward_kind(x, N, D, M, GPBLUR_KERNEL_RBF, g_mean, g_var, g_sample, var, seed, offset, stream_id,
-                             offset_dev, dx, stage_grad, ws, ws_bytes, stream);
-}
-
-int gpblur_svgp_point_forward_shared(const void* param_stage, const float* x, long long N, int D, int M, float* mean,
-                                     float* var, float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
-                                     const unsigned long long* offset_dev, int training, void* ws, size_t ws_bytes,
-                                     void* stream) {
-  return gpblur_svgp_point_forward_shared_kind(param_stage, x, N, D, M, GPBLUR_KERNEL_RBF, mean, var, sample, seed,
-                                               offset, stream_id, offset_dev, training, ws, ws_bytes, stream);
-}
-
-int gpblur_svgp_point_forward_shared_kind(const void* param_stage, const float* x, long long N, int D, int M, int kind,
-                                          float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
-                                          uint32_t stream_id, const unsigned long long* offset_dev, int training,
-                                          void* ws, size_t ws_bytes, void* stream) {
-  OffsetDevScope ods(offset_dev);
-  if (!param_stage || (reinterpret_cast<uintptr_t>(param_stage) & 255) || N < 0 || D < 1 || M < 1) return GPBLUR_EINVAL;
-  if (!kernel_kind_valid(kind)) return GPBLUR_EINVAL;
-  if (D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return GPBLUR_EUNSUPPORTED;
-  if (N > 0 && (!x || !mean || !var)) return GPBLUR_EINVAL;
-  if (!ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
-  WsLayout L = make_layout(N, D, M, training ? 1 : 0);
-  L.kind = kind;
-  if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
-  if (N == 0) return GPBLUR_OK;
-  ParamStageScope pss(param_stage);
-  return dispatch_point_forward(L, ws, x, mean, var, sample, seed, offset, stream_id, (cudaStream_t)stream);
-}
-
-int gpblur_svgp_point_backward_shared(const void* param_stage, const float* x, long long N, int D, int M,
-                                      const float* g_mean, const float* g_var, const float* g_sample, const float* var,
-                                      uint64_t seed, uint64_t offset, uint32_t stream_id,
-                                      const unsigned long long* offset_dev, float* dx, double* stage_grad, void* ws,
-                                      size_t ws_bytes, void* stream) {
-  if (!param_stage || (reinterpret_cast<uintptr_t>(param_stage) & 255)) return GPBLUR_EINVAL;
-  ParamStageScope pss(param_stage);
-  return gpblur_svgp_point_backward(x, N, D, M, g_mean, g_var, g_sample, var, seed, offset, stream_id, offset_dev, dx,
-                                    stage_grad, ws, ws_bytes, stream);
-}
-
-int gpblur_svgp_point_backward_segments_kind(const void* param_stage, const float* x, long long N, int D, int M,
-                                             int kind, int nseg, const long long* seg_start,
-                                             const float* const* g_mean, const float* const* g_var,
-                                             const float* const* g_sample, const float* var, uint64_t seed,
-                                             uint64_t offset, uint32_t stream_id,
-                                             const unsigned long long* offset_dev, float* dx, double* stage_grad,
-                                             void* ws, size_t ws_bytes, void* stream) {
-  if (nseg < 1 || nseg > kMaxSegments || !seg_start || seg_start[0] != 0) return GPBLUR_EINVAL;
-  if (param_stage && (reinterpret_cast<uintptr_t>(param_stage) & 255)) return GPBLUR_EINVAL;
-  SegGrads sg{};
-  sg.nseg = nseg;
-  for (int i = 0; i < nseg; ++i) {
-    if (seg_start[i] < 0 || seg_start[i] > N || (i > 0 && seg_start[i] < seg_start[i - 1])) return GPBLUR_EINVAL;
-    sg.start[i] = seg_start[i];
-    sg.gm[i] = g_mean ? g_mean[i] : nullptr;
-    sg.gv[i] = g_var ? g_var[i] : nullptr;
-    sg.gs[i] = g_sample ? g_sample[i] : nullptr;
-  }
-  SegGradsScope sgs(sg);
-  ParamStageScope pss(param_stage);
-  return point_backward_kind(x, N, D, M, kind, nullptr, nullptr, nullptr, var, seed, offset, stream_id, offset_dev, dx,
-                             stage_grad, ws, ws_bytes, stream);
-}
-
-int gpblur_svgp_point_backward_segments(const void* param_stage, const float* x, long long N, int D, int M, int nseg,
-                                        const long long* seg_start, const float* const* g_mean,
-                                        const float* const* g_var, const float* const* g_sample, const float* var,
-                                        uint64_t seed, uint64_t offset, uint32_t stream_id,
-                                        const unsigned long long* offset_dev, float* dx, double* stage_grad, void* ws,
-                                        size_t ws_bytes, void* stream) {
-  if (nseg < 1 || nseg > kMaxSegments || !seg_start || seg_start[0] != 0) return GPBLUR_EINVAL;
-  SegGrads sg{};
-  sg.nseg = nseg;
-  for (int i = 0; i < nseg; ++i) {
-    if (seg_start[i] < 0 || seg_start[i] > N || (i > 0 && seg_start[i] < seg_start[i - 1])) return GPBLUR_EINVAL;
-    sg.start[i] = seg_start[i];
-    sg.gm[i] = g_mean ? g_mean[i] : nullptr;
-    sg.gv[i] = g_var ? g_var[i] : nullptr;
-    sg.gs[i] = g_sample ? g_sample[i] : nullptr;
-  }
-  SegGradsScope sgs(sg);
-  // (the kernels look at the flat pointers only to decide whether a kind of gradient exists at all)
-  if (param_stage) {
-    return gpblur_svgp_point_backward_shared(param_stage, x, N, D, M, nullptr, nullptr, nullptr, var, seed, offset,
-                                             stream_id, offset_dev, dx, stage_grad, ws, ws_bytes, stream);
-  }
-  return gpblur_svgp_point_backward(x, N, D, M, nullptr, nullptr, nullptr, var, seed, offset, stream_id, offset_dev, dx,
-                                    stage_grad, ws, ws_bytes, stream);
-}
-
-int gpblur_svgp_param_stage_backward(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
-                                     const float* g_kl, float* grad_bucket, void* stage, size_t stage_bytes,
-                                     void* stream) {
-  int rc = validate(p, 0, D, M);
-  if (rc) return rc;
-  if (!stage_grad || !grad_bucket || !stage || (reinterpret_cast<uintptr_t>(stage) & 255)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream);
-}
-
-int gpblur_svgp_param_stage_backward_acc(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
-                                         const float* g_kl, float* grad_bucket, int accumulate, void* stage,
-                                         size_t stage_bytes, void* stream) {
-  int rc = validate(p, 0, D, M);
-  if (rc) return rc;
-  if (!stage_grad || !grad_bucket || !stage || (reinterpret_cast<uintptr_t>(stage) & 255)) return GPBLUR_EINVAL;
-  const WsLayout L = make_layout(0, D, M, 0);
-  if (stage_bytes < L.total) return GPBLUR_EWORKSPACE;
-  return launch_mm_backward(*p, L, stage, stage_grad, g_kl, grad_bucket, (cudaStream_t)stream, accumulate ? 1 : 0);
 }
 
 int gpblur_svgp_backward(const gpblur_svgp_params* p, const float* x, long long N, int D, int M,
@@ -634,12 +464,13 @@ int gpblur_svgp_backward(const gpblur_svgp_params* p, const float* x, long long 
                          float* grad_bucket, void* ws, size_t ws_bytes, void* stream) {
   int rc = validate(p, N, D, M);
   if (rc) return rc;
-  if (!grad_bucket || !ws || (reinterpret_cast<uintptr_t>(ws) & 255)) return GPBLUR_EINVAL;
+  if (!grad_bucket || !aligned256(ws)) return GPBLUR_EINVAL;
   const WsLayout L = make_layout(N, D, M, 1);
   if (ws_bytes < L.total) return GPBLUR_EWORKSPACE;
   double* sgrad = ws_ptr<double>(ws, L.sgrad);
-  rc = gpblur_svgp_point_backward(x, N, D, M, g_mean, g_var, g_sample, var, seed, offset, stream_id, nullptr, dx,
-                                  sgrad, ws, ws_bytes, stream);
+  const long long start = 0;
+  rc = gpblur_svgp_point_backward(nullptr, x, N, D, M, GPBLUR_KERNEL_RBF, 1, &start, &g_mean, &g_var, &g_sample, var,
+                                  seed, offset, stream_id, nullptr, dx, sgrad, ws, ws_bytes, stream);
   if (rc) return rc;
   return launch_mm_backward(*p, L, ws, sgrad, g_kl, grad_bucket, (cudaStream_t)stream);
 }
@@ -724,12 +555,6 @@ int gpblur_rsample_backward(const float* var, const float* g_out, long long n, u
   return check_launch("rsample_bwd");
 }
 
-int gpblur_rbf_covariance(const float* x1, const float* x2, long long n1, long long n2, int D,
-                          const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out,
-                          void* stream) {
-  return gpblur_covariance(x1, x2, n1, n2, D, GPBLUR_KERNEL_RBF, raw_lengthscale, ard, raw_outputscale, out, stream);
-}
-
 int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                       const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream) {
   if (n1 < 0 || n2 < 0 || D < 1 || !raw_lengthscale || !raw_outputscale || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
@@ -804,6 +629,6 @@ int gpblur_profile_collect(double* ms, unsigned long long* counts, int n) {
 
 unsigned long long gpblur_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 const char* gpblur_last_cuda_error(void) { return g_err; }
-const char* gpblur_version(void) { return "gpblur 0.1 (sm_100a)"; }
+const char* gpblur_version(void) { return "gpblur 0.2 (sm_100a)"; }
 
 }  // extern "C"

@@ -117,7 +117,7 @@ struct WsLayout {
   size_t A, W, Spart, upart, WXpart, vecpart, gsc, rrow, cpart, sgrad;
   size_t total;
   size_t D2zz64;            // fp64 inducing-pair distances d2 of the Kzz build (Matern kinds: read by the backward)
-  int kind;                 // covariance function (GPBLUR_KERNEL_*); make_layout leaves RBF, the *_kind entry points set it
+  int kind;                 // covariance function (GPBLUR_KERNEL_*); make_layout leaves RBF, the entry points set it
 };
 
 // ---- UMMA slab images of the constant operands (tensor-core path) -------------------------------------------
@@ -413,14 +413,7 @@ struct ProfScope {
   ~ProfScope();
 };
 void note_launch(int n = 1);
-// Device-resident Philox offset addend of the entry point running on this host thread (null = none).  Set by the
-// extern "C" layer around the launchers; read when the kernel arguments are filled.
-const unsigned long long* current_offset_dev();
-// Parameter stage the point kernels of the current API call read their constant operands from (thread-local, set by
-// the gpblur_svgp_point_*_shared entry points); nullptr: the stage lives in the call's own workspace.
-const void* current_param_stage();
-struct SegGrads;
-SegGrads current_seg_grads();   // per-segment upstream gradients of the current backward call (nseg == 0: none)
+// `offset_dev` (nullable): device-resident addend of the Philox offset, read when the kernel runs (CUDA-graph replays)
 __device__ __forceinline__ uint64_t rng_offset(uint64_t offset, const unsigned long long* offset_dev) {
   return offset + (offset_dev ? (uint64_t)*offset_dev : 0ull);
 }
@@ -437,20 +430,24 @@ int launch_mm_backward(const gpblur_svgp_params& p, const WsLayout& L, void* sta
                        const float* g_kl, float* grad_bucket, cudaStream_t st, int accumulate = 0, int max_ctas = 0);
 // reduces the split partials left in `ws` by the point backward + N-reduction GEMMs into sgrad (fixed order, fp64)
 int launch_stage_grad_reduce(const WsLayout& L, const void* ws, double* sgrad, cudaStream_t st);
-int launch_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var,
+struct SegGrads;   // per-segment upstream gradients of a point backward (gpblur_tile.cuh)
+// The point launchers read the constant operands from `stage` (the parameter stage: the caller's workspace itself
+// when the stage was built there) and write the per-call buffers into `ws`.
+int launch_point_forward(const WsLayout& L, const void* stage, void* ws, const float* x, float* mean, float* var,
                          float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
-                         cudaStream_t st);
-int launch_point_backward(const WsLayout& L, void* ws, const float* x, const float* g_mean,
-                          const float* g_var, const float* g_sample, const float* var, uint64_t seed,
-                          uint64_t offset, uint32_t stream_id, float* dx, cudaStream_t st);
+                         const unsigned long long* offset_dev, cudaStream_t st);
+int launch_point_backward(const WsLayout& L, const void* stage, void* ws, const float* x, const SegGrads& seg,
+                          const float* var, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                          const unsigned long long* offset_dev, float* dx, cudaStream_t st);
 int launch_reductions(const WsLayout& L, void* ws, const float* x, cudaStream_t st);
 // tensor-core (tcgen05 3xTF32) variants; *_supported() decides per problem shape
 bool tc_point_supported(const WsLayout& L);
-int launch_tc_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var, float* sample,
-                            uint64_t seed, uint64_t offset, uint32_t stream_id, cudaStream_t st);
-int launch_tc_point_backward(const WsLayout& L, void* ws, const float* x, const float* g_mean, const float* g_var,
-                             const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
-                             uint32_t stream_id, float* dx, cudaStream_t st);
+int launch_tc_point_forward(const WsLayout& L, const void* stage, void* ws, const float* x, float* mean, float* var,
+                            float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                            const unsigned long long* offset_dev, cudaStream_t st);
+int launch_tc_point_backward(const WsLayout& L, const void* stage, void* ws, const float* x, const SegGrads& seg,
+                             const float* var, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                             const unsigned long long* offset_dev, float* dx, cudaStream_t st);
 int tc_vector_partials(const WsLayout& L);
 
 }  // namespace gpblur

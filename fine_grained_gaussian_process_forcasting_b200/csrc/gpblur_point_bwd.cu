@@ -10,11 +10,11 @@ int launch_point_backward_dp128(const PointBwdArgs& a, cudaStream_t st);
 
 int bwd_vector_partials(const WsLayout& L) { return bwd_persistent_grid(L, bwd_tile_points(L)); }
 
-int launch_point_backward(const WsLayout& L, void* ws, const float* x, const float* g_mean, const float* g_var,
-                          const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
-                          uint32_t stream_id, float* dx, cudaStream_t st) {
+int launch_point_backward(const WsLayout& L, const void* stage, void* ws, const float* x, const SegGrads& seg,
+                          const float* var, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                          const unsigned long long* offset_dev, float* dx, cudaStream_t st) {
   if (L.N <= 0) return GPBLUR_OK;
-  PointBwdArgs a{L, ws, current_param_stage() ? current_param_stage() : ws, x, g_mean, g_var, g_sample, var, seed, offset, stream_id, dx, 0, current_offset_dev(), current_seg_grads()};
+  PointBwdArgs a{L, ws, stage, x, var, seed, offset, stream_id, dx, 0, offset_dev, seg};
   switch (L.DP) {
     case 16: return launch_point_backward_dp16(a, st);
     case 32: return launch_point_backward_dp32(a, st);

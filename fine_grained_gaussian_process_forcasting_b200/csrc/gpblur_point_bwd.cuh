@@ -94,7 +94,7 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
       if (gn < N) {
         float gs;
         bool has_gs;
-        upstream_grads(a.seg, a.g_mean, a.g_var, a.g_sample, gn, gm, gv, gs, has_gs);
+        upstream_grads(a.seg, gn, gm, gv, gs, has_gs);
         const float v = a.var[gn];
         if (has_gs) {
           const float eps = philox_normal(a.seed, rng_offset(a.offset, a.offset_dev) + (uint64_t)gn, a.stream_id);

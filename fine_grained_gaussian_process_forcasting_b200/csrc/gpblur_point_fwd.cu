@@ -227,10 +227,11 @@ int dispatch_fwd_tn(const PointFwdArgs& a, cudaStream_t st) {
 
 }  // namespace
 
-int launch_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var, float* sample,
-                         uint64_t seed, uint64_t offset, uint32_t stream_id, cudaStream_t st) {
+int launch_point_forward(const WsLayout& L, const void* stage, void* ws, const float* x, float* mean, float* var,
+                         float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                         const unsigned long long* offset_dev, cudaStream_t st) {
   if (L.N <= 0) return GPBLUR_OK;
-  PointFwdArgs a{L, ws, current_param_stage() ? current_param_stage() : ws, x, mean, var, sample, seed, offset, stream_id, 0, current_offset_dev()};
+  PointFwdArgs a{L, ws, stage, x, mean, var, sample, seed, offset, stream_id, 0, offset_dev};
   if (L.MP == 32) return dispatch_fwd_tn<4, 32>(a, st);
   if (L.MP == 64) return dispatch_fwd_tn<4, 64>(a, st);
   return dispatch_fwd_tn<8, 128>(a, st);

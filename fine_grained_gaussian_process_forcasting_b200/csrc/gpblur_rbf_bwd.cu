@@ -1,4 +1,4 @@
-// Backward of the dense ScaleKernel(RBF) covariance (gpblur_rbf_covariance): what torch autograd computes through
+// Backward of the dense ScaleKernel(RBF) covariance (gpblur_covariance): what torch autograd computes through
 // gpytorch's kernel evaluation when an exact GP is trained (/root/reference/denoising_model/GPModel.py:4-13 builds
 // MultivariateNormal(mean, ScaleKernel(RBF)(x)); the marginal log likelihood differentiates the covariance w.r.t. the
 // raw lengthscale / outputscale and the inputs).  With W = G o K (G = upstream gradient of the covariance):
@@ -140,10 +140,6 @@ extern "C" size_t gpblur_covariance_backward_scratch_bytes(long long n1, long lo
   return (kind == GPBLUR_KERNEL_RBF ? wb : 2 * wb) + (size_t)n1 * (size_t)(D + 1) * 8;
 }
 
-extern "C" size_t gpblur_rbf_covariance_backward_scratch_bytes(long long n1, long long n2, int D) {
-  return gpblur_covariance_backward_scratch_bytes(n1, n2, D, GPBLUR_KERNEL_RBF);
-}
-
 extern "C" int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                                           const float* raw_lengthscale, int ard, const float* raw_outputscale,
                                           const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
@@ -182,13 +178,4 @@ extern "C" int gpblur_covariance_backward(const float* x1, const float* x2, long
                                            g_raw_outputscale);
   note_launch(g_x2 ? 4 : 3);
   return check_launch("rbf_cov_backward");
-}
-
-extern "C" int gpblur_rbf_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D,
-                                              const float* raw_lengthscale, int ard, const float* raw_outputscale,
-                                              const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
-                                              float* g_raw_outputscale, void* scratch, size_t scratch_bytes,
-                                              void* stream) {
-  return gpblur_covariance_backward(x1, x2, n1, n2, D, GPBLUR_KERNEL_RBF, raw_lengthscale, ard, raw_outputscale, g_out,
-                                    g_x1, g_x2, g_raw_lengthscale, g_raw_outputscale, scratch, scratch_bytes, stream);
 }

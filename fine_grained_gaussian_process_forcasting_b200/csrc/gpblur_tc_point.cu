@@ -47,15 +47,12 @@ constexpr int kMaxDs = 4;       // d-slabs of the x tile (D <= 128)
 struct Tc2Args {
   WsLayout L;
   void* ws;
-  const void* stage;   // parameter stage (== ws when the stage was built in / copied into the workspace)
+  const void* stage;   // parameter stage (== ws when the stage was built in the workspace)
   const float* x;
   float* mean;
   float* var;
   float* sample;
-  const float* g_mean;
-  const float* g_var;
-  const float* g_sample;
-  SegGrads seg;          // per-segment upstream gradients (nseg == 0: g_mean / g_var / g_sample above)
+  SegGrads seg;          // per-segment upstream gradients (backward)
   const float* var_in;
   float* dx;
   uint64_t seed, offset;
@@ -987,7 +984,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
         if (live) {
           float gsv;
           bool has_gs;
-          upstream_grads(a.seg, a.g_mean, a.g_var, a.g_sample, gn, gm, gv, gsv, has_gs);
+          upstream_grads(a.seg, gn, gm, gv, gsv, has_gs);
           const float vr = a.var_in[gn];
           if (has_gs) {
             const float eps = philox_normal(a.seed, rng_offset(a.offset, a.offset_dev) + (uint64_t)gn, a.stream_id);
@@ -1256,11 +1253,12 @@ bool tc_point_supported(const WsLayout& L) {
 
 int tc_vector_partials(const WsLayout& L) { return tc2_grid(L); }
 
-int launch_tc_point_forward(const WsLayout& L, void* ws, const float* x, float* mean, float* var, float* sample,
-                            uint64_t seed, uint64_t offset, uint32_t stream_id, cudaStream_t st) {
+int launch_tc_point_forward(const WsLayout& L, const void* stage, void* ws, const float* x, float* mean, float* var,
+                            float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                            const unsigned long long* offset_dev, cudaStream_t st) {
   Tc2Args a{};
-  a.L = L; a.ws = ws; a.stage = current_param_stage() ? current_param_stage() : ws; a.x = x; a.mean = mean; a.var = var; a.sample = sample;
-  a.seed = seed; a.offset = offset; a.offset_dev = current_offset_dev(); a.stream_id = stream_id;
+  a.L = L; a.ws = ws; a.stage = stage; a.x = x; a.mean = mean; a.var = var; a.sample = sample;
+  a.seed = seed; a.offset = offset; a.offset_dev = offset_dev; a.stream_id = stream_id;
   a.ntiles = (int)((L.N + TNP - 1) / TNP);
   a.trace = debug_trace_buffer();
   const int grid = tc2_grid(L);
@@ -1271,12 +1269,12 @@ int launch_tc_point_forward(const WsLayout& L, void* ws, const float* x, float* 
   return check_launch("tc_point_fwd");
 }
 
-int launch_tc_point_backward(const WsLayout& L, void* ws, const float* x, const float* g_mean, const float* g_var,
-                             const float* g_sample, const float* var, uint64_t seed, uint64_t offset,
-                             uint32_t stream_id, float* dx, cudaStream_t st) {
+int launch_tc_point_backward(const WsLayout& L, const void* stage, void* ws, const float* x, const SegGrads& seg,
+                             const float* var, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                             const unsigned long long* offset_dev, float* dx, cudaStream_t st) {
   Tc2Args a{};
-  a.L = L; a.ws = ws; a.stage = current_param_stage() ? current_param_stage() : ws; a.x = x; a.g_mean = g_mean; a.g_var = g_var; a.g_sample = g_sample; a.seg = current_seg_grads(); a.var_in = var; a.dx = dx;
-  a.seed = seed; a.offset = offset; a.offset_dev = current_offset_dev(); a.stream_id = stream_id;
+  a.L = L; a.ws = ws; a.stage = stage; a.x = x; a.seg = seg; a.var_in = var; a.dx = dx;
+  a.seed = seed; a.offset = offset; a.offset_dev = offset_dev; a.stream_id = stream_id;
   a.ntiles = (int)((L.N + TNP - 1) / TNP);
   a.trace = debug_trace_buffer();
   const int grid = tc2_grid(L);

@@ -84,7 +84,7 @@ __device__ __forceinline__ void stage_points(float* dst, const float* __restrict
 struct PointFwdArgs {
   WsLayout L;
   void* ws;
-  const void* stage;   // parameter stage (== ws when the stage was built in / copied into the workspace)
+  const void* stage;   // parameter stage (== ws when the stage was built in the workspace)
   const float* x;
   float* mean;
   float* var;
@@ -95,9 +95,9 @@ struct PointFwdArgs {
   const unsigned long long* offset_dev;   // optional device-resident addend of `offset` (CUDA-graph replays)
 };
 
-// Upstream gradients given per SEGMENT of the point range (several activations of one training step evaluated in one
-// call: gpblur_svgp_point_backward_segments): segment s covers points [start[s], start[s + 1]) and brings its own
-// (nullable) g_mean / g_var / g_sample arrays, indexed from the start of the segment.  nseg == 0: not used.
+// Upstream gradients of a point backward, given per SEGMENT of the point range (several activations of one training
+// step evaluated in one call): segment s covers points [start[s], start[s + 1]) and brings its own (nullable)
+// g_mean / g_var / g_sample arrays, indexed from the start of the segment.  1 <= nseg <= kMaxSegments, start[0] = 0.
 constexpr int kMaxSegments = 4;
 struct SegGrads {
   int nseg;
@@ -106,12 +106,13 @@ struct SegGrads {
   const float* gv[kMaxSegments];
   const float* gs[kMaxSegments];
 };
-__device__ __forceinline__ void upstream_grads(const SegGrads& sg, const float* g_mean, const float* g_var,
-                                               const float* g_sample, long long gn, float& gm, float& gv, float& gsv,
+__device__ __forceinline__ void upstream_grads(const SegGrads& sg, long long gn, float& gm, float& gv, float& gsv,
                                                bool& has_gs) {
-  const float *pm = g_mean, *pv = g_var, *ps = g_sample;
+  // one segment (every single-call backward): the pointers are fixed kernel-parameter loads, no indexed lookup in
+  // front of the gradient loads
+  const float *pm = sg.gm[0], *pv = sg.gv[0], *ps = sg.gs[0];
   long long ln = gn;
-  if (sg.nseg > 0) {
+  if (sg.nseg > 1) {
     int s = 0;
 #pragma unroll
     for (int i = 1; i < kMaxSegments; ++i)
@@ -128,11 +129,8 @@ __device__ __forceinline__ void upstream_grads(const SegGrads& sg, const float* 
 struct PointBwdArgs {
   WsLayout L;
   void* ws;
-  const void* stage;   // parameter stage (== ws when the stage was built in / copied into the workspace)
+  const void* stage;   // parameter stage (== ws when the stage was built in the workspace)
   const float* x;
-  const float* g_mean;
-  const float* g_var;
-  const float* g_sample;
   const float* var;
   uint64_t seed, offset;
   uint32_t stream_id;

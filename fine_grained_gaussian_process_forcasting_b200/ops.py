@@ -68,9 +68,6 @@ def workspace_bytes(N: int, D: int, M: int, training: bool) -> int:
     n = _WS_BYTES_CACHE.get(key)
     if n is None:
         n = int(_cabi.lib().gpblur_svgp_workspace_bytes(N, D, M, int(training)))
-        if n == 0:
-            raise RuntimeError(f"unsupported SVGP shape N={N} D={D} M={M} (D <= {_cabi.GPBLUR_MAX_D}, "
-                               f"M <= {_cabi.GPBLUR_MAX_M})")
         if len(_WS_BYTES_CACHE) < 4096:
             _WS_BYTES_CACHE[key] = n
     return n
@@ -85,16 +82,18 @@ _STAGE_BYTES_CACHE = {}
 def param_stage_bytes(D: int, M: int) -> int:
     n = _STAGE_BYTES_CACHE.get((D, M))
     if n is None:
-        n = _STAGE_BYTES_CACHE[(D, M)] = int(_cabi.lib().gpblur_svgp_param_stage_bytes(D, M))
+        n = int(_cabi.lib().gpblur_svgp_param_stage_bytes(D, M))
+        if n == 0:
+            raise RuntimeError(f"unsupported SVGP shape D={D} M={M} (D <= {_cabi.GPBLUR_MAX_D}, "
+                               f"M <= {_cabi.GPBLUR_MAX_M})")
+        _STAGE_BYTES_CACHE[(D, M)] = n
     return n
 
 
 def svgp_forward_raw(x: Tensor, Z: Tensor, raw_ell: Tensor, raw_os: Tensor, m: Tensor, s: Tensor,
                      w: Optional[Tensor], b: Tensor, seed: int, offset: int, stream_id: int,
-                     want_sample: bool, training: bool, param_stage: Optional[Tensor] = None):
-    """x [N, D] -> (mean [N], var [N], sample [N] | None, kl [1], info [1] int32, workspace uint8).
-    `param_stage`: the leading param_stage_bytes(D, M) bytes of the workspace of an earlier forward with the same
-    parameter values; if given, the M x M stage is copied instead of recomputed."""
+                     want_sample: bool, training: bool):
+    """x [N, D] -> (mean [N], var [N], sample [N] | None, kl [1], info [1] int32, workspace uint8)."""
     _need_cuda(x, Z, raw_ell, raw_os, m, s, w, b)
     N, D = x.shape
     M = Z.shape[0]
@@ -107,10 +106,10 @@ def svgp_forward_raw(x: Tensor, Z: Tensor, raw_ell: Tensor, raw_os: Tensor, m: T
     ws = torch.empty(workspace_bytes(N, D, M, training), device=dev, dtype=torch.uint8)
     p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
     with torch.cuda.device(dev):
-        rc = _cabi.lib().gpblur_svgp_forward_cached(
+        rc = _cabi.lib().gpblur_svgp_forward(
             C.byref(p), _ptr(x), N, D, M, _ptr(mean), _ptr(var), _ptr(sample),
             seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF,
-            _ptr(kl), _ptr(info), int(training), _ptr(ws), ws.numel(), _ptr(param_stage), _stream())
+            _ptr(kl), _ptr(info), int(training), _ptr(ws), ws.numel(), _stream())
     _cabi.check(rc, "gpblur_svgp_forward")
     return mean, var, sample, kl, info, ws
 
@@ -328,29 +327,15 @@ def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: floa
     M, D = Z.shape
     dev = Z.device
     if out is None:
-        nbytes = param_stage_bytes(D, M)
-        if nbytes == 0:
-            raise RuntimeError(f"unsupported SVGP shape D={D} M={M} (D <= {_cabi.GPBLUR_MAX_D}, "
-                               f"M <= {_cabi.GPBLUR_MAX_M})")
-        stage = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+        stage = torch.empty(param_stage_bytes(D, M), device=dev, dtype=torch.uint8)
         kl = torch.empty(1, device=dev, dtype=torch.float32)
         info = torch.empty(1, device=dev, dtype=torch.int32)
     else:
         stage, kl, info = out
     p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
     with torch.cuda.device(dev):
-        if kind:
-            rc = _cabi.lib().gpblur_svgp_param_stage_kind(C.byref(p), D, M, int(kind), float(extra_jitter), int(max_ctas),
-                                                          _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
-        elif max_ctas:
-            rc = _cabi.lib().gpblur_svgp_param_stage_shared_sms(C.byref(p), D, M, float(extra_jitter), int(max_ctas),
-                                                                _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
-        elif extra_jitter:
-            rc = _cabi.lib().gpblur_svgp_param_stage_jitter(C.byref(p), D, M, float(extra_jitter), _ptr(kl), _ptr(info),
-                                                            _ptr(stage), stage.numel(), _stream())
-        else:
-            rc = _cabi.lib().gpblur_svgp_param_stage(C.byref(p), D, M, _ptr(kl), _ptr(info), _ptr(stage), stage.numel(),
-                                                     _stream())
+        rc = _cabi.lib().gpblur_svgp_param_stage(C.byref(p), D, M, int(kind), float(extra_jitter), int(max_ctas),
+                                                 _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
     _cabi.check(rc, "gpblur_svgp_param_stage")
     return stage, kl, info
 
@@ -358,7 +343,7 @@ def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: floa
 def point_forward_raw(stage: Tensor, x: Tensor, M: int, seed: int, offset: int, stream_id: int, want_sample: bool,
                       training: bool, out: Optional[Tensor] = None, offset_dev: Optional[Tensor] = None,
                       ws: Optional[Tensor] = None, kind: int = 0):
-    """x [N, D] + parameter stage -> (mean [N], var [N], sample [N] | None, workspace uint8).
+    """x [N, D] + parameter stage (read in place) -> (mean [N], var [N], sample [N] | None, workspace uint8).
     `out`: preallocated float32 [(3 | 2) * N] receiving mean | var | sample."""
     _need_cuda(x, stage)
     N, D = x.shape
@@ -370,59 +355,27 @@ def point_forward_raw(stage: Tensor, x: Tensor, M: int, seed: int, offset: int, 
     if ws is None:
         ws = torch.empty(workspace_bytes(N, D, M, training), device=dev, dtype=torch.uint8)
     with torch.cuda.device(dev):
-        # "_shared": the kernels read the stage in place (no device-to-device copy of it into `ws`)
-        tail = (_ptr(mean), _ptr(var), _ptr(sample), seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF,
-                stream_id & 0xFFFFFFFF, _ptr(offset_dev), int(training), _ptr(ws), ws.numel(), _stream())
-        if kind:
-            rc = _cabi.lib().gpblur_svgp_point_forward_shared_kind(_ptr(stage), _ptr(x), N, D, M, int(kind), *tail)
-        else:
-            rc = _cabi.lib().gpblur_svgp_point_forward_shared(_ptr(stage), _ptr(x), N, D, M, *tail)
-    _cabi.check(rc, "gpblur_svgp_point_forward_shared")
+        rc = _cabi.lib().gpblur_svgp_point_forward(
+            _ptr(stage), _ptr(x), N, D, M, int(kind), _ptr(mean), _ptr(var), _ptr(sample), seed & 0xFFFFFFFFFFFFFFFF,
+            offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev), int(training), _ptr(ws), ws.numel(),
+            _stream())
+    _cabi.check(rc, "gpblur_svgp_point_forward")
     return mean, var, sample, ws
 
 
 def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, offset, stream_id, ws,
                        need_dx: bool = True, dx: Optional[Tensor] = None, sgrad: Optional[Tensor] = None,
-                       offset_dev: Optional[Tensor] = None, stage: Optional[Tensor] = None, kind: int = 0):
+                       offset_dev: Optional[Tensor] = None, stage: Optional[Tensor] = None, kind: int = 0,
+                       seg_sizes=None):
     """-> (dx [N, D] | None, stage_grad float64 [stage_grad_doubles(D, M)]).
-    `stage`: the parameter stage the matching point_forward_raw call read (None: the stage was built in `ws` itself by
-    svgp_forward_raw)."""
-    _need_cuda(x, ws, g_mean, g_var, g_sample, var)
+    Upstream gradients `g_mean` / `g_var` / `g_sample`: [N] tensors or None.  With `seg_sizes` (1 to 4 point counts
+    summing to N) they come per segment of the point range instead: lists of one tensor or None per segment, indexed
+    from the start of the segment.  `stage`: the parameter stage the matching point_forward_raw call read (None: the
+    stage was built in `ws` itself by svgp_forward_raw).  `dx` / `sgrad`: preallocated outputs."""
     N, D = x.shape
-    dev = x.device
-    if dx is None and need_dx:
-        dx = torch.empty(N, D, device=dev, dtype=torch.float32)
-    if sgrad is None:
-        sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
-    if kind:               # the kind-taking point backward is the segments form: one segment
-        keep = [None if t is None else _f32c(t) for t in (g_mean, g_var, g_sample)]
-        ptrs = [(C.c_void_p * 1)(_ptr(t)) for t in keep]
-        with torch.cuda.device(dev):
-            rc = _cabi.lib().gpblur_svgp_point_backward_segments_kind(
-                _ptr(stage), _ptr(x), N, D, M, int(kind), 1, (C.c_longlong * 1)(0), *ptrs, _ptr(var),
-                seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev),
-                _ptr(dx if need_dx else None), _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
-        _cabi.check(rc, "gpblur_svgp_point_backward_segments_kind")
-        return (dx if need_dx else None), sgrad
-    with torch.cuda.device(dev):
-        args = (_ptr(x), N, D, M, _ptr(g_mean), _ptr(g_var), _ptr(g_sample), _ptr(var),
-                seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev),
-                _ptr(dx if need_dx else None), _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
-        if stage is not None:
-            rc = _cabi.lib().gpblur_svgp_point_backward_shared(_ptr(stage), *args)
-        else:
-            rc = _cabi.lib().gpblur_svgp_point_backward(*args)
-    _cabi.check(rc, "gpblur_svgp_point_backward")
-    return (dx if need_dx else None), sgrad
-
-
-def point_backward_segments_raw(x: Tensor, M: int, seg_sizes, g_means, g_vars, g_samples, var, seed, offset, stream_id,
-                                ws, need_dx: bool = True, offset_dev: Optional[Tensor] = None,
-                                stage: Optional[Tensor] = None, kind: int = 0):
-    """point_backward_raw with the upstream gradients given per segment of the point range (lists of tensors or None,
-    one entry per segment, indexed from the start of the segment) -> (dx [N, D] | None, stage_grad)."""
-    _need_cuda(x, ws, var)
-    N, D = x.shape
+    if seg_sizes is None:          # one segment: all N points
+        seg_sizes, g_mean, g_var, g_sample = [N], [g_mean], [g_var], [g_sample]
+    _need_cuda(x, ws, var, stage, *g_mean, *g_var, *g_sample)
     dev = x.device
     nseg = len(seg_sizes)
     starts, o = [], 0
@@ -434,19 +387,20 @@ def point_backward_segments_raw(x: Tensor, M: int, seg_sizes, g_means, g_vars, g
     def ptr_array(ts):
         return (C.c_void_p * nseg)(*[(_ptr(t) if t is not None else None) for t in ts])
 
-    keep = [None if t is None else _f32c(t) for t in list(g_means) + list(g_vars) + list(g_samples)]   # alive until launch
+    keep = [None if t is None else _f32c(t) for t in list(g_mean) + list(g_var) + list(g_sample)]   # alive until launch
     gm, gv, gs = keep[:nseg], keep[nseg:2 * nseg], keep[2 * nseg:]
-    dx = torch.empty(N, D, device=dev, dtype=torch.float32) if need_dx else None
-    sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
+    if not need_dx:
+        dx = None
+    elif dx is None:
+        dx = torch.empty(N, D, device=dev, dtype=torch.float32)
+    if sgrad is None:
+        sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
     with torch.cuda.device(dev):
-        tail = (nseg, (C.c_longlong * nseg)(*starts), ptr_array(gm), ptr_array(gv), ptr_array(gs), _ptr(var),
-                seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF, _ptr(offset_dev), _ptr(dx),
-                _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
-        if kind:
-            rc = _cabi.lib().gpblur_svgp_point_backward_segments_kind(_ptr(stage), _ptr(x), N, D, M, int(kind), *tail)
-        else:
-            rc = _cabi.lib().gpblur_svgp_point_backward_segments(_ptr(stage), _ptr(x), N, D, M, *tail)
-    _cabi.check(rc, "gpblur_svgp_point_backward_segments")
+        rc = _cabi.lib().gpblur_svgp_point_backward(
+            _ptr(stage), _ptr(x), N, D, M, int(kind), nseg, (C.c_longlong * nseg)(*starts), ptr_array(gm), ptr_array(gv),
+            ptr_array(gs), _ptr(var), seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFF,
+            _ptr(offset_dev), _ptr(dx), _ptr(sgrad), _ptr(ws), ws.numel(), _stream())
+    _cabi.check(rc, "gpblur_svgp_point_backward")
     return dx, sgrad
 
 
@@ -461,17 +415,9 @@ def param_stage_backward_raw(Z, raw_ell, raw_os, m, s, w, b, sgrad: Tensor, g_kl
         bucket = torch.empty(grad_bucket_floats(D, M), device=Z.device, dtype=torch.float32)
     p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
     with torch.cuda.device(Z.device):
-        if kind:
-            rc = _cabi.lib().gpblur_svgp_param_stage_backward_kind(
-                C.byref(p), D, M, int(kind), _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas),
-                _ptr(stage), stage.numel(), _stream())
-        elif max_ctas:
-            rc = _cabi.lib().gpblur_svgp_param_stage_backward_shared_sms(
-                C.byref(p), D, M, _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas), _ptr(stage),
-                stage.numel(), _stream())
-        else:
-            rc = _cabi.lib().gpblur_svgp_param_stage_backward_acc(C.byref(p), D, M, _ptr(sgrad), _ptr(g_kl), _ptr(bucket),
-                                                                  int(accumulate), _ptr(stage), stage.numel(), _stream())
+        rc = _cabi.lib().gpblur_svgp_param_stage_backward(
+            C.byref(p), D, M, int(kind), _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas),
+            _ptr(stage), stage.numel(), _stream())
     _cabi.check(rc, "gpblur_svgp_param_stage_backward")
     return bucket
 
@@ -571,11 +517,7 @@ class _ParamStageFunction(torch.autograd.Function):
         bc = _f32c(b).reshape(-1, 1)                                  # [1, 1] shared or [H, 1]
         dev = Zc.device
         _need_cuda(Zc)
-        nbytes = param_stage_bytes(D, M)
-        if nbytes == 0:
-            raise RuntimeError(f"unsupported SVGP shape D={D} M={M} (D <= {_cabi.GPBLUR_MAX_D}, "
-                               f"M <= {_cabi.GPBLUR_MAX_M})")
-        stage = torch.empty(H, nbytes, device=dev, dtype=torch.uint8)
+        stage = torch.empty(H, param_stage_bytes(D, M), device=dev, dtype=torch.uint8)
         kl = torch.empty(H, device=dev, dtype=torch.float32)
         info = torch.empty(H, device=dev, dtype=torch.int32)
         fork = _Fork(dev, H)
@@ -586,7 +528,7 @@ class _ParamStageFunction(torch.autograd.Function):
                 param_stage_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h], None if wc is None else wc[h % wc.shape[0]],
                                 bc[h % bc.shape[0]], out=(stage[h], kl[h:h + 1], info[h:h + 1]),
                                 extra_jitter=float(holder.get("extra_jitter", 0.0)), max_ctas=cap,
-                                kind=holder.get("kind", 0))
+                                kind=holder["kind"])
         finally:
             fork.join()
         holder["stage"] = stage
@@ -626,7 +568,7 @@ class _ParamStageFunction(torch.autograd.Function):
             # (distributed.FlatGradBucket): the kernel accumulates straight into it, autograd gets no gradient to add
             param_stage_backward_raw(Zc[0], ellc[0], osc[0], mc[0], sc[0], wc[0], bc[0], sgrad[0],
                                      None if gk is None else gk[0:1], stage[0], bucket=sink, accumulate=True,
-                                     kind=holder.get("kind", 0))
+                                     kind=holder["kind"])
             holder["consumed"] = True
             return (None,) * 8
         bucket = torch.empty(H, nb, device=dev, dtype=torch.float32)
@@ -638,7 +580,7 @@ class _ParamStageFunction(torch.autograd.Function):
                 param_stage_backward_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h],
                                          None if wc is None else wc[h % wc.shape[0]], bc[h % bc.shape[0]], sgrad[h],
                                          None if gk is None else gk[h:h + 1], stage[h], bucket=bucket[h], max_ctas=cap,
-                                         kind=holder.get("kind", 0))
+                                         kind=holder["kind"])
         finally:
             fork.join()
         holder["consumed"] = True        # the graph behind this token is gone: the next forward rebuilds the stage
@@ -692,13 +634,13 @@ class _PointFunction(torch.autograd.Function):
             for h in range(H):
                 fork.enter(h)
                 point_forward_raw(stage[h], x2, M, seed, offset + h * hs, stream_id, want_sample, training,
-                                  out=out[h], offset_dev=offset_dev, ws=wss[h], kind=holder.get("kind", 0))
+                                  out=out[h], offset_dev=offset_dev, ws=wss[h], kind=holder["kind"])
         finally:
             fork.join()
         if training:
             ctx.save_for_backward(x2, out, *wss)
             ctx.stage = stage                                  # read in place by the backward kernels
-            ctx.kind = holder.get("kind", 0)
+            ctx.kind = holder["kind"]
         ctx.meta = (seed, offset, stream_id, M, shape, H, batched, nout, hs)
         ctx.offset_dev = offset_dev
         ctx.set_materialize_grads(False)
@@ -788,9 +730,9 @@ def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outpu
         if ent is not None and stage_cache.get("key") == key and not ent[3]["consumed"] \
                 and ent[0].requires_grad == want_grad:
             return ent
-    holder = {} if grad_sink is None else {"grad_sink": grad_sink}
-    if kind:
-        holder["kind"] = kind
+    holder = {"kind": kind}
+    if grad_sink is not None:
+        holder["grad_sink"] = grad_sink
     with torch.cuda.nvtx.range("gpblur.param_stage") if _NVTX else _null_ctx():
         token, kl, info = _ParamStageFunction.apply(*params, holder)
     # Cholesky status (LAPACK-style info, 0 = ok).  Reading it synchronises with the device, as gpytorch's
@@ -800,11 +742,9 @@ def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outpu
         if k != 0:
             import warnings
             for jit in JITTER_RETRIES:
-                holder = {"extra_jitter": jit}
+                holder = {"kind": kind, "extra_jitter": jit}
                 if grad_sink is not None:
                     holder["grad_sink"] = grad_sink
-                if kind:
-                    holder["kind"] = kind
                 token, kl, info = _ParamStageFunction.apply(*params, holder)
                 if int(info.max().item()) == 0:
                     warnings.warn(f"Kzz + 1e-4 I is not positive definite (pivot {k}): added jitter of {jit:.1e} to the "
@@ -881,11 +821,11 @@ class _PointSegFunction(torch.autograd.Function):
         stage = holder["stage"]
         ws = torch.empty(workspace_bytes(N, D, M, training), device=x2.device, dtype=torch.uint8)
         point_forward_raw(stage[0], x2, M, seed, offset, stream_id, want_sample, training, out=out,
-                          offset_dev=offset_dev, ws=ws, kind=holder.get("kind", 0))
+                          offset_dev=offset_dev, ws=ws, kind=holder["kind"])
         if training:
             ctx.save_for_backward(x2, out, ws)
             ctx.stage = stage
-            ctx.kind = holder.get("kind", 0)
+            ctx.kind = holder["kind"]
         ctx.meta = (seed, offset, stream_id, M, tuple(x.shape), sizes, nout)
         ctx.offset_dev = offset_dev
         ctx.set_materialize_grads(False)
@@ -904,9 +844,9 @@ class _PointSegFunction(torch.autograd.Function):
         need = ctx.needs_input_grad
         gms, gvs, gss = list(grads[0::3]), list(grads[1::3]), list(grads[2::3])
         with torch.cuda.nvtx.range("gpblur.point_backward") if _NVTX else _null_ctx():
-            dx, sgrad = point_backward_segments_raw(x2, M, sizes, gms, gvs, gss, out[N:2 * N], seed, offset, stream_id, ws,
-                                                    need_dx=need[0], offset_dev=ctx.offset_dev, stage=ctx.stage[0],
-                                                    kind=ctx.kind)
+            dx, sgrad = point_backward_raw(x2, M, gms, gvs, gss, out[N:2 * N], seed, offset, stream_id, ws,
+                                           need_dx=need[0], offset_dev=ctx.offset_dev, stage=ctx.stage[0], kind=ctx.kind,
+                                           seg_sizes=sizes)
         return (dx.reshape(xshape) if dx is not None else None, sgrad if need[1] else None) + (None,) * 8
 
 

@@ -36,14 +36,14 @@ extern "C" {
 #define GPBLUR_MAX_D 128
 #define GPBLUR_MAX_M 1024
 
-/* Covariance function of a layer (the `kind` argument of the *_kind entry points below).  With x~ = (x - c) / ell,
+/* Covariance function of a layer (the `kind` argument of the entry points below).  With x~ = (x - c) / ell,
  * d2 = |x~ - z~|^2 and r = sqrt(max(d2, 1e-30)) (gpytorch's covar_dist), k = os f:
- *   RBF         f = exp(-d2 / 2)                         (every entry point without a kind argument)
+ *   RBF         f = exp(-d2 / 2)                         (gpblur_svgp_forward / gpblur_svgp_backward)
  *   MATERN12    f = exp(-r)                              (gpytorch MaternKernel(nu=0.5))
  *   MATERN32    f = (1 + sqrt3 r) exp(-sqrt3 r)          (nu=1.5)
  *   MATERN52    f = (1 + sqrt5 r + 5/3 r^2) exp(-sqrt5 r) (nu=2.5)
- * A parameter stage must be consumed (point forward / backward, stage backward) with the kind it was built with;
- * nothing on the device checks this. */
+ * An unknown kind returns GPBLUR_EINVAL.  A parameter stage must be consumed (point forward / backward, stage backward)
+ * with the kind it was built with; nothing on the device checks this. */
 #define GPBLUR_KERNEL_RBF 0
 #define GPBLUR_KERNEL_MATERN12 1
 #define GPBLUR_KERNEL_MATERN32 2
@@ -89,16 +89,6 @@ int gpblur_svgp_forward(const gpblur_svgp_params* p, const float* x, long long N
  * fp32 operands derived from them).  They depend only on the parameters, not on x. */
 size_t gpblur_svgp_param_stage_bytes(int D, int M);
 
-/* Same as gpblur_svgp_forward, but the M x M stage is COPIED from `param_stage` (the first
- * gpblur_svgp_param_stage_bytes() bytes of the workspace of an earlier forward with the SAME parameter values)
- * instead of being recomputed.  The reference evaluates the GP twice per training step with unchanged parameters
- * (/root/reference/denoising_model/denoise_model_2.py:50-51, encoder and decoder side) and gpytorch re-factorises
- * Kzz both times; this entry point shares one factorisation between the two calls. */
-int gpblur_svgp_forward_cached(const gpblur_svgp_params* p, const float* x, long long N, int D, int M,
-                               float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
-                               uint32_t stream_id, float* kl, int* info, int training, void* ws,
-                               size_t ws_bytes, const void* param_stage, void* stream);
-
 /* Backward of gpblur_svgp_forward (replaces torch autograd through gpytorch, incl.
  * LinalgCholeskyExBackward0 / LinalgSolveTriangularBackward0).
  * Upstream gradients g_mean, g_var, g_sample [N] (each nullable) and g_kl [1] (nullable);
@@ -123,96 +113,51 @@ int gpblur_svgp_backward(const gpblur_svgp_params* p, const float* x, long long 
  *
  * stage_grad holds gpblur_svgp_stage_grad_doubles(D, M) doubles:
  *   [ u (Mp) | colsum(W) (Mp), q (Dp), wbar (Dp), scalars (4) | S = sum g_var a a^T (Mp x Mp) | W^T X (Mp x Dp) ]
- * gpblur_svgp_forward / gpblur_svgp_backward below are the single-call compositions of these four. */
+ * gpblur_svgp_forward / gpblur_svgp_backward above are the single-call compositions of these four (RBF, the stage
+ * built in `ws`).  All four calls on one stage take the same `kind` (GPBLUR_KERNEL_*). */
 size_t gpblur_svgp_stage_grad_doubles(int D, int M);
-int gpblur_svgp_param_stage(const gpblur_svgp_params* p, int D, int M, float* kl, int* info,
-                            void* stage, size_t stage_bytes, void* stream);
-/* `ws` (gpblur_svgp_workspace_bytes(N, D, M, training)) receives a copy of the stage and, when training, the
- * saved whitened cross-covariance; hand the same `ws` to gpblur_svgp_point_backward.
+
+/* Parameters -> M x M stage in `stage` (256-byte aligned, gpblur_svgp_param_stage_bytes(D, M) bytes), kl [1], info [1].
+ * `extra_jitter` >= 0 is added to the diagonal of Kzz on top of the variational jitter 1e-4.  It replaces the retry
+ * loop of gpytorch's psd_safe_cholesky (called from VariationalStrategy.forward,
+ * /root/reference/denoising_model/DeepGP.py:33-38): when `info` reports a non-positive pivot the host retries with
+ * 1e-6, 1e-5, 1e-4 and raises NotPSDError after that.  The jitter of the data-side diagonal diag(Kxx) stays 1e-4.
+ * `max_ctas` bounds the cooperative grid (0 = none, else >= 8).  A multi-output layer (DeepGP.py:21-26: H independent
+ * GPs) launches its H stages on H streams with (SM count / H) CTAs each, so that they run side by side. */
+int gpblur_svgp_param_stage(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter, int max_ctas,
+                            float* kl, int* info, void* stage, size_t stage_bytes, void* stream);
+
+/* (stage, x [N, D]) -> mean [N], var [N], sample [N] (nullable), as gpblur_svgp_forward.  The kernels read their
+ * constant operands in place from `param_stage` (non-null, 256-byte aligned), which must stay unchanged until the
+ * matching backward call has run.  `ws` (gpblur_svgp_workspace_bytes(N, D, M, training)) holds the per-call buffers;
+ * with training != 0 hand the same `ws` to gpblur_svgp_point_backward.
  * `offset_dev` (nullable): device-resident uint64 added to `offset` when the kernel runs, so that a step captured in
  * a CUDA graph draws fresh Philox counters on every replay (the host bumps the device word between replays). */
-int gpblur_svgp_point_forward(const void* param_stage, const float* x, long long N, int D, int M,
-                              float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
-                              uint32_t stream_id, const unsigned long long* offset_dev, int training,
-                              void* ws, size_t ws_bytes, void* stream);
-int gpblur_svgp_point_backward(const float* x, long long N, int D, int M, const float* g_mean,
-                               const float* g_var, const float* g_sample, const float* var,
-                               uint64_t seed, uint64_t offset, uint32_t stream_id,
-                               const unsigned long long* offset_dev, float* dx, double* stage_grad,
-                               void* ws, size_t ws_bytes, void* stream);
-/* The same pair WITHOUT the copy of the stage into `ws`: the kernels read their constant operands (Z~ / Linv operand
- * images, vectors, hyper-parameters) straight from `param_stage`, which must stay valid and unchanged until the
- * matching backward call has run; `ws` only holds the per-call buffers (its stage prefix is left untouched).  One
- * device-to-device copy of the whole stage (4.7 MB at M = 256: ~10 us) less per call. */
-int gpblur_svgp_point_forward_shared(const void* param_stage, const float* x, long long N, int D, int M,
-                                     float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
-                                     uint32_t stream_id, const unsigned long long* offset_dev, int training,
-                                     void* ws, size_t ws_bytes, void* stream);
-int gpblur_svgp_point_backward_shared(const void* param_stage, const float* x, long long N, int D, int M,
-                                      const float* g_mean, const float* g_var, const float* g_sample,
-                                      const float* var, uint64_t seed, uint64_t offset, uint32_t stream_id,
-                                      const unsigned long long* offset_dev, float* dx, double* stage_grad,
-                                      void* ws, size_t ws_bytes, void* stream);
-/* Several activations of one step in ONE call (the reference blurs the encoder and the decoder activations with the
- * same GP, /root/reference/denoising_model/denoise_model_2.py:50-51): run the forward on the concatenated points
- * `x` [N, D]; in the backward the upstream gradients stay where autograd produced them - segment s covers points
- * [seg_start[s], seg_start[s + 1]) (seg_start[0] = 0, nseg <= 4) and g_mean[s] / g_var[s] / g_sample[s] (host arrays
- * of nullable device pointers, or null arrays) are indexed from the start of the segment.  `param_stage` may be null
- * when the stage lives in `ws`. */
-int gpblur_svgp_point_backward_segments(const void* param_stage, const float* x, long long N, int D, int M, int nseg,
-                                        const long long* seg_start, const float* const* g_mean,
-                                        const float* const* g_var, const float* const* g_sample, const float* var,
-                                        uint64_t seed, uint64_t offset, uint32_t stream_id,
-                                        const unsigned long long* offset_dev, float* dx, double* stage_grad,
-                                        void* ws, size_t ws_bytes, void* stream);
-/* gpblur_svgp_param_stage_backward with `accumulate` != 0: the gradients are ADDED to `grad_bucket`, which then is
- * the caller's live flat gradient buffer (what the data-parallel all-reduce operates on) - no intermediate bucket
- * and no per-parameter accumulation kernels on the framework side. */
-int gpblur_svgp_param_stage_backward_acc(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
-                                         const float* g_kl, float* grad_bucket, int accumulate, void* stage,
-                                         size_t stage_bytes, void* stream);
+int gpblur_svgp_point_forward(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                              float* mean, float* var, float* sample, uint64_t seed, uint64_t offset, uint32_t stream_id,
+                              const unsigned long long* offset_dev, int training, void* ws, size_t ws_bytes, void* stream);
 
-/* Same as gpblur_svgp_param_stage with `extra_jitter` >= 0 added to the diagonal of Kzz on top of the variational
- * jitter 1e-4.  Replaces the retry loop of gpytorch's psd_safe_cholesky (called from VariationalStrategy.forward,
- * /root/reference/denoising_model/DeepGP.py:33-38): when `info` reports a non-positive pivot the host retries with
- * 1e-6, 1e-5, 1e-4 and raises NotPSDError after that.  The jitter of the data-side diagonal diag(Kxx) stays 1e-4. */
-int gpblur_svgp_param_stage_jitter(const gpblur_svgp_params* p, int D, int M, double extra_jitter, float* kl,
-                                   int* info, void* stage, size_t stage_bytes, void* stream);
+/* Backward of gpblur_svgp_point_forward, with the forward's `ws`, RNG arguments and `var` output: writes dx [N, D]
+ * (nullable) and stage_grad.  `param_stage` is the stage the forward read, or null when the stage lives in `ws`.
+ * The upstream gradients come per segment, so that several activations evaluated as one call (the reference blurs the
+ * encoder and the decoder activations with the same GP) keep them where autograd produced them: segment s covers
+ * points [seg_start[s], seg_start[s + 1]) (nseg in [1, 4], seg_start[0] = 0, non-decreasing, <= N), and g_mean[s] /
+ * g_var[s] / g_sample[s] (host arrays of nullable device pointers, or null arrays) are indexed from the start of the
+ * segment.  One segment covers all N points. */
+int gpblur_svgp_point_backward(const void* param_stage, const float* x, long long N, int D, int M, int kind,
+                               int nseg, const long long* seg_start, const float* const* g_mean,
+                               const float* const* g_var, const float* const* g_sample, const float* var,
+                               uint64_t seed, uint64_t offset, uint32_t stream_id, const unsigned long long* offset_dev,
+                               float* dx, double* stage_grad, void* ws, size_t ws_bytes, void* stream);
 
-/* The two M x M stage entry points with an upper bound `max_ctas` (0 = none, else >= 8) on the size of their cooperative
- * grid.  A multi-output layer (/root/reference/denoising_model/DeepGP.py:21-26: H independent GPs) launches its H
- * stages on H streams with (SM count / H) CTAs each, so that they run side by side instead of one after the other. */
-int gpblur_svgp_param_stage_shared_sms(const gpblur_svgp_params* p, int D, int M, double extra_jitter, int max_ctas,
-                                       float* kl, int* info, void* stage, size_t stage_bytes, void* stream);
-int gpblur_svgp_param_stage_backward_shared_sms(const gpblur_svgp_params* p, int D, int M, const double* stage_grad,
-                                                const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
-                                                void* stage, size_t stage_bytes, void* stream);
-
-/* The entry points above with the covariance function as `kind` (GPBLUR_KERNEL_*; an unknown kind returns
- * GPBLUR_EINVAL).  The plain entry points are these with GPBLUR_KERNEL_RBF.  `param_stage` of the point calls may be
- * null when the stage lives in `ws` (as for gpblur_svgp_point_backward_segments). */
-int gpblur_svgp_param_stage_kind(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter,
-                                 int max_ctas, float* kl, int* info, void* stage, size_t stage_bytes, void* stream);
-int gpblur_svgp_param_stage_backward_kind(const gpblur_svgp_params* p, int D, int M, int kind,
-                                          const double* stage_grad, const float* g_kl, float* grad_bucket,
-                                          int accumulate, int max_ctas, void* stage, size_t stage_bytes, void* stream);
-int gpblur_svgp_point_forward_shared_kind(const void* param_stage, const float* x, long long N, int D, int M, int kind,
-                                          float* mean, float* var, float* sample, uint64_t seed, uint64_t offset,
-                                          uint32_t stream_id, const unsigned long long* offset_dev, int training,
-                                          void* ws, size_t ws_bytes, void* stream);
-int gpblur_svgp_point_backward_segments_kind(const void* param_stage, const float* x, long long N, int D, int M,
-                                             int kind, int nseg, const long long* seg_start,
-                                             const float* const* g_mean, const float* const* g_var,
-                                             const float* const* g_sample, const float* var, uint64_t seed,
-                                             uint64_t offset, uint32_t stream_id,
-                                             const unsigned long long* offset_dev, float* dx, double* stage_grad,
-                                             void* ws, size_t ws_bytes, void* stream);
-
-/* `stage` is the buffer filled by gpblur_svgp_param_stage; its fp64 scratch regions are overwritten. */
-int gpblur_svgp_param_stage_backward(const gpblur_svgp_params* p, int D, int M,
-                                     const double* stage_grad, const float* g_kl,
-                                     float* grad_bucket, void* stage, size_t stage_bytes,
-                                     void* stream);
+/* (stage, summed stage_grad, g_kl [1] nullable) -> flat parameter-gradient bucket.  `stage` is the buffer filled by
+ * gpblur_svgp_param_stage; its fp64 scratch regions are overwritten.  `accumulate` != 0 ADDS the gradients to
+ * `grad_bucket`, which then is the caller's live flat gradient buffer (what the data-parallel all-reduce operates on):
+ * no intermediate bucket and no per-parameter accumulation kernels on the framework side.  `max_ctas` as for
+ * gpblur_svgp_param_stage. */
+int gpblur_svgp_param_stage_backward(const gpblur_svgp_params* p, int D, int M, int kind, const double* stage_grad,
+                                     const float* g_kl, float* grad_bucket, int accumulate, int max_ctas,
+                                     void* stage, size_t stage_bytes, void* stream);
 
 /* Expected log-likelihood part of the ELBO.
  * Replaces DeepApproximateMLL(VariationalELBO(likelihood, model, num_data))(dist, y) built at
@@ -253,26 +198,16 @@ int gpblur_rsample_backward(const float* var, const float* g_out, long long n, u
                             uint64_t offset, uint32_t stream_id, float* g_mean, float* g_var,
                             void* stream);
 
-/* Dense ScaleKernel(RBF) covariance for the exact-GP model
- * (/root/reference/denoising_model/GPModel.py:10-13): x1 [n1, D], x2 [n2, D], one lengthscale per
- * dimension (pass the same value D times for the isotropic kernel) -> out [n1, n2]. */
-int gpblur_rbf_covariance(const float* x1, const float* x2, long long n1, long long n2, int D,
-                          const float* raw_lengthscale, int ard, const float* raw_outputscale,
-                          float* out, void* stream);
-
-/* Backward of gpblur_rbf_covariance (what autograd computes through the kernel evaluation when the exact GP of
- * /root/reference/denoising_model/GPModel.py:4-13 is trained): g_out [n1, n2] -> g_x1 [n1, D] (nullable), g_x2 [n2, D]
- * (nullable; when x2 is the same tensor as x1 the caller adds the two), g_raw_lengthscale [D] (ard) or [1],
- * g_raw_outputscale [1].  `scratch`: gpblur_rbf_covariance_backward_scratch_bytes(n1, n2, D) bytes, 256-byte aligned. */
-size_t gpblur_rbf_covariance_backward_scratch_bytes(long long n1, long long n2, int D);
-int gpblur_rbf_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D,
-                                   const float* raw_lengthscale, int ard, const float* raw_outputscale,
-                                   const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
-                                   float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream);
-/* The dense covariance and its backward for any GPBLUR_KERNEL_* `kind` (the rbf entry points are these with
- * GPBLUR_KERNEL_RBF).  The backward's scratch: gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind). */
+/* Dense ScaleKernel covariance of kind `kind` for the exact-GP model (/root/reference/denoising_model/GPModel.py:10-13):
+ * x1 [n1, D], x2 [n2, D], raw_lengthscale [D] (ard != 0) or [1] -> out [n1, n2]. */
 int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                       const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream);
+
+/* Backward of gpblur_covariance (what autograd computes through the kernel evaluation when the exact GP of
+ * /root/reference/denoising_model/GPModel.py:4-13 is trained): g_out [n1, n2] -> g_x1 [n1, D] (nullable), g_x2 [n2, D]
+ * (nullable; when x2 is the same tensor as x1 the caller adds the two), g_raw_lengthscale [D] (ard) or [1],
+ * g_raw_outputscale [1].  `scratch`: gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind) bytes, 256-byte
+ * aligned. */
 size_t gpblur_covariance_backward_scratch_bytes(long long n1, long long n2, int D, int kind);
 int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                                const float* raw_lengthscale, int ard, const float* raw_outputscale,

@@ -319,7 +319,7 @@ def test_sharded_wrapper_single_process(cuda):
 
 
 def test_param_stage_is_shared_between_calls_and_invalidated_by_updates(cuda):
-    """The enc / dec calls of one step share the M x M stage (gpblur_svgp_forward_cached); an in-place parameter
+    """The enc / dec calls of one step share the M x M stage (gpblur_svgp_param_stage); an in-place parameter
     update (optimizer step) bumps the tensor version and forces a recompute."""
     from fine_grained_gaussian_process_forcasting_b200.DeepGP import DeepGPp
     from fine_grained_gaussian_process_forcasting_b200 import gpcompat, _cabi

@@ -245,7 +245,7 @@ def test_rbf_covariance(cuda):
 @pytest.mark.parametrize("n1,n2,D,ard,same", [(37, 21, 5, False, False), (40, 40, 16, True, True), (130, 77, 64, True, False),
                                                (9, 9, 3, False, True), (17, 33, 128, True, False)])
 def test_rbf_covariance_backward(cuda, n1, n2, D, ard, same):
-    """gpblur_rbf_covariance_backward against fp64 autograd through the oracle's direct-difference kernel: gradients of
+    """gpblur_covariance_backward against fp64 autograd through the oracle's direct-difference kernel: gradients of
     both inputs (the SAME tensor on both sides for K(x, x)), raw lengthscale(s) and raw outputscale."""
     from fine_grained_gaussian_process_forcasting_b200 import ops
     g = torch.Generator().manual_seed(n1 * 7 + D)
