@@ -9,8 +9,12 @@
 //   phase 3  triangular inverse Linv = L^-1 by recursive doubling (all-GEMM, parallel over tiles)
 //   phase 4  fp32 operands for the per-point kernels: Linv^T, diag(c) Linv, beta = Linv^T m
 // backward (replaces LinalgCholeskyExBackward0 + kernel-matrix autograd):
-//   Gbar = beta u^T + 2 Linv^T diag(c) S ; Lbar = -tril(Gbar) ; Kbar = sym(Linv^T Phi(L^T Lbar) Linv)
-//   then the Kzz-path gradients of Z, lengthscale, outputscale and the final parameter bucket.
+//   Lbar = -tril(Linv^T X), X = m u^T + 2 diag(c) S ; Kbar = sym(Linv^T Phi(L^T Lbar) Linv), in closed form
+//   sym(Kbar) = Linv^T P Linv with P = -1/2 (m_hi u_lo + 2 c_hi S_hi,lo) (two products, see PForm)
+//   phase A  Tm = P Linv
+//   phase B  sym(Kbar) = Linv^T Tm, Wzz = sym(Kbar) o (Kzz - jitter I) (Matern kinds: o g(d2)) in its epilogue
+//   phase C  Kzz-path gradients of Z and the per-(i, d) lengthscale terms (V = Wzz Z~)
+//   phase D  final parameter bucket
 //
 // All matrices are [MP, MP] row-major doubles with MP a multiple of 32 (identity padding).
 #include <cooperative_groups.h>
@@ -144,8 +148,19 @@ __device__ __forceinline__ void tile_gemm(double acc[4], const MatRef& A, int r0
 // trip and two CTA barriers per 32 k).
 constexpr int KW = 256;
 constexpr int PW = KW + 2;                               // pitch (doubles): fragment loads hit every bank pair twice
+// operand buffers + k-vectors [3][KW] (m / u / c of PForm) + row vectors [3][TB] of PForm
 template <int RT>
-constexpr size_t wide_bytes() { return (size_t)(RT + TB) * PW * sizeof(double) + KW * sizeof(double); }
+constexpr size_t wide_bytes() { return ((size_t)(RT + TB) * PW + 3 * KW + 3 * TB) * sizeof(double); }
+
+// A operand of the first backward product: the staged rows of the (exactly symmetric) stage gradient S become
+//   P(r, k) = -1/2 (m_hi u_lo + 2 c_hi S(hi, lo)),  hi = max(r, k), lo = min(r, k),
+// i.e. P = (Phi + Phi^T) / 2 with Phi = Phi(L^T Lbar) = -Phi(m u^T + 2 diag(c) S) (see mm_backward_kernel).
+// m, c are 0 and u, S are 0 in the padding, so P is 0 there.
+struct PForm {
+  const float* m = nullptr;    // variational mean
+  const double* u = nullptr;   // u of the stage gradient
+  const float* c = nullptr;    // s^2 - 1
+};
 
 __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gsrc) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc)
@@ -164,18 +179,21 @@ __device__ __forceinline__ void cp_async_wait() {
 // RT = 16 or 32 rows per tile (16: up to 128 tiles per phase at M = 256, one per SM; 32: half the operand traffic
 // per flop, for the sizes where every SM has several tiles anyway).
 //  * B may be an fp32 matrix (B.pf): staged as floats, widened when the fragment is read;
-//  * kscale != nullptr: A(r, k) is multiplied by kscale[k] (fp32, global) when the fragment is read;
-//  * rowsum != nullptr (RT doubles of shared memory): receives the row sums of the A block, fixed order.
+//  * rowsum != nullptr (RT doubles of shared memory): receives the row sums of the A block, fixed order;
+//  * pform.m != nullptr: A (non-transposed) is S, and P (see PForm) is multiplied instead.
 // `wide`: wide_bytes<RT>() of shared memory.
 template <int RT>
 __device__ __forceinline__ void wide_gemm(double (&acc)[RT / 8], const MatRef& A, int r0, const MatRef& B, int c0, int k0,
-                                          int k1, double* wide, const float* kscale = nullptr, double* rowsum = nullptr) {
+                                          int k1, double* wide, double* rowsum = nullptr, PForm pform = PForm{}) {
   if (k0 >= k1) return;
   constexpr int NCB = RT / 16;                           // 8-column blocks per warp
   const int tid = threadIdx.x, tx = tid & 31, ty = tid >> 5;
   double* Aw = wide;                                     // [RT rows][k]
   double* Bw = wide + RT * PW;                           // [32 cols][k]
-  double* sc = Bw + TB * PW;                             // [k] scale of the chunk
+  double* pm = Bw + TB * PW;                             // [k] m of the chunk (PForm)
+  double* pu = pm + KW;                                  // [k] u of the chunk (PForm)
+  double* pc = pu + KW;                                  // [k] c of the chunk (PForm)
+  double* prow = pc + KW;                                // [3][RT] m, u, c of the tile rows (PForm)
   float* Bf = reinterpret_cast<float*>(Bw);              // fp32 B: [col][k], pitch 2 PW floats
   const int g = tx >> 2, t = tx & 3;
   const int rw = RT == 16 ? 8 * (ty & 1) : 8 * (ty & 3);
@@ -185,8 +203,18 @@ __device__ __forceinline__ void wide_gemm(double (&acc)[RT / 8], const MatRef& A
     const int klen = (k1 - kc) < KW ? (k1 - kc) : KW;   // multiple of 32
     const int ngroups = (klen + 63) / 64;
     __syncthreads();                                     // previous chunk / previous user of `wide` is done
-    if (kscale)
-      for (int k = tid; k < klen; k += kThreads) sc[k] = (double)kscale[kc + k];
+    if (pform.m) {
+      for (int k = tid; k < klen; k += kThreads) {
+        pm[k] = (double)pform.m[kc + k];
+        pu[k] = pform.u[kc + k];
+        pc[k] = (double)pform.c[kc + k];
+      }
+      if (tid < RT) {
+        prow[tid] = (double)pform.m[r0 + tid];
+        prow[RT + tid] = pform.u[r0 + tid];
+        prow[2 * RT + tid] = (double)pform.c[r0 + tid];
+      }
+    }
     for (int gq = 0; gq < 4; ++gq) {
       if (gq < ngroups) {
         const int kg0 = gq * 64, kgl = (klen - kg0) < 64 ? (klen - kg0) : 64;   // 64 or 32
@@ -216,6 +244,17 @@ __device__ __forceinline__ void wide_gemm(double (&acc)[RT / 8], const MatRef& A
       else cp_async_wait<0>();
       __syncthreads();
       const int kg0 = gq * 64, kgl = (klen - kg0) < 64 ? (klen - kg0) : 64;
+      if (pform.m) {
+        // S(r, k) -> P(r, k) in place; S(r, k) = S(hi, lo) because S is exactly symmetric (stage_grad_reduce_kernel)
+        const int sh = kgl == 64 ? 6 : 5;
+        for (int e = tid; e < RT * kgl; e += kThreads) {
+          const int row = e >> sh, k = kg0 + (e & (kgl - 1));
+          double& s = Aw[row * PW + k];
+          s = (kc + k >= r0 + row) ? -fma(pc[k], s, 0.5 * pm[k] * prow[RT + row])
+                                   : -fma(prow[2 * RT + row], s, 0.5 * prow[row] * pu[k]);
+        }
+        __syncthreads();
+      }
       if (rowsum) {
         // row sums of this k-group (rows ty, ty + 8, ...), fixed order: groups in sequence, shuffle tree inside
 #pragma unroll
@@ -228,11 +267,9 @@ __device__ __forceinline__ void wide_gemm(double (&acc)[RT / 8], const MatRef& A
         }
       }
       const double* ap = Aw + (rw + g) * PW + t + kg0;
-      const double* sp = sc + t + kg0;
 #pragma unroll 4
       for (int k4 = 0; k4 < kgl; k4 += 8) {
         double a0 = ap[k4], a1 = ap[k4 + 4];
-        if (kscale) { a0 *= sp[k4]; a1 *= sp[k4 + 4]; }
 #pragma unroll
         for (int cb = 0; cb < NCB; ++cb) {
           double b0, b1;
@@ -1306,11 +1343,13 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   const float* WXpart = ws_cptr<float>(a.ws, L.WXpart);
   const float* vecpart = ws_cptr<float>(a.ws, L.vecpart);
   const float* cpart = ws_cptr<float>(a.ws, L.cpart);
-  const int tp = MP < 128 ? MP : 128;   // tile size used by the Gram reduction (lower tile triangle valid)
   const bool tc = a.ncpart > 0;
-  // S region: the FFMA Gram holds only the lower tile triangle (tile size tp) of full [MP x MP] partials, read in
-  // output order (mirrored tiles transposed); the tensor-core Gram packed lower-triangle 128 x 128 blocks, read in
-  // packed order (coalesced) and written to (i, j) and, outside the diagonal blocks, to its mirror (j, i)
+  // S region: the FFMA Gram holds only the lower tile triangle (tiles of min(MP, 128)) of full [MP x MP] partials, read in
+  // output order (upper elements transposed); the tensor-core Gram packed lower-triangle 128 x 128 blocks, read in
+  // packed order (coalesced), lower elements only, each written to (i, j) and its mirror (j, i).
+  // Both paths sum the partials of the LOWER element for (i, j) and (j, i), so S is exactly symmetric: the Gram
+  // computes the two elements of a pair inside a diagonal block separately, and mm_backward_kernel's first product
+  // reads S(i, k) as S(max, min).
   const size_t n_u = MP, n_vec = L.vec_len, n_S = tc ? tc_gram_floats(MP) : (size_t)MP * MP, n_WX = (size_t)MP * DP;
   const size_t total = n_u + n_vec + n_S + n_WX;
   const size_t s_out = n_u + n_vec;   // first S element of the stage gradient
@@ -1323,6 +1362,7 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   for (size_t ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
     const size_t e = ch * 32 + lane;
     size_t dst = e, mirror = 0;   // output element(s); mirror 0: none
+    bool skip = false;            // upper element of a diagonal block (tensor-core Gram): written by its mirror
     if (e >= s_out + n_S) dst = e - n_S + (size_t)MP * MP;
     double s = 0.0;
     if (e >= s_out && e < s_out + n_S) {
@@ -1336,15 +1376,16 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
         src = Spart + idx;
         pstride = tc_gram_floats(MP);
         if (!tc_gram_diag_block(MP, i >> 7, j >> 7)) nsp = L.splitsO;
-        if ((i >> 7) != (j >> 7)) mirror = s_out + (size_t)j * MP + i;
+        skip = i < j;
+        if (i > j) mirror = s_out + (size_t)j * MP + i;
       } else {
         i = (int)(idx / MP); j = (int)(idx - (size_t)i * MP);
-        const bool lower = i / tp >= j / tp;
+        const bool lower = i >= j;
         src = Spart + (size_t)(lower ? i : j) * MP + (lower ? j : i);
         pstride = (size_t)MP * MP;
       }
       dst = s_out + (size_t)i * MP + j;
-      if (L.N > 0) {
+      if (L.N > 0 && !skip) {
         // loads batched 4 deep before the (ordered) adds: independent requests in flight
         int sp = g;
         for (; sp + 24 < nsp; sp += 32) {
@@ -1370,7 +1411,7 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
     __syncthreads();
     red[g][lane] = s;
     __syncthreads();
-    if (g == 0 && e < total) {
+    if (g == 0 && e < total && !skip) {
       double t = 0.0;
 #pragma unroll
       for (int w = 0; w < 8; ++w) t += red[w][lane];
@@ -1404,9 +1445,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   const float* mvec = ws_cptr<float>(a.ws, L.mvec);
   const float* cvec = ws_cptr<float>(a.ws, L.cvec);
   const float* svec = ws_cptr<float>(a.ws, L.svec);
-  const float* beta = ws_cptr<float>(a.ws, L.beta);
   const double* K64 = ws_cptr<double>(a.ws, L.K64);
-  const double* L64 = ws_cptr<double>(a.ws, L.L64);
   const double* Li64 = ws_cptr<double>(a.ws, L.Linv64);
   double* T64 = ws_ptr<double>(a.ws, L.T64);
   double* U64 = ws_ptr<double>(a.ws, L.U64);
@@ -1415,7 +1454,8 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   const double* vec64 = a.sgrad + MP;
   const double* S64 = vec64 + L.vec_len;
   const double* WX64 = S64 + (size_t)MP * MP;
-  // fp64 vector scratch: [row sums of sym(Kb) o (Kzz - jitter I) MP (Matern kinds) | unused vec_len | diag(S) MP | rz MP]
+  // fp64 vector scratch: [per-item sums of sym(Kb) o (Kzz - jitter I) (Matern kinds; NH nb^2 <= MP items) | unused
+  // vec_len | unused MP | rz MP]
   double* v64 = ws_ptr<double>(a.ws, L.v64);
   double* kbk64 = v64;
   double* rz64 = v64 + 2 * MP + L.vec_len;
@@ -1427,121 +1467,77 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   GPBLUR_STAMP();
 
   // Work items of the product phases: item t -> tile t / NH = (bi, bj), rows bi * 32 + RT (t % NH) .. + RT.
-  // ---------------- phase 1: Lbar = -tril( beta u^T + 2 Linv^T diag(c) S ) -> U64 ----------------
-  // (diag(c) is applied to the k index of the A operand on the fly: the former elementwise phase 0 and its barrier are gone)
+  // ---------------- phase A: Tm = P Linv -> T64 (full) ----------------
+  // P = sym(Phi(L^T Lbar)) in closed form (PForm): the lower triangle of L^T Lbar reads only the lower triangle of
+  // Lbar = -tril(Linv^T X), X = m u^T + 2 diag(c) S, and L^T Linv^T = I, so Phi(L^T Lbar) = -Phi(X); and
+  // sym(Linv^T Phi Linv) = Linv^T P Linv.  Linv is lower triangular: k runs from the column block up.
   for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
     const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
-    if (bi < bj) {
-#pragma unroll
-      for (int i = 0; i < NR; ++i) U64[(size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane] = 0.0;
-      continue;
-    }
     double acc[NR] = {};
-    wide_gemm<RT>(acc, MatRef{Li64, MP, true}, r0, MatRef{S64, MP, false}, bj * TB, bi * TB, MP, gsm, cvec);
-#pragma unroll
-    for (int i = 0; i < NR; ++i) {
-      const int gi = r0 + warp + 8 * i, gj = bj * TB + lane;
-      const double g = (double)beta[gi] * u64[gj] + 2.0 * acc[i];
-      U64[(size_t)gi * MP + gj] = (gj <= gi) ? -g : 0.0;
-    }
-  }
-  GPBLUR_GRID_SYNC();
-
-  GPBLUR_STAMP();
-  GPBLUR_STAMP();
-  // ---------------- phase 2: Phi( L^T Lbar ) -> T64 (lower) ----------------
-  for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
-    const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
-    if (bi < bj) {
-#pragma unroll
-      for (int i = 0; i < NR; ++i) T64[(size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane] = 0.0;
-      continue;
-    }
-    double acc[NR] = {};
-    wide_gemm<RT>(acc, MatRef{L64, MP, true}, r0, MatRef{U64, MP, false}, bj * TB, bi * TB, MP, gsm);
-#pragma unroll
-    for (int i = 0; i < NR; ++i) {
-      const int gi = r0 + warp + 8 * i, gj = bj * TB + lane;
-      double v = acc[i];
-      if (gj > gi) v = 0.0;
-      else if (gj == gi) v *= 0.5;
-      T64[(size_t)gi * MP + gj] = v;
-    }
-  }
-  GPBLUR_GRID_SYNC();
-
-  GPBLUR_STAMP();
-  // ---------------- phase 3: Tm = Phi Linv -> U64 (lower) ----------------
-  for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
-    const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
-    if (bi < bj) {
-#pragma unroll
-      for (int i = 0; i < NR; ++i) U64[(size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane] = 0.0;
-      continue;
-    }
-    double acc[NR] = {};
-    // sum over k in [bj-tile, bi-tile]; operand zeros handle the ragged edges inside the diagonal tiles
-    wide_gemm<RT>(acc, MatRef{T64, MP, false}, r0, MatRef{Li64, MP, false}, bj * TB, bj * TB, (bi + 1) * TB, gsm);
-#pragma unroll
-    for (int i = 0; i < NR; ++i) U64[(size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane] = acc[i];
-  }
-  GPBLUR_GRID_SYNC();
-
-  GPBLUR_STAMP();
-  // ---------------- phase 4: Kb = Linv^T Tm -> T64 (full) ----------------
-  for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
-    const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
-    const int kb0 = bi > bj ? bi : bj;
-    double acc[NR] = {};
-    wide_gemm<RT>(acc, MatRef{Li64, MP, true}, r0, MatRef{U64, MP, false}, bj * TB, kb0 * TB, MP, gsm);
+    wide_gemm<RT>(acc, MatRef{S64, MP, false}, r0, MatRef{Li64, MP, false}, bj * TB, bj * TB, MP, gsm, nullptr,
+                  PForm{mvec, u64, cvec});
 #pragma unroll
     for (int i = 0; i < NR; ++i) T64[(size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane] = acc[i];
   }
   GPBLUR_GRID_SYNC();
 
   GPBLUR_STAMP();
-  const double zz_jitter = ws_cptr<double>(a.ws, L.hyp64)[H_JIT];
-  // ---------------- phase 5: Wzz = sym(Kb) o (Kzz - jitter I) -> U64 ----------------
-  // (building Wzz on the fly while phase 6 stages its A operand was tried: the transposed read made it 2x slower)
+  // ---------------- phase B: sym(Kb) = Linv^T Tm ; Wzz = sym(Kb) o (Kzz - jitter I) -> U64 ----------------
   // Matern kinds: Wzz = sym(Kb) o g(d2) from the distances the forward kept; the outputscale term
-  // sum sym(Kb) o (Kzz - jitter I) is no longer sum Wzz: its row sums go to kbk64 (one warp per row, fixed order)
-  if constexpr (MAT) {
+  // sum sym(Kb) o (Kzz - jitter I) is no longer sum Wzz: one partial per item -> kbk64[t], added in fixed order in D
+  {
+    const double zz_jitter = hyp64[H_JIT];
     const double os = hyp64[H_OS];
     const double* D2 = ws_cptr<double>(a.ws, L.D2zz64);
-    for (int i = blockIdx.x * 8 + warp; i < MP; i += G * 8) {
-      double rs = 0.0;
-      for (int j = lane; j < MP; j += 32) {
-        const size_t idx = (size_t)i * MP + j;
+    __shared__ double kred[8];
+    for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
+      const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
+      // operands of the epilogue, requested before the product
+      double e_k[NR];
+      [[maybe_unused]] double e_d2[NR];
+#pragma unroll
+      for (int i = 0; i < NR; ++i) {
+        const size_t idx = (size_t)(r0 + warp + 8 * i) * MP + bj * TB + lane;
+        e_k[i] = K64[idx];
+        if constexpr (MAT) e_d2[i] = D2[idx];
+      }
+      double acc[NR] = {};
+      wide_gemm<RT>(acc, MatRef{Li64, MP, true}, r0, MatRef{T64, MP, false}, bj * TB, bi * TB, MP, gsm);
+      double kbk = 0.0;
+#pragma unroll
+      for (int i = 0; i < NR; ++i) {
+        const int gi = r0 + warp + 8 * i, gj = bj * TB + lane;
         double v = 0.0;
-        if (i < M && j < M) {
-          const double kb = 0.5 * (T64[idx] + T64[(size_t)j * MP + i]);
-          double kk, g;
-          kernel_kg64(L.kind, D2[idx], os, kk, g);
-          v = kb * g;
-          rs += kb * (K64[idx] - (i == j ? zz_jitter : 0.0));
+        if (gi < M && gj < M) {
+          const double kz = e_k[i] - (gi == gj ? zz_jitter : 0.0);
+          if constexpr (MAT) {
+            double kk, g;
+            kernel_kg64(L.kind, e_d2[i], os, kk, g);
+            v = acc[i] * g;
+            kbk += acc[i] * kz;
+          } else {
+            v = acc[i] * kz;
+          }
         }
-        U64[idx] = v;
+        U64[(size_t)gi * MP + gj] = v;
       }
-      rs = warp_sum(rs);
-      if (lane == 0) kbk64[i] = rs;
-    }
-    GPBLUR_GRID_SYNC();
-  } else {
-    for (int idx = gtid; idx < MP * MP; idx += gsize) {
-      const int i = idx / MP, j = idx - i * MP;
-      double v = 0.0;
-      if (i < M && j < M) {
-        const double kb = 0.5 * (T64[idx] + T64[(size_t)j * MP + i]);
-        const double kz = K64[idx] - (i == j ? zz_jitter : 0.0);
-        v = kb * kz;
+      if constexpr (MAT) {
+        kbk = warp_sum(kbk);
+        if (lane == 0) kred[warp] = kbk;
+        __syncthreads();
+        if (tid == 0) {
+          double s = 0.0;
+#pragma unroll
+          for (int w8 = 0; w8 < 8; ++w8) s += kred[w8];
+          kbk64[t] = s;
+        }
       }
-      U64[idx] = v;
     }
-    GPBLUR_GRID_SYNC();
   }
+  GPBLUR_GRID_SYNC();
 
   GPBLUR_STAMP();
-  // ---------------- phase 6: Kzz-path + a-space gradients of Z; per-(i, d) terms of d ell -------
+  // ---------------- phase C: Kzz-path + a-space gradients of Z; per-(i, d) terms of d ell -------
   // V = Wzz Z~ is an [MP, MP] x [MP, DP] product: 16 x 32 tiles on the FP64 tensor path (a thread-per-(i, d) loop over
   // j exposed one L2 round trip per few terms: 16 us at M = 256, 166 us at M = 1024); the row sums of Wzz come from
   // the staged operand with a fixed shuffle tree.
@@ -1568,7 +1564,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
         e_cs[r2] = vec64[i];
       }
       double acc[NR] = {};
-      wide_gemm<RT>(acc, MatRef{U64, MP, false}, r0, MatRef{nullptr, DP, false, Zt}, bd * TB, 0, MP, gsm, nullptr, rz_s);
+      wide_gemm<RT>(acc, MatRef{U64, MP, false}, r0, MatRef{nullptr, DP, false, Zt}, bd * TB, 0, MP, gsm, rz_s);
       double tsum = 0.0;
 #pragma unroll
       for (int r2 = 0; r2 < NR; ++r2) {
@@ -1579,7 +1575,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
           tsum += zgrad_terms(i, d, acc[r2], rz, e_wx[r2], e_z[r2], e_cs[r2]);
         }
       }
-      // column sums over the RT rows of the item (fixed order) -> t64[item row block][d]; phase 7 adds the NH nb blocks
+      // column sums over the RT rows of the item (fixed order) -> t64[item row block][d]; phase D adds the NH nb blocks
       __syncthreads();
       tred[warp][lane] = tsum;
       __syncthreads();
@@ -1611,7 +1607,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   GPBLUR_GRID_SYNC();
 
   GPBLUR_STAMP();
-  // ---------------- phase 7: final bucket (block 0) ----------------
+  // ---------------- phase D: final bucket (block 0) ----------------
   if (blockIdx.x == 0) {
     const double os = hyp64[H_OS];
     const double gkl = a.g_kl ? (double)a.g_kl[0] : 0.0;
@@ -1631,7 +1627,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
       const int d = tid % DP, part = tid / DP;
       double s = 0.0;
 #pragma unroll 8
-      const int trows = DP >= TB ? NH * nb : M;   // phase 6 leaves per-item column sums (DP >= 32) or the full terms
+      const int trows = DP >= TB ? NH * nb : M;   // phase C leaves per-item column sums (DP >= 32) or the full terms
       for (int i = part; i < trows; i += npart) s += t64[(size_t)i * DP + d];
       colred[tid] = s;
       __syncthreads();
@@ -1651,9 +1647,10 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
     if (warp == 0) {
       // sum sym(Kb) o (Kzz - jitter I) + sum kbar o k: for RBF both are the sums of the W matrices
       constexpr bool rbf = !MAT;
-      const double* rows = rbf ? rz64 : kbk64;
+      const double* parts = rbf ? rz64 : kbk64;    // row sums of Wzz | per-item sums of phase B
+      const int nparts = rbf ? M : NH * nb * nb;
       double s = 0.0;
-      for (int i = lane; i < M; i += 32) s += rows[i];
+      for (int i = lane; i < nparts; i += 32) s += parts[i];
       s = warp_sum(s);
       if (lane == 0) {
         const double dos = (s + sc[rbf ? VS_RSUM : VS_KBK]) / os + sc[VS_GVAR];
@@ -1667,26 +1664,25 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   (void)hyp;
 }
 
-// MP = 32: the backward of the one-block stage in ONE CTA (see mm_small_forward_kernel).  All operands (S, L, L^-1, Kzz,
-// Z~, W^T X: < 70 KB) are fetched into shared memory in one round trip; the chain of four 32 x 32 x 32 products, the
-// Kzz-path terms and the final bucket then run between CTA barriers instead of grid barriers + L2 round trips
+// MP = 32: the backward of the one-block stage in ONE CTA (see mm_small_forward_kernel).  All operands (S, L^-1, Kzz,
+// Z~, W^T X: < 60 KB) are fetched into shared memory in one round trip; the two 32 x 32 x 32 products of sym(Kbar),
+// the Kzz-path terms and the final bucket then run between CTA barriers instead of grid barriers + L2 round trips
 // (general kernel at M = 32: 23 us in-kernel, 45 us with the cooperative launch around it).
-constexpr size_t kSmallBwdSmem = (size_t)(6 * TB * TLD + 2 * TB * (GPBLUR_MAX_D + 1) + 6 * TB + GPBLUR_MAX_D + 8) * sizeof(double);
+constexpr size_t kSmallBwdSmem = (size_t)(5 * TB * TLD + 2 * TB * (GPBLUR_MAX_D + 1) + 6 * TB + GPBLUR_MAX_D + 8) * sizeof(double);
 
 template <bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* Ss = reinterpret_cast<double*>(smem_raw);   // [32][33] S (stage gradient), later Wzz
   double* Li = Ss + TB * TLD;                         // L^-1
-  double* Lm = Li + TB * TLD;                         // L
-  double* Kz = Lm + TB * TLD;                         // Kzz + jitter
-  double* Us = Kz + TB * TLD;                         // Lbar, then Tm
-  double* Ts = Us + TB * TLD;                         // Phi, then Kbar
+  double* Kz = Li + TB * TLD;                         // Kzz + jitter
+  double* Us = Kz + TB * TLD;                         // P, then sym(Kbar) o (Kzz - jitter I) (Matern kinds)
+  double* Ts = Us + TB * TLD;                         // Tm
   double* Zd = Ts + TB * TLD;                         // [32][DP + 1] Z~ (double)
   double* Wx = Zd + TB * (GPBLUR_MAX_D + 1);          // [32][DP + 1] W^T X (stage gradient)
   double* u_s = Wx + TB * (GPBLUR_MAX_D + 1);         // [32]
-  double* beta_s = u_s + TB;                          // [32]
-  double* c_s = beta_s + TB;                          // [32]
+  double* m_s = u_s + TB;                             // [32]
+  double* c_s = m_s + TB;                             // [32]
   double* cs_s = c_s + TB;                            // [32] colsum(W)
   double* rz_s = cs_s + TB;                           // [32] row sums of Wzz
   double* tcol = rz_s + TB;                           // [DP] column sums of the lengthscale terms
@@ -1702,9 +1698,7 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   const float* mvec = ws_cptr<float>(a.ws, L.mvec);
   const float* cvec = ws_cptr<float>(a.ws, L.cvec);
   const float* svec = ws_cptr<float>(a.ws, L.svec);
-  const float* beta = ws_cptr<float>(a.ws, L.beta);
   const double* K64 = ws_cptr<double>(a.ws, L.K64);
-  const double* L64 = ws_cptr<double>(a.ws, L.L64);
   const double* Li64 = ws_cptr<double>(a.ws, L.Linv64);
   const double* u64 = a.sgrad;
   const double* vec64 = a.sgrad + MP;
@@ -1719,7 +1713,6 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     const int r = warp + 8 * i;
     Ss[r * TLD + lane] = S64[(size_t)r * MP + lane];
     Li[r * TLD + lane] = Li64[(size_t)r * MP + lane];
-    Lm[r * TLD + lane] = L64[(size_t)r * MP + lane];
     Kz[r * TLD + lane] = K64[(size_t)r * MP + lane];
   }
   for (int idx = tid; idx < MP * DP; idx += kThreads) {
@@ -1729,7 +1722,7 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   }
   if (tid < MP) {
     u_s[tid] = u64[tid];
-    beta_s[tid] = (double)beta[tid];
+    m_s[tid] = (double)mvec[tid];
     c_s[tid] = (double)cvec[tid];
     cs_s[tid] = vec64[tid];
   }
@@ -1737,58 +1730,25 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   __syncthreads();
 
   // out(r, lane) for r = warp + 8 i:  sum_k A(r, k) B(k, lane), A / B given as element functions of shared memory
-  // ---- phase 1: Lbar = -tril( beta u^T + 2 Linv^T diag(c) S ) -> Us ----
+  // ---- phase A: P = sym(Phi(L^T Lbar)) = -1/2 (m_hi u_lo + 2 c_hi S_hi,lo) -> Us (see PForm); Tm = P Linv -> Ts ----
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int r = warp + 8 * i;
+    const int hi = r > lane ? r : lane, lo = r > lane ? lane : r;
+    Us[r * TLD + lane] = -fma(c_s[hi], Ss[hi * TLD + lo], 0.5 * m_s[hi] * u_s[lo]);
+  }
+  __syncthreads();
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int r = warp + 8 * i;
     double acc = 0.0;
-    for (int k = 0; k < TB; ++k) acc = fma(Li[k * TLD + r] * c_s[k], Ss[k * TLD + lane], acc);
-    const double g = beta_s[r] * u_s[lane] + 2.0 * acc;
-    Us[r * TLD + lane] = (lane <= r) ? -g : 0.0;
+    for (int k = 0; k < TB; ++k) acc = fma(Us[r * TLD + k], Li[k * TLD + lane], acc);
+    Ts[r * TLD + lane] = acc;
   }
   __syncthreads();
-  // ---- phase 2: Phi( L^T Lbar ) -> Ts (lower, halved diagonal) ----
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int r = warp + 8 * i;
-    double acc = 0.0;
-    for (int k = 0; k < TB; ++k) acc = fma(Lm[k * TLD + r], Us[k * TLD + lane], acc);
-    Ts[r * TLD + lane] = lane > r ? 0.0 : (lane == r ? 0.5 * acc : acc);
-  }
-  __syncthreads();
-  // ---- phase 3: Tm = Phi Linv -> Us ----
-  {
-    double o[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = warp + 8 * i;
-      double acc = 0.0;
-      for (int k = 0; k < TB; ++k) acc = fma(Ts[r * TLD + k], Li[k * TLD + lane], acc);
-      o[i] = acc;
-    }
-    __syncthreads();                       // (phase 2 results fully consumed before Us is overwritten - Us is not read
-#pragma unroll                             //  in phase 3, but keep the phases cleanly separated)
-    for (int i = 0; i < 4; ++i) Us[(warp + 8 * i) * TLD + lane] = o[i];
-  }
-  __syncthreads();
-  // ---- phase 4: Kbar = Linv^T Tm -> Ts (full) ----
-  {
-    double o[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = warp + 8 * i;
-      double acc = 0.0;
-      for (int k = 0; k < TB; ++k) acc = fma(Li[k * TLD + r], Us[k * TLD + lane], acc);
-      o[i] = acc;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) Ts[(warp + 8 * i) * TLD + lane] = o[i];
-  }
-  __syncthreads();
-  // ---- phase 5: Wzz = sym(Kbar) o (Kzz - jitter I) -> Ss ; row sums ----
+  // ---- phase B: sym(Kbar) = Linv^T Tm ; Wzz = sym(Kbar) o (Kzz - jitter I) -> Ss ; row sums ----
   // (Matern kinds: Wzz = sym(Kbar) o g(d2); the products sym(Kbar) o (Kzz - jitter I) of the outputscale term are
-  //  parked in Us, free since phase 4, and summed into kbk)
+  //  parked in Us, free since phase A, and summed into kbk)
   constexpr bool rbf = !MAT;
   double kbk = 0.0;
   {
@@ -1798,13 +1758,14 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int r = warp + 8 * i;
+      double kb = 0.0;
+      for (int k = 0; k < TB; ++k) kb = fma(Li[k * TLD + r], Ts[k * TLD + lane], kb);
       double v = 0.0;
       if (rbf) {
-        if (r < M && lane < M) v = 0.5 * (Ts[r * TLD + lane] + Ts[lane * TLD + r]) * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
+        if (r < M && lane < M) v = kb * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
       } else {
         double u = 0.0;
         if (r < M && lane < M) {
-          const double kb = 0.5 * (Ts[r * TLD + lane] + Ts[lane * TLD + r]);
           double kk, g;
           kernel_kg64(L.kind, D2[(size_t)r * MP + lane], os, kk, g);
           v = kb * g;
@@ -1826,8 +1787,8 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     kbk = warp_sum(kbk);
   }
   __syncthreads();
-  // (diag(S) of the stage gradient is needed in phase 7 and Ss now holds Wzz: it is re-read from global memory there)
-  // ---- phase 6: V = Wzz Z~ ; Kzz-path + a-space gradients of Z ; per-(i, d) lengthscale terms ----
+  // (diag(S) of the stage gradient is needed in phase D and Ss now holds Wzz: it is re-read from global memory there)
+  // ---- phase C: V = Wzz Z~ ; Kzz-path + a-space gradients of Z ; per-(i, d) lengthscale terms ----
   for (int d0 = 0; d0 < DP; d0 += TB) {
     const int d = d0 + lane;
     double tsum = 0.0;
@@ -1857,7 +1818,7 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     }
     __syncthreads();
   }
-  // ---- phase 7: final bucket ----
+  // ---- phase D: final bucket ----
   {
     const double os = hyp64[H_OS];
     const double gkl = a.g_kl ? (double)a.g_kl[0] : 0.0;
@@ -1891,7 +1852,7 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
       }
     }
   }
-  if (tid == 0) { const unsigned long long t = global_ns(); for (int k = 1; k < 9; ++k) stamps[k] = t; }
+  if (tid == 0) { const unsigned long long t = global_ns(); for (int k = 1; k < 5; ++k) stamps[k] = t; }
 }
 
 // Cooperative launches + cg grid.sync() by default.  GPBLUR_MM_COOP=0: plain launches + a counter barrier on a word

@@ -20,8 +20,8 @@ for M in (32, 128, 256, 1024):
     torch.cuda.synchronize()
     t = ops.debug_fetch(4, B * L, D, M, ws).cpu().tolist()
     f = [(t[i + 1] - t[i]) / 1e3 for i in range(0, 7)]
-    b = [(t[16 + i + 1] - t[16 + i]) / 1e3 for i in range(0, 8)]
+    b = [(t[16 + i + 1] - t[16 + i]) / 1e3 for i in range(0, 4)]
     print(f"M={M}: fwd phases us [p0, p1 Kzz, p2 chol+inv, -, -, p4 fp32 operands, TF32 slab images] = {[round(v,1) for v in f]} total {sum(f):.1f}")
     print(f"        tail (not in the total): beta {(t[13]-t[7])/1e3:.1f} us, zn {(t[8]-t[13])/1e3:.1f} us")
     print(f"        first diagonal block: load {(t[10]-t[9])/1e3:.1f} us, chol32 {(t[11]-t[10])/1e3:.1f} us, trinv32 {(t[12]-t[11])/1e3:.1f} us")
-    print(f"        bwd phases us [p0 reduce, p1, p2, p3, p4, p5, p6, p7] = {[round(v,1) for v in b]} total {sum(b):.1f}")
+    print(f"        bwd phases us [A Tm = P Linv, B sym(Kbar) + Wzz, C V = Wzz Z~, D bucket] = {[round(v,1) for v in b]} total {sum(b):.1f}")
