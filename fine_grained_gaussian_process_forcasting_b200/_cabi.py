@@ -17,7 +17,7 @@ GPBLUR_MAX_D = 128
 GPBLUR_MAX_M = 1024
 
 # covariance functions (GPBLUR_KERNEL_*): name used by ops.py -> kind
-KERNEL_KINDS = {"rbf": 0, "matern12": 1, "matern32": 2, "matern52": 3}
+KERNEL_KINDS = {"rbf": 0, "matern12": 1, "matern32": 2, "matern52": 3, "rq": 4}
 
 ERRORS = {
     -1: "GPBLUR_EINVAL (bad shape / null pointer / misaligned workspace)",
@@ -37,12 +37,14 @@ class SvgpParams(C.Structure):
         ("variational_stddev", C.c_void_p),
         ("mean_weights", C.c_void_p),
         ("mean_bias", C.c_void_p),
+        ("raw_alpha", C.c_void_p),
     ]
 
 
 # name -> (restype, argtypes); must list every symbol declared in include/gpblur.h
 SIGNATURES = {
     "gpblur_svgp_grad_bucket_floats": (C.c_size_t, [C.c_int, C.c_int]),
+    "gpblur_svgp_grad_bucket_floats_kind": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "gpblur_svgp_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_int, C.c_int, C.c_int]),
     "gpblur_svgp_forward": (C.c_int, [
         C.POINTER(SvgpParams), C.c_void_p, C.c_longlong, C.c_int, C.c_int,
@@ -54,6 +56,7 @@ SIGNATURES = {
         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_svgp_stage_grad_doubles": (C.c_size_t, [C.c_int, C.c_int]),
+    "gpblur_svgp_stage_grad_doubles_kind": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "gpblur_svgp_param_stage": (C.c_int, [
         C.POINTER(SvgpParams), C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
         C.c_size_t, C.c_void_p]),
@@ -70,10 +73,17 @@ SIGNATURES = {
     "gpblur_covariance": (C.c_int, [
         C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
         C.c_void_p, C.c_void_p]),
+    "gpblur_covariance_alpha": (C.c_int, [
+        C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+        C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpblur_covariance_backward_scratch_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong, C.c_int, C.c_int]),
     "gpblur_covariance_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int,
                                              C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gpblur_covariance_backward_alpha": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int,
+                                                   C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_size_t, C.c_void_p]),
     "gpblur_step_scratch_floats": (C.c_size_t, [C.c_int]),
     "gpblur_blur_apply_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int,
                                             C.c_void_p, C.c_void_p]),

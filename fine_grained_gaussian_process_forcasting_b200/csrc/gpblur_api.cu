@@ -249,11 +249,12 @@ __global__ void rsample_bwd_kernel(const float* __restrict__ var, const float* _
   g_var[i] = g * philox_normal(seed, offset + (uint64_t)i, stream_id) * 0.5f * rsqrtf(var[i]);
 }
 
-// dense ScaleKernel(RBF | Matern): 16 x 16 output tile per CTA, direct differences
+// dense ScaleKernel(RBF | Matern | RQ): 16 x 16 output tile per CTA, direct differences
 template <int KIND>
 __global__ void rbf_cov_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n1,
                                long long n2, int D, const float* __restrict__ raw_ell, int ard,
-                               const float* __restrict__ raw_os, float* __restrict__ out) {
+                               const float* __restrict__ raw_os, const float* __restrict__ raw_alpha,
+                               float* __restrict__ out) {
   __shared__ float a[16][33], b[16][33], ie[32];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const long long i0 = (long long)blockIdx.y * 16, j0 = (long long)blockIdx.x * 16;
@@ -288,6 +289,11 @@ __global__ void rbf_cov_kernel(const float* __restrict__ x1, const float* __rest
     const float os = r > 20.f ? r : log1pf(expf(r));
     if constexpr (KIND == GPBLUR_KERNEL_RBF) {
       out[(size_t)i * n2 + j] = os * expf(-0.5f * acc);
+    } else if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+      const float ra = raw_alpha[0], alpha = ra > 20.f ? ra : log1pf(expf(ra));
+      float k, g, ka;
+      rq_kg(acc, os, alpha, 0.5f / alpha, k, g, ka);
+      out[(size_t)i * n2 + j] = k;
     } else {
       float k, g;
       matern_kg<KIND>(acc, os, k, g);
@@ -321,6 +327,11 @@ extern "C" {
 
 size_t gpblur_svgp_grad_bucket_floats(int D, int M) { return (size_t)M * D + 2 * (size_t)M + 2 * (size_t)D + 2; }
 
+size_t gpblur_svgp_grad_bucket_floats_kind(int D, int M, int kind) {
+  if (!kernel_kind_valid(kind)) return 0;
+  return gpblur_svgp_grad_bucket_floats(D, M) + (kind == GPBLUR_KERNEL_RQ ? 1 : 0);
+}
+
 size_t gpblur_svgp_workspace_bytes(long long N, int D, int M, int training) {
   if (N < 0 || D < 1 || M < 1 || D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return 0;
   return make_layout(N, D, M, training).total;
@@ -349,6 +360,7 @@ static int check_stage(const gpblur_svgp_params* p, int D, int M, int kind, cons
   const int rc = validate(p, 0, D, M);
   if (rc) return rc;
   if (!kernel_kind_valid(kind) || !aligned256(stage)) return GPBLUR_EINVAL;
+  if (kind == GPBLUR_KERNEL_RQ && !p->raw_alpha) return GPBLUR_EINVAL;
   *L = make_layout(0, D, M, 0);
   L->kind = kind;
   return stage_bytes < L->total ? GPBLUR_EWORKSPACE : GPBLUR_OK;
@@ -387,9 +399,11 @@ size_t gpblur_svgp_param_stage_bytes(int D, int M) {
   return make_layout(0, D, M, 0).total;   // the inference layout is exactly the parameter stage
 }
 
-size_t gpblur_svgp_stage_grad_doubles(int D, int M) {
-  if (D < 1 || M < 1 || D > GPBLUR_MAX_D || M > GPBLUR_MAX_M) return 0;
-  return stage_grad_doubles(padded_m(M), padded_d(D));
+size_t gpblur_svgp_stage_grad_doubles(int D, int M) { return gpblur_svgp_stage_grad_doubles_kind(D, M, GPBLUR_KERNEL_RBF); }
+
+size_t gpblur_svgp_stage_grad_doubles_kind(int D, int M, int kind) {
+  if (D < 1 || M < 1 || D > GPBLUR_MAX_D || M > GPBLUR_MAX_M || !kernel_kind_valid(kind)) return 0;
+  return stage_grad_doubles(padded_m(M), padded_d(D), kind);
 }
 
 int gpblur_svgp_param_stage(const gpblur_svgp_params* p, int D, int M, int kind, double extra_jitter, int max_ctas,
@@ -557,23 +571,33 @@ int gpblur_rsample_backward(const float* var, const float* g_out, long long n, u
 
 int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                       const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream) {
+  return gpblur_covariance_alpha(x1, x2, n1, n2, D, kind, raw_lengthscale, ard, raw_outputscale, nullptr, out, stream);
+}
+
+int gpblur_covariance_alpha(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                            const float* raw_lengthscale, int ard, const float* raw_outputscale, const float* raw_alpha,
+                            float* out, void* stream) {
   if (n1 < 0 || n2 < 0 || D < 1 || !raw_lengthscale || !raw_outputscale || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
+  if (kind == GPBLUR_KERNEL_RQ && !raw_alpha) return GPBLUR_EINVAL;
   if (n1 == 0 || n2 == 0) return GPBLUR_OK;
   if (!x1 || !x2 || !out) return GPBLUR_EINVAL;
   dim3 grid((unsigned)((n2 + 15) / 16), (unsigned)((n1 + 15) / 16));
   cudaStream_t st = (cudaStream_t)stream;
   switch (kind) {
     case GPBLUR_KERNEL_MATERN12:
-      rbf_cov_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, out);
       break;
     case GPBLUR_KERNEL_MATERN32:
-      rbf_cov_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, out);
       break;
     case GPBLUR_KERNEL_MATERN52:
-      rbf_cov_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      rbf_cov_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, out);
+      break;
+    case GPBLUR_KERNEL_RQ:
+      rbf_cov_kernel<GPBLUR_KERNEL_RQ><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, out);
       break;
     default:
-      rbf_cov_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, out);
+      rbf_cov_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, out);
   }
   note_launch();
   return check_launch("rbf_cov");

@@ -17,19 +17,24 @@ constexpr int kKS = 16;                 // K-slice depth of the staged operand t
 constexpr int kMaxPersist = 296;        // persistent CTAs of the backward point kernel (2 x 148 SMs)
 constexpr int kMaxSplits = 148;          // split-K factor cap of the N-reduction GEMMs
 
-// hyp (fp32) slots
-enum { H_OS = 0, H_JIT = 1, H_CWB = 2, H_KL = 3, H_COUNT = 8 };
+// hyp (fp32) slots; H_ALPHA / H_I2A: alpha and 1 / (2 alpha) of the rational quadratic kind (hyp64: H_ALPHA only)
+enum { H_OS = 0, H_JIT = 1, H_CWB = 2, H_KL = 3, H_ALPHA = 4, H_I2A = 5, H_COUNT = 8 };
 constexpr int kStampSlots = 32;   // phase timestamps (globaltimer ns) of the M x M kernels: [0,16) forward, [16,32) backward
-// per-CTA vector partial layout of the backward point kernel: [colsum MP | q DP | wbar DP | scalars 4]
-// VS_KBK = sum kbar o k: the outputscale gradient of the Matern kinds (for RBF, W = kbar o k and VS_RSUM is that sum)
-enum { VS_GMU = 0, VS_RSUM = 1, VS_GVAR = 2, VS_KBK = 3, VS_COUNT = 4 };
+// per-CTA vector partial layout of the backward point kernels: [colsum MP | q DP | wbar DP | scalars VS_PART]
+// VS_KBK = sum kbar o k: the outputscale gradient of the Matern and RQ kinds (for RBF, W = kbar o k and VS_RSUM is that
+// sum); VS_KBA = sum kbar o dk/dalpha (RQ only).  The stage gradient keeps the first VS_COUNT scalars in its vector
+// section (vec_len) and VS_KBA, for RQ only, as its last element (stage_grad_doubles), so that its layout is the same
+// for every other kind.
+enum { VS_GMU = 0, VS_RSUM = 1, VS_GVAR = 2, VS_KBK = 3, VS_COUNT = 4, VS_KBA = 4, VS_PART = 5 };
 
 // ---- covariance functions (GPBLUR_KERNEL_*, include/gpblur.h) ----------------------------------------------------
 // k = os f(r) with r = sqrt(max(d2, 1e-30)), and g = -2 os df/d(d2) = -os f'(r) / r: every distance gradient is the RBF
 // one with W = kbar o g in place of kbar o k (for RBF g = k).  g = 0 where the clamp is active (d2 <= 1e-30).  Every
-// kernel site evaluates the Matern kinds through these functions; the RBF sites keep their own exp.
+// kernel site evaluates the Matern and RQ kinds through these functions; the RBF sites keep their own exp.
+// Rational quadratic (no clamp: d2 enters directly): u = d2 / (2 alpha), k = os (1 + u)^-alpha, g = k / (1 + u), and
+// ka = dk/dalpha = k (u / (1 + u) - log1p(u)).
 __host__ __device__ constexpr bool kernel_kind_valid(int kind) {
-  return kind >= GPBLUR_KERNEL_RBF && kind <= GPBLUR_KERNEL_MATERN52;
+  return kind >= GPBLUR_KERNEL_RBF && kind <= GPBLUR_KERNEL_RQ;
 }
 __device__ __forceinline__ float ex2_fast(float v) {
   float y;
@@ -59,9 +64,26 @@ __device__ __forceinline__ void matern_kg(float d2, float os, float& k, float& g
     g = live ? (5.0f / 3.0f) * p * e : 0.f;
   }
 }
-// fp64 (the M x M stage): any kind
-__device__ __forceinline__ void kernel_kg64(int kind, double d2, double os, double& k, double& g) {
+// fp32 rational quadratic: alpha and i2a = 1 / (2 alpha) from hyp[H_ALPHA] / hyp[H_I2A].  log1pf, not log2(1 + u):
+// near the RBF limit (alpha >~ 1e2, u ~ 1e-3) 1 + u rounds and would cost ~1e-4 relative in k.  The caller zeroes
+// padded columns.
+__device__ __forceinline__ void rq_kg(float d2, float os, float alpha, float i2a, float& k, float& g, float& ka) {
+  const float u = d2 * i2a, lp = log1pf(u), q = __frcp_rn(1.0f + u);
+  k = os * ex2_fast(-1.4426950408889634f * alpha * lp);
+  g = k * q;
+  ka = k * (u * q - lp);
+}
+// fp64 (the M x M stage): any kind; ka = dk/dalpha is set for RQ only (alpha is read for RQ only)
+__device__ __forceinline__ void kernel_kg64(int kind, double d2, double os, double alpha, double& k, double& g,
+                                            double& ka) {
   if (kind == GPBLUR_KERNEL_RBF) { k = os * exp(-0.5 * d2); g = k; return; }
+  if (kind == GPBLUR_KERNEL_RQ) {
+    const double u = d2 / (2.0 * alpha), lp = log1p(u), q = 1.0 / (1.0 + u);
+    k = os * exp(-alpha * lp);
+    g = k * q;
+    ka = k * (u * q - lp);
+    return;
+  }
   const double r = sqrt(fmax(d2, 1e-30));
   const bool live = d2 > 1e-30;
   if (kind == GPBLUR_KERNEL_MATERN12) {
@@ -106,7 +128,8 @@ struct WsLayout {
   int splitsS, splitsZ;     // split-K factors of the Gram (its diagonal bands on the tensor-core path) / W^T X
   int splitsO;              // tensor-core path: split-K factor of the off-diagonal Gram units (0: none, MP <= 256)
   int nvec;                 // number of per-CTA vector partials (persistent backward CTAs)
-  int vec_len;              // floats per vector partial
+  int vec_len;              // doubles of the stage gradient's vector section: MP + 2 DP + VS_COUNT
+  int vp_len;               // floats per vector partial: MP + 2 DP + VS_PART
   // byte offsets
   size_t hyp, hyp64, stamps, inv_ell, ell, center, wl, Zt, ZtT, zn, znc, mvec, cvec, svec, beta;
   size_t K64, L64, Linv64, T64, U64, LinvT32, LC32, Linv32, LCT32;
@@ -236,6 +259,16 @@ inline int choose_splits(long long N, int ntiles) {
 // (measured at c2 on B200: 0.6 / 1.0 / 1.5 gave 0.362 / 0.351 / 0.359 ms per step)
 constexpr double kWxCost = 1.0;
 
+// "Stage gradient": everything the per-point backward of ONE call contributes to the parameter gradients, reduced
+// over that call's points (fp64, fixed summation order).  It is linear in the upstream gradients, so the stage
+// gradients of several calls that share one parameter stage are simply added before the M x M backward runs once.
+//   [ u MP | vec vec_len (colsum MP, q DP, wbar DP, scalars) | S MP x MP (full, symmetric) | W^T X  MP x DP |
+//     RQ only: sum kbar o dk/dalpha ]
+__host__ __device__ inline size_t stage_grad_doubles(int MP, int DP, int kind) {
+  return (size_t)MP + (size_t)(MP + 2 * DP + VS_COUNT) + (size_t)MP * MP + (size_t)MP * DP +
+         (kind == GPBLUR_KERNEL_RQ ? 1 : 0);
+}
+
 inline WsLayout make_layout(long long N, int D, int M, int training) {
   WsLayout w;
   w.N = N; w.D = D; w.M = M; w.training = training; w.kind = GPBLUR_KERNEL_RBF;
@@ -304,6 +337,7 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
   }
   w.nvec = kMaxPersist;
   w.vec_len = w.MP + 2 * w.DP + VS_COUNT;
+  w.vp_len = w.MP + 2 * w.DP + VS_PART;
   w.v64 = take((size_t)(3 * MP + w.vec_len) * 8);
   w.t64 = take((size_t)MP * DP * 8);
   w.D2zz64 = take(MP * MP * 8);      // last region of the parameter stage: the offsets before it do not depend on it
@@ -317,11 +351,11 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
     w.Spart = take((size_t)(w.splitsS > w.splitsO ? w.splitsS : w.splitsO) * MP * MP * 4);
     w.upart = take((size_t)w.splitsS * MP * 4);
     w.WXpart = take((size_t)w.splitsZ * MP * DP * 4);
-    w.vecpart = take((size_t)w.nvec * w.vec_len * 4);
+    w.vecpart = take((size_t)w.nvec * w.vp_len * 4);
     w.gsc = take((size_t)2 * (N > 0 ? N : 1) * 4);   // folded upstream grads g_mu, g_var [N] each
     w.rrow = take((size_t)(N > 0 ? N : 1) * 4);           // row sums r[n] of W (tensor-core backward)
     w.cpart = take((size_t)w.splitsZ * MP * 4);           // column sums of W per split (tensor-core W^T X)
-    w.sgrad = take(((size_t)MP + w.vec_len + (size_t)MP * MP + (size_t)MP * DP) * 8);   // see stage_grad_doubles()
+    w.sgrad = take(stage_grad_doubles(w.MP, w.DP, GPBLUR_KERNEL_RQ) * 8);   // the longest stage gradient
   } else {
     w.A = w.W = w.Spart = w.upart = w.WXpart = w.vecpart = w.gsc = w.rrow = w.cpart = w.sgrad = o;
   }
@@ -329,13 +363,6 @@ inline WsLayout make_layout(long long N, int D, int M, int training) {
   return w;
 }
 
-// "Stage gradient": everything the per-point backward of ONE call contributes to the parameter gradients, reduced
-// over that call's points (fp64, fixed summation order).  It is linear in the upstream gradients, so the stage
-// gradients of several calls that share one parameter stage are simply added before the M x M backward runs once.
-//   [ u MP | vec vec_len (colsum MP, q DP, wbar DP, scalars) | S MP x MP (full, symmetric) | W^T X  MP x DP ]
-__host__ __device__ inline size_t stage_grad_doubles(int MP, int DP) {
-  return (size_t)MP + (size_t)(MP + 2 * DP + VS_COUNT) + (size_t)MP * MP + (size_t)MP * DP;
-}
 
 template <typename T>
 __host__ __device__ inline T* ws_ptr(void* ws, size_t off) {

@@ -12,7 +12,7 @@
 //   Lbar = -tril(Linv^T X), X = m u^T + 2 diag(c) S ; Kbar = sym(Linv^T Phi(L^T Lbar) Linv), in closed form
 //   sym(Kbar) = Linv^T P Linv with P = -1/2 (m_hi u_lo + 2 c_hi S_hi,lo) (two products, see PForm)
 //   phase A  Tm = P Linv
-//   phase B  sym(Kbar) = Linv^T Tm, Wzz = sym(Kbar) o (Kzz - jitter I) (Matern kinds: o g(d2)) in its epilogue
+//   phase B  sym(Kbar) = Linv^T Tm, Wzz = sym(Kbar) o (Kzz - jitter I) (Matern / RQ kinds: o g(d2)) in its epilogue
 //   phase C  Kzz-path gradients of Z and the per-(i, d) lengthscale terms (V = Wzz Z~)
 //   phase D  final parameter bucket
 //
@@ -473,6 +473,14 @@ __device__ __forceinline__ void park_operand(double* dst, const double (&v)[4], 
   }
 }
 
+// RQ: alpha (fp64 and fp32) and 1 / (2 alpha) (fp32) for the point kernels and the backward
+__device__ __forceinline__ void set_alpha(float* hyp, double* hyp64, const float* raw_alpha) {
+  const double alpha = softplus64((double)raw_alpha[0]);
+  hyp64[H_ALPHA] = alpha;
+  hyp[H_ALPHA] = (float)alpha;
+  hyp[H_I2A] = (float)(0.5 / alpha);
+}
+
 struct MmFwdArgs {
   gpblur_svgp_params p;
   WsLayout L;
@@ -485,7 +493,7 @@ struct MmFwdArgs {
   unsigned* flags;       // two zeroed words: diagonal blocks published, worker arrivals (phase 2)
 };
 
-// MAT: a Matern kind (L.kind); the RBF instantiation carries none of the Matern code
+// MAT: any kind but RBF (L.kind, evaluated through kernel_kg64); the RBF instantiation carries none of that code
 template <bool MAT>
 __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
   cg::grid_group grid = cg::this_grid();
@@ -545,6 +553,7 @@ __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
   // built by the worker CTAs of phase 2 while CTA 0 factorises the first diagonal block.
   {
     const double os = softplus64((double)a.p.raw_outputscale[0]);
+    const double alpha = MAT && L.kind == GPBLUR_KERNEL_RQ ? softplus64((double)a.p.raw_alpha[0]) : 0.0;
     const int ntiles = nb * (nb + 1) / 2;
     const int tx = lane, ty = warp;
     for (int t = p1_id; t >= 0 && t < ntiles; t += p1_n) {
@@ -600,8 +609,8 @@ __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
           if constexpr (!MAT) {
             kv = os * exp(-0.5 * acc[i]) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
           } else {
-            double kk, g;
-            kernel_kg64(L.kind, acc[i], os, kk, g);
+            double kk, g, ka;
+            kernel_kg64(L.kind, acc[i], os, alpha, kk, g, ka);
             kv = kk + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
             D2[(size_t)gi * MP + gj] = acc[i];
             D2[(size_t)gj * MP + gi] = acc[i];
@@ -658,6 +667,7 @@ __global__ void __launch_bounds__(kThreads) mm_forward_kernel(MmFwdArgs a) {
       hyp[H_KL] = (float)(0.5 * t);
       hyp64[H_OS] = os;
       hyp64[H_KL] = 0.5 * t;
+      if (MAT && L.kind == GPBLUR_KERNEL_RQ) set_alpha(hyp, hyp64, a.p.raw_alpha);
       if (a.kl) a.kl[0] = (float)(0.5 * t);
       if (a.info) a.info[0] = 0;
     }
@@ -1188,6 +1198,7 @@ __global__ void __launch_bounds__(kThreads) mm_small_forward_kernel(MmFwdArgs a)
       hyp[H_KL] = (float)(0.5 * part);
       hyp64[H_OS] = os;
       hyp64[H_KL] = 0.5 * part;
+      if (MAT && L.kind == GPBLUR_KERNEL_RQ) set_alpha(hyp, hyp64, a.p.raw_alpha);
       if (a.kl) a.kl[0] = (float)(0.5 * part);
       if (a.info) a.info[0] = 0;
     }
@@ -1224,8 +1235,8 @@ __global__ void __launch_bounds__(kThreads) mm_small_forward_kernel(MmFwdArgs a)
         if constexpr (!MAT) {
           kv = os * exp(-0.5 * acc) + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
         } else {
-          double kk, g;
-          kernel_kg64(L.kind, acc, os, kk, g);
+          double kk, g, ka;
+          kernel_kg64(L.kind, acc, os, hyp64[H_ALPHA], kk, g, ka);
           kv = kk + (gi == gj ? (double)kJitter + a.extra_jitter : 0.0);
           ws_ptr<double>(a.ws, L.D2zz64)[(size_t)gi * MP + gj] = acc;
         }
@@ -1318,7 +1329,7 @@ struct MmBwdArgs {
   gpblur_svgp_params p;
   WsLayout L;
   void* ws;               // parameter stage (fp64 scratch regions T64 / U64 / v64 / t64 are overwritten)
-  const double* sgrad;    // summed stage gradient [u | vec | S | W^T X], see stage_grad_doubles()
+  const double* sgrad;    // summed stage gradient [u | vec | S | W^T X (| RQ: sum kbar o dk/dalpha)], stage_grad_doubles()
   const float* g_kl;
   float* bucket;
   int accumulate;         // != 0: add into `bucket` (it is the caller's live gradient buffer) instead of overwriting it
@@ -1351,7 +1362,8 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
   // computes the two elements of a pair inside a diagonal block separately, and mm_backward_kernel's first product
   // reads S(i, k) as S(max, min).
   const size_t n_u = MP, n_vec = L.vec_len, n_S = tc ? tc_gram_floats(MP) : (size_t)MP * MP, n_WX = (size_t)MP * DP;
-  const size_t total = n_u + n_vec + n_S + n_WX;
+  const size_t n_kba = L.kind == GPBLUR_KERNEL_RQ ? 1 : 0;   // RQ: sum kbar o dk/dalpha, after W^T X
+  const size_t total = n_u + n_vec + n_S + n_WX + n_kba;
   const size_t s_out = n_u + n_vec;   // first S element of the stage gradient
   // A CTA owns 32 consecutive input elements per iteration (lanes, coalesced); warp g sums partials g, g + 8, ...
   // and the 8 warp sums are folded in fixed order through shared memory (bit-deterministic), which keeps 8x more
@@ -1400,12 +1412,14 @@ __global__ void __launch_bounds__(kThreads, 6) stage_grad_reduce_kernel(SgReduce
         for (int sp = g; sp < L.splitsS; sp += 8) s += (double)upart[(size_t)sp * MP + e];
       } else if (e < n_u + n_vec) {
         const size_t k = e - n_u;
-        for (int c = g; c < a.nvec_used; c += 8) s += (double)vecpart[(size_t)c * L.vec_len + k];
+        for (int c = g; c < a.nvec_used; c += 8) s += (double)vecpart[(size_t)c * L.vp_len + k];
         if (tc && k < (size_t)MP)
           for (int c = g; c < a.ncpart; c += 8) s += (double)cpart[(size_t)c * MP + k];
-      } else {
+      } else if (e < s_out + n_S + n_WX) {
         const size_t idx = e - s_out - n_S;
         for (int sp = g; sp < L.splitsZ; sp += 8) s += (double)WXpart[(size_t)sp * MP * DP + idx];
+      } else {
+        for (int c = g; c < a.nvec_used; c += 8) s += (double)vecpart[(size_t)c * L.vp_len + L.vec_len];   // VS_KBA
       }
     }
     __syncthreads();
@@ -1449,15 +1463,16 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
   const double* Li64 = ws_cptr<double>(a.ws, L.Linv64);
   double* T64 = ws_ptr<double>(a.ws, L.T64);
   double* U64 = ws_ptr<double>(a.ws, L.U64);
-  // stage gradient (read-only): [u MP | vec vec_len | S MP x MP | W^T X MP x DP]
+  // stage gradient (read-only): [u MP | vec vec_len | S MP x MP | W^T X MP x DP | RQ: sum kbar o dk/dalpha]
   const double* u64 = a.sgrad;
   const double* vec64 = a.sgrad + MP;
   const double* S64 = vec64 + L.vec_len;
   const double* WX64 = S64 + (size_t)MP * MP;
-  // fp64 vector scratch: [per-item sums of sym(Kb) o (Kzz - jitter I) (Matern kinds; NH nb^2 <= MP items) | unused
-  // vec_len | unused MP | rz MP]
+  // fp64 vector scratch: [per-item sums of sym(Kb) o (Kzz - jitter I) (Matern / RQ kinds; NH nb^2 <= MP items) |
+  // per-item sums of sym(Kb) o dKzz/dalpha (RQ; in vec_len >= MP) | unused MP | rz MP]
   double* v64 = ws_ptr<double>(a.ws, L.v64);
   double* kbk64 = v64;
+  double* kba64 = v64 + MP;
   double* rz64 = v64 + 2 * MP + L.vec_len;
   double* t64 = ws_ptr<double>(a.ws, L.t64);   // [MP, DP] per-(i, d) terms of d lengthscale
 
@@ -1483,13 +1498,16 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
 
   GPBLUR_STAMP();
   // ---------------- phase B: sym(Kb) = Linv^T Tm ; Wzz = sym(Kb) o (Kzz - jitter I) -> U64 ----------------
-  // Matern kinds: Wzz = sym(Kb) o g(d2) from the distances the forward kept; the outputscale term
-  // sum sym(Kb) o (Kzz - jitter I) is no longer sum Wzz: one partial per item -> kbk64[t], added in fixed order in D
+  // Matern / RQ kinds: Wzz = sym(Kb) o g(d2) from the distances the forward kept; the outputscale term
+  // sum sym(Kb) o (Kzz - jitter I) is no longer sum Wzz: one partial per item -> kbk64[t], added in fixed order in D.
+  // RQ: likewise the alpha term sum sym(Kb) o dKzz/dalpha -> kba64[t].
   {
     const double zz_jitter = hyp64[H_JIT];
     const double os = hyp64[H_OS];
+    const bool rq = MAT && L.kind == GPBLUR_KERNEL_RQ;
+    const double alpha = rq ? hyp64[H_ALPHA] : 0.0;
     const double* D2 = ws_cptr<double>(a.ws, L.D2zz64);
-    __shared__ double kred[8];
+    __shared__ double kred[8], ared[8];
     for (int t = blockIdx.x; t < NH * nb * nb; t += G) {
       const int tile = t / NH, bi = tile / nb, bj = tile - bi * nb, r0 = bi * TB + RT * (t % NH);
       // operands of the epilogue, requested before the product
@@ -1503,7 +1521,7 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
       }
       double acc[NR] = {};
       wide_gemm<RT>(acc, MatRef{Li64, MP, true}, r0, MatRef{T64, MP, false}, bj * TB, bi * TB, MP, gsm);
-      double kbk = 0.0;
+      double kbk = 0.0, kba = 0.0;
 #pragma unroll
       for (int i = 0; i < NR; ++i) {
         const int gi = r0 + warp + 8 * i, gj = bj * TB + lane;
@@ -1511,10 +1529,11 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
         if (gi < M && gj < M) {
           const double kz = e_k[i] - (gi == gj ? zz_jitter : 0.0);
           if constexpr (MAT) {
-            double kk, g;
-            kernel_kg64(L.kind, e_d2[i], os, kk, g);
+            double kk, g, ka = 0.0;
+            kernel_kg64(L.kind, e_d2[i], os, alpha, kk, g, ka);
             v = acc[i] * g;
             kbk += acc[i] * kz;
+            kba += acc[i] * ka;
           } else {
             v = acc[i] * kz;
           }
@@ -1524,12 +1543,21 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
       if constexpr (MAT) {
         kbk = warp_sum(kbk);
         if (lane == 0) kred[warp] = kbk;
+        if (rq) {
+          kba = warp_sum(kba);
+          if (lane == 0) ared[warp] = kba;
+        }
         __syncthreads();
         if (tid == 0) {
-          double s = 0.0;
+          double s = 0.0, sa = 0.0;
 #pragma unroll
           for (int w8 = 0; w8 < 8; ++w8) s += kred[w8];
           kbk64[t] = s;
+          if (rq) {
+#pragma unroll
+            for (int w8 = 0; w8 < 8; ++w8) sa += ared[w8];
+            kba64[t] = sa;
+          }
         }
       }
     }
@@ -1658,6 +1686,16 @@ __global__ void __launch_bounds__(kThreads) mm_backward_kernel(MmBwdArgs a) {
         GPBLUR_PUT(&b_b[0], (float)sc[VS_GMU]);
       }
     }
+    if (MAT && L.kind == GPBLUR_KERNEL_RQ && warp == 1) {
+      // d raw_alpha: sum sym(Kb) o dKzz/dalpha (per-item sums of phase B, fixed order) + sum kbar o dk/dalpha
+      double s = 0.0;
+      for (int i = lane; i < NH * nb * nb; i += 32) s += kba64[i];
+      s = warp_sum(s);
+      if (lane == 0) {
+        const double da = s + WX64[(size_t)MP * DP];
+        GPBLUR_PUT(&b_b[1], (float)(da * sigmoid64((double)a.p.raw_alpha[0])));
+      }
+    }
   }
   GPBLUR_STAMP();
 #undef GPBLUR_STAMP
@@ -1676,8 +1714,8 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   double* Ss = reinterpret_cast<double*>(smem_raw);   // [32][33] S (stage gradient), later Wzz
   double* Li = Ss + TB * TLD;                         // L^-1
   double* Kz = Li + TB * TLD;                         // Kzz + jitter
-  double* Us = Kz + TB * TLD;                         // P, then sym(Kbar) o (Kzz - jitter I) (Matern kinds)
-  double* Ts = Us + TB * TLD;                         // Tm
+  double* Us = Kz + TB * TLD;                         // P, then sym(Kbar) o (Kzz - jitter I) (Matern / RQ kinds)
+  double* Ts = Us + TB * TLD;                         // Tm, then sym(Kbar) o dKzz/dalpha (RQ)
   double* Zd = Ts + TB * TLD;                         // [32][DP + 1] Z~ (double)
   double* Wx = Zd + TB * (GPBLUR_MAX_D + 1);          // [32][DP + 1] W^T X (stage gradient)
   double* u_s = Wx + TB * (GPBLUR_MAX_D + 1);         // [32]
@@ -1747,13 +1785,17 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
   }
   __syncthreads();
   // ---- phase B: sym(Kbar) = Linv^T Tm ; Wzz = sym(Kbar) o (Kzz - jitter I) -> Ss ; row sums ----
-  // (Matern kinds: Wzz = sym(Kbar) o g(d2); the products sym(Kbar) o (Kzz - jitter I) of the outputscale term are
-  //  parked in Us, free since phase A, and summed into kbk)
+  // (Matern / RQ kinds: Wzz = sym(Kbar) o g(d2); the products sym(Kbar) o (Kzz - jitter I) of the outputscale term are
+  //  parked in Us, free since phase A, and summed into kbk; RQ: the products sym(Kbar) o dKzz/dalpha go to Ts once
+  //  every thread has read Tm, and are summed in phase D)
   constexpr bool rbf = !MAT;
+  const bool rq = MAT && L.kind == GPBLUR_KERNEL_RQ;
   double kbk = 0.0;
+  double ua[4] = {0.0, 0.0, 0.0, 0.0};
   {
     const double zz_jitter = hyp64[H_JIT];
     const double os = hyp64[H_OS];
+    const double alpha = rq ? hyp64[H_ALPHA] : 0.0;
     const double* D2 = ws_cptr<double>(a.ws, L.D2zz64);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -1766,10 +1808,11 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
       } else {
         double u = 0.0;
         if (r < M && lane < M) {
-          double kk, g;
-          kernel_kg64(L.kind, D2[(size_t)r * MP + lane], os, kk, g);
+          double kk, g, ka = 0.0;
+          kernel_kg64(L.kind, D2[(size_t)r * MP + lane], os, alpha, kk, g, ka);
           v = kb * g;
           u = kb * (Kz[r * TLD + lane] - (r == lane ? zz_jitter : 0.0));
+          ua[i] = kb * ka;
         }
         Us[r * TLD + lane] = u;
       }
@@ -1777,6 +1820,10 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
     }
   }
   __syncthreads();
+  if (rq) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) Ts[(warp + 8 * i) * TLD + lane] = ua[i];
+  }
   if (tid < MP) {
     double rz = 0.0;
     for (int j = 0; j < TB; ++j) rz += Ss[tid * TLD + j];
@@ -1850,6 +1897,14 @@ __global__ void __launch_bounds__(kThreads) mm_small_backward_kernel(MmBwdArgs a
         GPBLUR_PUT(&b_os[0], (float)(dos * sigmoid64((double)a.p.raw_outputscale[0])));
         GPBLUR_PUT(&b_b[0], (float)sc[VS_GMU]);
       }
+    }
+    if (rq && warp == 6) {
+      // d raw_alpha: column sums of the parked products (rows in order), lanes by the shuffle tree, + sum kbar o dk/dalpha
+      double s = 0.0;
+      for (int r = 0; r < M; ++r) s += Ts[r * TLD + lane];
+      s = warp_sum(s);
+      if (lane == 0)
+        GPBLUR_PUT(&b_b[1], (float)((s + WX64[(size_t)MP * DP]) * sigmoid64((double)a.p.raw_alpha[0])));
     }
   }
   if (tid == 0) { const unsigned long long t = global_ns(); for (int k = 1; k < 5; ++k) stamps[k] = t; }
@@ -1977,7 +2032,7 @@ int launch_mm_backward(const gpblur_svgp_params& p, const WsLayout& L, void* sta
 
 int stage_grad_reduce_impl(const WsLayout& L, const void* ws, double* sgrad, int nvec_used, int ncpart,
                            cudaStream_t st) {
-  const size_t total = stage_grad_doubles(L.MP, L.DP);   // at most the elements the kernel reads
+  const size_t total = stage_grad_doubles(L.MP, L.DP, L.kind);   // at most the elements the kernel reads
   int grid = (int)((total + 31) / 32);
   if (grid > 16 * 148) grid = 16 * 148;
   SgReduceArgs args{L, ws, sgrad, nvec_used, ncpart};

@@ -4,7 +4,7 @@
 //   g_mu, g_var  <- upstream (mean, variance, reparameterised sample folded, variance clamp respected)
 //   k            <- recomputed from X and the staged Z~ tiles (stage A, as in the forward)
 //   kbar[n, :]   = g_mu[n] beta + 2 g_var[n] (diag(c) Linv)^T a[n, :]        block-triangular GEMM on saved A
-//   W            = kbar o k ;  r[n] = sum_m W ;  colsum[m] = sum_n W     (Matern kinds: W = kbar o g)
+//   W            = kbar o k ;  r[n] = sum_m W ;  colsum[m] = sum_n W     (Matern / RQ kinds: W = kbar o g)
 //   dx[n, :]     = ( W Z~ - r x~ ) / ell + g_mu w                             GEMM on the resident W chunk
 // W is also written to HBM once: the N-reduction GEMMs (gpblur_reduce.cu) turn it into dZ / d lengthscale.
 // Per-CTA vector partials (colsum, q = sum r x~^2, wbar, scalar sums) are reduced by the M x M stage.
@@ -24,10 +24,11 @@ struct BwdSmem {
   }
 };
 
-// KIND (GPBLUR_KERNEL_*): for the Matern kinds the recomputed chunk holds d2 instead of k, and step (c) forms
-// W = kbar o g and the sum of kbar o k (vector partial slot VS_KBK) from it
+// KIND (GPBLUR_KERNEL_*): for the Matern / RQ kinds the recomputed chunk holds d2 instead of k, and step (c) forms
+// W = kbar o g and the sum of kbar o k (vector partial slot VS_KBK) from it; RQ also the sum of kbar o dk/dalpha
+// (VS_KBA).  The body sits behind the entry points point_bwd_kernel (RBF, Matern) and point_bwd_rq_kernel (RQ).
 template <class Cfg, int DP, int KIND>
-__global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_kernel(PointBwdArgs a) {
+__device__ __forceinline__ void point_bwd_body(const PointBwdArgs& a) {
   constexpr int PT = Cfg::PT, CT = Cfg::CT, CW = Cfg::CW, TN = Cfg::TN, TXN = Cfg::TXN, TYN = Cfg::TYN;
   using S = BwdSmem<Cfg, DP>;
   constexpr int ldx = S::ldx, lda = S::lda, ldw = S::ldw, BZ = S::BZ;
@@ -81,7 +82,9 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
   for (int i = tid; i < MP; i += kThreads) colsum_s[i] = 0.f;
   for (int i = tid; i < DP; i += kThreads) { q_s[i] = 0.f; t1_s[i] = 0.f; }
   if (tid < 16) sc_s[tid] = 0.f;
-  float kbk_acc = 0.f;                            // Matern kinds: this thread's share of sum kbar o k
+  float kbk_acc = 0.f;                            // Matern / RQ kinds: this thread's share of sum kbar o k
+  float kba_acc = 0.f;                            // RQ: this thread's share of sum kbar o dk/dalpha
+  const float alpha = KIND == GPBLUR_KERNEL_RQ ? hyp[H_ALPHA] : 0.f, i2a = KIND == GPBLUR_KERNEL_RQ ? hyp[H_I2A] : 0.f;
 
   for (int tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
     const long long n0 = (long long)tile * TN;
@@ -201,6 +204,13 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
             const float kb = fmaf(gv2, acc[e][f], gm * bet[f]);
             if constexpr (KIND == GPBLUR_KERNEL_RBF) {
               w[f] = kb * kk[f];
+            } else if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+              float kv, g, ka;
+              rq_kg(kk[f], os, alpha, i2a, kv, g, ka);
+              if (!(kk[f] < 1e20f)) { kv = 0.f; g = 0.f; ka = 0.f; }   // padded column (d2 = 1e30)
+              w[f] = kb * g;
+              kbk_acc = fmaf(kb, kv, kbk_acc);
+              kba_acc = fmaf(kb, ka, kba_acc);
             } else {
               float kv, g;
               matern_kg<KIND>(kk[f], os, kv, g);
@@ -358,15 +368,35 @@ __global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_ker
       sc_s[VS_KBK] = t;
     }
   }
+  if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+    __syncthreads();
+    const float s = warp_sum(kba_acc);
+    if (lane == 0) dpart[warp] = s;
+    __syncthreads();
+    if (tid == 0) {
+      float t = 0.f;
+      for (int w8 = 0; w8 < kThreads / 32; ++w8) t += dpart[w8];
+      sc_s[VS_KBA] = t;
+    }
+  }
   __syncthreads();
-  float* vp = vecpart + (size_t)blockIdx.x * L.vec_len;
+  float* vp = vecpart + (size_t)blockIdx.x * L.vp_len;
   for (int i = tid; i < MP; i += kThreads) vp[i] = colsum_s[i];
   for (int d = tid; d < DP; d += kThreads) {
     vp[MP + d] = q_s[d];
     // wbar_d = sum_n g_mu x_nd = ell_d * sum_n g_mu x~_nd + c_d * sum_n g_mu
     vp[MP + DP + d] = (d < D) ? ellv[d] * t1_s[d] + center[d] * sc_s[VS_GMU] : 0.f;
   }
-  if (tid < VS_COUNT) vp[MP + 2 * DP + tid] = sc_s[tid];
+  if (tid < VS_PART) vp[MP + 2 * DP + tid] = sc_s[tid];
+}
+
+template <class Cfg, int DP, int KIND>
+__global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_kernel(PointBwdArgs a) {
+  point_bwd_body<Cfg, DP, KIND>(a);
+}
+template <class Cfg, int DP>
+__global__ void __launch_bounds__(kThreads, Cfg::TN <= 64 ? 2 : 1) point_bwd_rq_kernel(PointBwdArgs a) {
+  point_bwd_body<Cfg, DP, GPBLUR_KERNEL_RQ>(a);
 }
 
 // tile height used by the backward for a given problem (shared with the M x M stage, which needs the
@@ -388,18 +418,22 @@ template <class Cfg, int DP, int KIND>
 int launch_bwd_kind(const PointBwdArgs& a0, cudaStream_t st) {
   PointBwdArgs a = a0;
   const size_t smem = sizeof(float) * BwdSmem<Cfg, DP>::floats(a.L.MP);
-  cudaFuncSetAttribute(point_bwd_kernel<Cfg, DP, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
+  auto* kernel = [] {
+    if constexpr (KIND == GPBLUR_KERNEL_RQ) return point_bwd_rq_kernel<Cfg, DP>;
+    else return point_bwd_kernel<Cfg, DP, KIND>;
+  }();
+  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
   a.ntiles = (int)((a.L.N + Cfg::TN - 1) / Cfg::TN);
   const int grid = bwd_persistent_grid(a.L, Cfg::TN);
   ProfScope ps(ST_POINT_BWD, st);
-  point_bwd_kernel<Cfg, DP, KIND><<<grid, kThreads, smem, st>>>(a);
+  kernel<<<grid, kThreads, smem, st>>>(a);
   note_launch();
   return check_launch("point_bwd");
 }
 
 template <class Cfg, int DP>
 int launch_bwd_cfg(const PointBwdArgs& a, cudaStream_t st) {
-  // the Matern kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
+  // the Matern / RQ kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
   if constexpr (Cfg::CW != 32) {
     if (a.L.kind != GPBLUR_KERNEL_RBF) return GPBLUR_EUNSUPPORTED;
     return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_RBF>(a, st);
@@ -408,6 +442,7 @@ int launch_bwd_cfg(const PointBwdArgs& a, cudaStream_t st) {
       case GPBLUR_KERNEL_MATERN12: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN12>(a, st);
       case GPBLUR_KERNEL_MATERN32: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN32>(a, st);
       case GPBLUR_KERNEL_MATERN52: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_MATERN52>(a, st);
+      case GPBLUR_KERNEL_RQ: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_RQ>(a, st);
       default: return launch_bwd_kind<Cfg, DP, GPBLUR_KERNEL_RBF>(a, st);
     }
   }

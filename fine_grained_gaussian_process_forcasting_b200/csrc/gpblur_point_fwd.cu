@@ -3,7 +3,7 @@
 // kernels; /root/reference/denoising_model/DeepGP.py:56-73,94-99 via VariationalStrategy.forward):
 //
 //   stage A  k[n, m]  = os * exp(-1/2 |x~_n - z~_m|^2)          norm expansion, FP32 FFMA, Z~ tiles staged
-//            (Matern kinds: os f(r) of the same d2, gpblur_common.cuh: matern_kg)
+//            (Matern / RQ kinds: os f of the same d2, gpblur_common.cuh: matern_kg / rq_kg)
 //   stage B  a[n, :]  = Linv k[n, :]                             block-triangular GEMM, K resident in smem
 //   epilogue mean = a.m + x.w + b ; var = max(os + jitter + sum (s^2-1) a^2, 1e-6) ;
 //            sample = mean + sqrt(var) * PhiloxNormal(seed, offset + n)
@@ -14,8 +14,9 @@ namespace gpblur {
 
 namespace {
 
+// The body sits behind the entry points point_fwd_kernel (RBF, Matern) and point_fwd_rq_kernel (RQ).
 template <class Cfg, int KIND>
-__global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kernel(PointFwdArgs a) {
+__device__ __forceinline__ void point_fwd_body(const PointFwdArgs& a) {
   constexpr int PT = Cfg::PT, CT = Cfg::CT, CW = Cfg::CW, TN = Cfg::TN;
   extern __shared__ __align__(16) float smem[];
   const WsLayout& L = a.L;
@@ -44,6 +45,7 @@ __global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kern
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int tx = Cfg::tx(), ty = Cfg::ty();
   const float os = hyp[H_OS], jit = hyp[H_JIT], cwb = hyp[H_CWB];
+  const float alpha = KIND == GPBLUR_KERNEL_RQ ? hyp[H_ALPHA] : 0.f, i2a = KIND == GPBLUR_KERNEL_RQ ? hyp[H_I2A] : 0.f;
 
   for (int tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
     const long long n0 = (long long)tile * TN;
@@ -83,6 +85,10 @@ __global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kern
           const float d2 = fmaxf(xn + zn[m] - 2.0f * acc[e][f], 0.f);
           if constexpr (KIND == GPBLUR_KERNEL_RBF) {
             kv[f] = (m < M) ? os * expf(-0.5f * d2) : 0.f;
+          } else if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+            float g, ka;
+            rq_kg(d2, os, alpha, i2a, kv[f], g, ka);
+            if (m >= M) kv[f] = 0.f;
           } else {
             float g;
             matern_kg<KIND>(d2, os, kv[f], g);
@@ -162,6 +168,15 @@ __global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kern
   }
 }
 
+template <class Cfg, int KIND>
+__global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_kernel(PointFwdArgs a) {
+  point_fwd_body<Cfg, KIND>(a);
+}
+template <class Cfg>
+__global__ void __launch_bounds__(kThreads, Cfg::PT <= 4 ? 2 : 1) point_fwd_rq_kernel(PointFwdArgs a) {
+  point_fwd_body<Cfg, GPBLUR_KERNEL_RQ>(a);
+}
+
 template <class Cfg>
 size_t fwd_smem_bytes(const WsLayout& L) {
   return sizeof(float) * ((size_t)Cfg::TN * (L.DP + 4) + (size_t)Cfg::TN * (L.MP + 4) + 2 * kKS * Cfg::CW +
@@ -172,23 +187,27 @@ template <class Cfg, int KIND>
 int launch_fwd_kind(const PointFwdArgs& a0, cudaStream_t st) {
   PointFwdArgs a = a0;
   const size_t smem = fwd_smem_bytes<Cfg>(a.L);
-  cudaFuncSetAttribute(point_fwd_kernel<Cfg, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
+  auto* kernel = [] {
+    if constexpr (KIND == GPBLUR_KERNEL_RQ) return point_fwd_rq_kernel<Cfg>;
+    else return point_fwd_kernel<Cfg, KIND>;
+  }();
+  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   // per device
   a.ntiles = (int)((a.L.N + Cfg::TN - 1) / Cfg::TN);
   int occ = 1;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, point_fwd_kernel<Cfg, KIND>, kThreads, smem);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kThreads, smem);
   if (occ < 1) occ = 1;
   int grid = occ * num_sms();
   if (grid > a.ntiles) grid = a.ntiles;
   if (grid < 1) grid = 1;
   ProfScope ps(ST_POINT_FWD, st);
-  point_fwd_kernel<Cfg, KIND><<<grid, kThreads, smem, st>>>(a);
+  kernel<<<grid, kThreads, smem, st>>>(a);
   note_launch();
   return check_launch("point_fwd");
 }
 
 template <class Cfg>
 int launch_fwd_cfg(const PointFwdArgs& a, cudaStream_t st) {
-  // the Matern kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
+  // the Matern / RQ kinds run on the FP32-FFMA kernels for MP = 32 only (MP >= 128 takes the tensor-core kernels)
   if constexpr (Cfg::CW != 32) {
     if (a.L.kind != GPBLUR_KERNEL_RBF) return GPBLUR_EUNSUPPORTED;
     return launch_fwd_kind<Cfg, GPBLUR_KERNEL_RBF>(a, st);
@@ -197,6 +216,7 @@ int launch_fwd_cfg(const PointFwdArgs& a, cudaStream_t st) {
       case GPBLUR_KERNEL_MATERN12: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN12>(a, st);
       case GPBLUR_KERNEL_MATERN32: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN32>(a, st);
       case GPBLUR_KERNEL_MATERN52: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_MATERN52>(a, st);
+      case GPBLUR_KERNEL_RQ: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_RQ>(a, st);
       default: return launch_fwd_kind<Cfg, GPBLUR_KERNEL_RBF>(a, st);
     }
   }

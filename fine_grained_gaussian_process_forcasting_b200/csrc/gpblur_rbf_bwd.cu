@@ -5,8 +5,9 @@
 //   g_x1[i, d] = -sum_j W_ij (x1_id - x2_jd) / l_d^2          g_x2[j, d] = +sum_i W_ij (x1_id - x2_jd) / l_d^2
 //   g_l_d      =  sum_ij W_ij (x1_id - x2_jd)^2 / l_d^3        g_os = sum_ij W_ij / os
 // and the chain rule through softplus (sigmoid of the raw value); an isotropic kernel sums g_l over d.
-// Matern kinds: W = G o g (gpblur_common.cuh: matern_kg) in the distance gradients, and g_os = sum_ij G_ij K_ij / os
-// from a second matrix Wk = G o K.
+// Matern and RQ kinds: W = G o g (gpblur_common.cuh: matern_kg / rq_kg) in the distance gradients, and
+// g_os = sum_ij G_ij K_ij / os from a second matrix Wk = G o K.  RQ: g_alpha = sum_ij G_ij dK_ij/dalpha from a third
+// matrix Wa, summed per row as one more row statistic.
 // Three launches: W (tile kernel, as the forward) -> row pass (g_x1, per-row lengthscale / W sums) and column pass
 // (g_x2) -> one CTA adds the per-row sums in row order (bit-deterministic).  O(n1 n2 D) work, exact-GP sizes.
 #include "gpblur_common.cuh"
@@ -22,7 +23,8 @@ __device__ __forceinline__ float sigmoid_f(float r) { return 1.0f / (1.0f + expf
 template <int KIND>
 __global__ void rbf_w_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n1, long long n2, int D,
                              const float* __restrict__ raw_ell, int ard, const float* __restrict__ raw_os,
-                             const float* __restrict__ g_out, float* __restrict__ W, float* __restrict__ Wk) {
+                             const float* __restrict__ raw_alpha, const float* __restrict__ g_out,
+                             float* __restrict__ W, float* __restrict__ Wk, float* __restrict__ Wa) {
   __shared__ float a[16][33], b[16][33], ie[32];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const long long i0 = (long long)blockIdx.y * 16, j0 = (long long)blockIdx.x * 16;
@@ -49,6 +51,14 @@ __global__ void rbf_w_kernel(const float* __restrict__ x1, const float* __restri
   if (i < n1 && j < n2) {
     if constexpr (KIND == GPBLUR_KERNEL_RBF) {
       W[(size_t)i * n2 + j] = g_out[(size_t)i * n2 + j] * softplus_f(raw_os[0]) * expf(-0.5f * acc);
+    } else if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+      const float alpha = softplus_f(raw_alpha[0]);
+      float k, g, ka;
+      rq_kg(acc, softplus_f(raw_os[0]), alpha, 0.5f / alpha, k, g, ka);
+      const float go = g_out[(size_t)i * n2 + j];
+      W[(size_t)i * n2 + j] = go * g;
+      Wk[(size_t)i * n2 + j] = go * k;
+      Wa[(size_t)i * n2 + j] = go * ka;
     } else {
       float k, g;
       matern_kg<KIND>(acc, softplus_f(raw_os[0]), k, g);
@@ -61,10 +71,12 @@ __global__ void rbf_w_kernel(const float* __restrict__ x1, const float* __restri
 
 // one CTA per row i of x1: threads = dimensions (d < D <= 128), loop over j.
 //   g_x1[i, d] ; rowstat[i, d] = sum_j W_ij (x1_id - x2_jd)^2 ; rowstat[i, D] = sum_j Wos_ij   (double)
-//   (Wos: W for RBF, Wk for the Matern kinds)
+//   (Wos: W for RBF, Wk for the Matern and RQ kinds); RQ (Wa non-null): rowstat[i, D + 1] = sum_j Wa_ij.
+//   Row stride rs = D + 1, D + 2 for RQ.
 __global__ void rbf_row_kernel(const float* __restrict__ x1, const float* __restrict__ x2, long long n2, int D,
                                const float* __restrict__ raw_ell, int ard, const float* __restrict__ W,
-                               const float* __restrict__ Wos, float* __restrict__ g_x1, double* __restrict__ rowstat) {
+                               const float* __restrict__ Wos, const float* __restrict__ Wa, int rs,
+                               float* __restrict__ g_x1, double* __restrict__ rowstat) {
   const long long i = blockIdx.x;
   const int d = threadIdx.x;
   const float* wr = W + (size_t)i * n2;
@@ -78,12 +90,12 @@ __global__ void rbf_row_kernel(const float* __restrict__ x1, const float* __rest
       s2 += (double)(w * df * df);
     }
     if (g_x1) g_x1[(size_t)i * D + d] = (float)(-s1 / ((double)ell * ell));
-    rowstat[(size_t)i * (D + 1) + d] = s2;
-  } else if (d == D) {
-    const float* wo = Wos + (size_t)i * n2;
+    rowstat[(size_t)i * rs + d] = s2;
+  } else if (d == D || (d == D + 1 && Wa)) {
+    const float* wo = (d == D ? Wos : Wa) + (size_t)i * n2;
     double s = 0.0;
     for (long long j = 0; j < n2; ++j) s += (double)wo[j];
-    rowstat[(size_t)i * (D + 1) + D] = s;
+    rowstat[(size_t)i * rs + d] = s;
   }
 }
 
@@ -101,15 +113,16 @@ __global__ void rbf_col_kernel(const float* __restrict__ x1, const float* __rest
   g_x2[(size_t)j * D + d] = (float)(s1 / ((double)ell * ell));
 }
 
-// rows added in row order: g_raw_ell [D] (ard) or [1], g_raw_os [1]
-__global__ void rbf_finish_kernel(const double* __restrict__ rowstat, long long n1, int D, const float* __restrict__ raw_ell,
-                                  int ard, const float* __restrict__ raw_os, float* __restrict__ g_raw_ell,
-                                  float* __restrict__ g_raw_os) {
+// rows added in row order: g_raw_ell [D] (ard) or [1], g_raw_os [1], RQ (rs = D + 2): g_raw_alpha [1]
+__global__ void rbf_finish_kernel(const double* __restrict__ rowstat, long long n1, int D, int rs,
+                                  const float* __restrict__ raw_ell, int ard, const float* __restrict__ raw_os,
+                                  const float* __restrict__ raw_alpha, float* __restrict__ g_raw_ell,
+                                  float* __restrict__ g_raw_os, float* __restrict__ g_raw_alpha) {
   __shared__ double iso[129];
   const int d = threadIdx.x;
   double t = 0.0;
-  if (d <= D)
-    for (long long i = 0; i < n1; ++i) t += rowstat[(size_t)i * (D + 1) + d];
+  if (d < rs)
+    for (long long i = 0; i < n1; ++i) t += rowstat[(size_t)i * rs + d];
   if (d < D) {
     const float r = raw_ell[ard ? d : 0];
     const double ell = (double)softplus_f(r);
@@ -119,6 +132,8 @@ __global__ void rbf_finish_kernel(const double* __restrict__ rowstat, long long 
   } else if (d == D) {
     const float r = raw_os[0];
     g_raw_os[0] = (float)(t / (double)softplus_f(r) * (double)sigmoid_f(r));
+  } else if (d == D + 1 && d < rs) {
+    g_raw_alpha[0] = (float)(t * (double)sigmoid_f(raw_alpha[0]));
   }
   __syncthreads();
   if (!ard && d == 0) {
@@ -134,48 +149,69 @@ __global__ void rbf_finish_kernel(const double* __restrict__ rowstat, long long 
 
 using namespace gpblur;
 
+// W matrices of a kind (W; W, Wk; W, Wk, Wa for RQ) and the row-statistic stride
+static int cov_wmats(int kind) { return kind == GPBLUR_KERNEL_RBF ? 1 : kind == GPBLUR_KERNEL_RQ ? 3 : 2; }
+static int cov_rowstride(int D, int kind) { return D + (kind == GPBLUR_KERNEL_RQ ? 2 : 1); }
+
 extern "C" size_t gpblur_covariance_backward_scratch_bytes(long long n1, long long n2, int D, int kind) {
   if (n1 < 0 || n2 < 0 || D < 1 || !kernel_kind_valid(kind)) return 0;
   const size_t wb = align_up((size_t)n1 * (size_t)n2 * 4);
-  return (kind == GPBLUR_KERNEL_RBF ? wb : 2 * wb) + (size_t)n1 * (size_t)(D + 1) * 8;
+  return cov_wmats(kind) * wb + (size_t)n1 * (size_t)cov_rowstride(D, kind) * 8;
 }
 
 extern "C" int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                                           const float* raw_lengthscale, int ard, const float* raw_outputscale,
                                           const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
                                           float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream) {
+  return gpblur_covariance_backward_alpha(x1, x2, n1, n2, D, kind, raw_lengthscale, ard, raw_outputscale, nullptr,
+                                          g_out, g_x1, g_x2, g_raw_lengthscale, g_raw_outputscale, nullptr, scratch,
+                                          scratch_bytes, stream);
+}
+
+extern "C" int gpblur_covariance_backward_alpha(const float* x1, const float* x2, long long n1, long long n2, int D,
+                                                int kind, const float* raw_lengthscale, int ard,
+                                                const float* raw_outputscale, const float* raw_alpha,
+                                                const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
+                                                float* g_raw_outputscale, float* g_raw_alpha, void* scratch,
+                                                size_t scratch_bytes, void* stream) {
   if (n1 < 1 || n2 < 1 || D < 1 || D > GPBLUR_MAX_D || !kernel_kind_valid(kind)) return GPBLUR_EINVAL;
   if (!x1 || !x2 || !raw_lengthscale || !raw_outputscale || !g_out || !g_raw_lengthscale || !g_raw_outputscale || !scratch)
     return GPBLUR_EINVAL;
+  if (kind == GPBLUR_KERNEL_RQ && (!raw_alpha || !g_raw_alpha)) return GPBLUR_EINVAL;
   if ((reinterpret_cast<uintptr_t>(scratch) & 255) ||
       scratch_bytes < gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind))
     return GPBLUR_EWORKSPACE;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const size_t wb = align_up((size_t)n1 * (size_t)n2 * 4);
-  const bool rbf = kind == GPBLUR_KERNEL_RBF;
+  const bool rbf = kind == GPBLUR_KERNEL_RBF, rq = kind == GPBLUR_KERNEL_RQ;
   float* W = static_cast<float*>(scratch);
   float* Wk = rbf ? W : reinterpret_cast<float*>(static_cast<char*>(scratch) + wb);
-  double* rowstat = reinterpret_cast<double*>(static_cast<char*>(scratch) + (rbf ? wb : 2 * wb));
-  const int threads = round_up(D + 1, 32);
+  float* Wa = rq ? reinterpret_cast<float*>(static_cast<char*>(scratch) + 2 * wb) : nullptr;
+  double* rowstat = reinterpret_cast<double*>(static_cast<char*>(scratch) + cov_wmats(kind) * wb);
+  const int rs = cov_rowstride(D, kind);
+  const int threads = round_up(rs, 32);
   ProfScope ps(ST_OTHER, st);
   dim3 grid((unsigned)((n2 + 15) / 16), (unsigned)((n1 + 15) / 16));
   switch (kind) {
     case GPBLUR_KERNEL_MATERN12:
-      rbf_w_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN12><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, g_out, W, Wk, Wa);
       break;
     case GPBLUR_KERNEL_MATERN32:
-      rbf_w_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN32><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, g_out, W, Wk, Wa);
       break;
     case GPBLUR_KERNEL_MATERN52:
-      rbf_w_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      rbf_w_kernel<GPBLUR_KERNEL_MATERN52><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, g_out, W, Wk, Wa);
+      break;
+    case GPBLUR_KERNEL_RQ:
+      rbf_w_kernel<GPBLUR_KERNEL_RQ><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, g_out, W, Wk, Wa);
       break;
     default:
-      rbf_w_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, g_out, W, Wk);
+      rbf_w_kernel<GPBLUR_KERNEL_RBF><<<grid, 256, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, raw_outputscale, raw_alpha, g_out, W, Wk, Wa);
   }
-  rbf_row_kernel<<<(unsigned)n1, threads, 0, st>>>(x1, x2, n2, D, raw_lengthscale, ard, W, Wk, g_x1, rowstat);
+  rbf_row_kernel<<<(unsigned)n1, threads, 0, st>>>(x1, x2, n2, D, raw_lengthscale, ard, W, Wk, Wa, rs, g_x1, rowstat);
   if (g_x2) rbf_col_kernel<<<(unsigned)n2, threads, 0, st>>>(x1, x2, n1, n2, D, raw_lengthscale, ard, W, g_x2);
-  rbf_finish_kernel<<<1, threads, 0, st>>>(rowstat, n1, D, raw_lengthscale, ard, raw_outputscale, g_raw_lengthscale,
-                                           g_raw_outputscale);
+  rbf_finish_kernel<<<1, threads, 0, st>>>(rowstat, n1, D, rs, raw_lengthscale, ard, raw_outputscale, raw_alpha,
+                                           g_raw_lengthscale, g_raw_outputscale, g_raw_alpha);
   note_launch(g_x2 ? 4 : 3);
   return check_launch("rbf_cov_backward");
 }

@@ -367,16 +367,28 @@ constexpr int kMaxFwdSlabs = 20 * 8;   // MP = 1024: 20 passes x (4 d-slabs + 4 
 // parity = A stage), so the latency chain of a slab (TMEM load -> exp -> stage acquire -> tcgen05.st -> arrive) has
 // two slab times; warp 16 issues.  Accumulator chunk c is read out (mean / variance partials, A saved for the
 // backward) by group c & 1 as soon as the issuer's commit on chunk[c] says that its last slab has retired.
-// Matern epilogue of a cross-covariance element.  t = min(log2e (S + xnc' + znc'), log2 os) = log2 os - 1/2 log2e d2
-// is the RBF exponent (RBF: k = 2^t).  The Matern kinds recover d2 = 2 ln2 (log2 os - t) >= 0 and evaluate k = os f and
-// g through matern_kg; a padded column (znc = -1e30) gives d2 ~ 1e30 and exactly k = g = 0.
+// Matern / RQ epilogue of a cross-covariance element.  t = min(log2e (S + xnc' + znc'), log2 os) = log2 os - 1/2 log2e d2
+// is the RBF exponent (RBF: k = 2^t).  The other kinds recover d2 = 2 ln2 (log2 os - t) >= 0 and evaluate k = os f,
+// g and (RQ) ka = dk/dalpha through matern_kg / rq_kg; a padded column (znc = -1e30) gives d2 ~ 1e30 and exactly
+// k = g = ka = 0 (RQ: (1 + u)^-alpha is not 0 there, so the column is masked on d2).  hp: alpha, 1 / (2 alpha) (RQ).
+struct RqHyp { float alpha, i2a; };
 template <int KIND>
-__device__ __forceinline__ void tc_kg(float t, float l2os, float os, float& k, float& g) {
-  matern_kg<KIND>((l2os - t) * 1.3862943611198906f, os, k, g);
+__device__ __forceinline__ void tc_kg(float t, float l2os, float os, RqHyp hp, float& k, float& g, float& ka) {
+  const float d2 = (l2os - t) * 1.3862943611198906f;
+  if constexpr (KIND == GPBLUR_KERNEL_RQ) {
+    rq_kg(d2, os, hp.alpha, hp.i2a, k, g, ka);
+    if (!(d2 < 1e20f)) { k = 0.f; g = 0.f; ka = 0.f; }
+  } else {
+    matern_kg<KIND>(d2, os, k, g);
+    ka = 0.f;
+  }
 }
 
+// The point kernels are __device__ bodies templated on the kind behind __global__ entry points: tc2_fwd_kernel /
+// tc2_bwd_kernel for RBF and the Matern kinds, tc2_fwd_rq_kernel / tc2_bwd_rq_kernel for RQ, so that each kernel family
+// of the compiled library covers a fixed set of kinds (tests/test_gpu_dispatch_matrix.py, tests/test_rq_dispatch.py).
 template <int BQ, int BWO, int NSTB, int KIND>
-__global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) {
+__device__ __forceinline__ void tc2_fwd_body(const Tc2Args& a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) Bars bars;
   __shared__ uint32_t tmem_slot;
@@ -454,6 +466,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) {
     const uint32_t aop_base = tmem_base + lane_base + AOP_COL;
     const float os = hyp[H_OS], jit = hyp[H_JIT], cwb = hyp[H_CWB];
     const float l2os = log2f(os);
+    const RqHyp hp = KIND == GPBLUR_KERNEL_RQ ? RqHyp{hyp[H_ALPHA], hyp[H_I2A]} : RqHyp{0.f, 0.f};
     const bool vec = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(a.x) & 15) == 0);
     const int slabs_per_tile = tab_n;
     int gs = 0;                                           // global slab counter (identical in every producer thread)
@@ -638,11 +651,11 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) {
                   v[j + 2] = tc::ex2_approx(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os));
                   v[j + 3] = tc::ex2_approx(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os));
                 } else {
-                  float g;
-                  tc_kg<KIND>(fminf(fmaf(v[j + 0], 1.4426950408889634f, xnc + z4.x), l2os), l2os, os, v[j + 0], g);
-                  tc_kg<KIND>(fminf(fmaf(v[j + 1], 1.4426950408889634f, xnc + z4.y), l2os), l2os, os, v[j + 1], g);
-                  tc_kg<KIND>(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os), l2os, os, v[j + 2], g);
-                  tc_kg<KIND>(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os), l2os, os, v[j + 3], g);
+                  float g, ka;
+                  tc_kg<KIND>(fminf(fmaf(v[j + 0], 1.4426950408889634f, xnc + z4.x), l2os), l2os, os, hp, v[j + 0], g, ka);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 1], 1.4426950408889634f, xnc + z4.y), l2os), l2os, os, hp, v[j + 1], g, ka);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 2], 1.4426950408889634f, xnc + z4.z), l2os), l2os, os, hp, v[j + 2], g, ka);
+                  tc_kg<KIND>(fminf(fmaf(v[j + 3], 1.4426950408889634f, xnc + z4.w), l2os), l2os, os, hp, v[j + 3], g, ka);
                 }
               }
               if (ptr) ptr[2] = clock64() + (long long)(v[0] == 12345.f);
@@ -785,7 +798,7 @@ __device__ __forceinline__ int warp_reduce16_index(int lane) {
 }
 
 template <int BT, int DXW, int NSTA, int NSTB, int KIND>
-__global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
+__device__ __forceinline__ void tc2_bwd_body(const Tc2Args& a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) BwdBars bb;
   __shared__ uint32_t tmem_slot;
@@ -793,7 +806,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
   __shared__ int tab_n;
   __shared__ float r_s[2][TNP];                   // row sums of W per k-half
   __shared__ float vec_s[2][4][2 * 128];          // [k-half][quadrant][q (DXW / 2) | t1 (DXW / 2)] per-warp partials
-  __shared__ float sc_s[8][4];                    // per-warp scalar sums
+  __shared__ float sc_s[8][VS_PART];              // per-warp scalar sums
   constexpr uint32_t S_COL = 0, T_COL = BT, DX_COL = 2 * BT, AOP_COL = 2 * BT + DXW;
   constexpr uint32_t USED_COLS = 2 * BT + DXW + NSTA * 64;
   constexpr uint32_t TMEM_COLS = USED_COLS <= 256 ? 256 : 512;
@@ -947,6 +960,7 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
     } else {
       // =================== row owners ===================
       const float os = hyp[H_OS], l2os = log2f(os);
+      const RqHyp hp = KIND == GPBLUR_KERNEL_RQ ? RqHyp{hyp[H_ALPHA], hyp[H_I2A]} : RqHyp{0.f, 0.f};
       const uint32_t tmem_s = tmem_base + lane_base + S_COL, tmem_t = tmem_base + lane_base + T_COL;
       const uint32_t tmem_dx = tmem_base + lane_base + DX_COL;
       const int et = tid - kGroup;                        // thread index within the group
@@ -959,7 +973,8 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
 #pragma unroll
       for (int i = 0; i < NPIECE; ++i) { qacc[i] = 0.f; tacc[i] = 0.f; }
       float s_gm = 0.f, s_r = 0.f, s_gv = 0.f;           // scalar sums (k-half 0 threads)
-      float s_kbk = 0.f;                                  // sum kbar o k of the Matern kinds (every thread)
+      float s_kbk = 0.f;                                  // sum kbar o k of the Matern / RQ kinds (every thread)
+      float s_kba = 0.f;                                  // sum kbar o dk/dalpha of RQ (every thread)
       uint32_t cnt = 0;                                   // W slabs produced so far (private stage NSTA - 1)
       // x rows of a tile go global -> shared memory with cp.async (coalesced: 16 bytes per thread and request, no
       // registers), one tile ahead: issued after the previous tile's dx epilogue, awaited at the tile head
@@ -1067,11 +1082,13 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
                 const float zz[4] = {z4.x, z4.y, z4.z, z4.w}, bb4[4] = {b4.x, b4.y, b4.z, b4.w};
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
-                  float k, g;
-                  tc_kg<KIND>(fminf(fmaf(__uint_as_float(kr[i + e]), 1.4426950408889634f, xnc + zz[e]), l2os), l2os, os, k, g);
+                  float k, g, ka;
+                  tc_kg<KIND>(fminf(fmaf(__uint_as_float(kr[i + e]), 1.4426950408889634f, xnc + zz[e]), l2os), l2os, os, hp,
+                              k, g, ka);
                   const float kb = fmaf(gv2, __uint_as_float(tr[i + e]), gm * bb4[e]);
                   w[i + e] = kb * g;
                   s_kbk = fmaf(kb, k, s_kbk);
+                  if constexpr (KIND == GPBLUR_KERNEL_RQ) s_kba = fmaf(kb, ka, s_kba);
                 }
               }
             }
@@ -1164,10 +1181,14 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
       {
         const float sg = warp_sum(s_gm), sr = warp_sum(s_r), sv = warp_sum(s_gv);
         const float sk = KIND == GPBLUR_KERNEL_RBF ? 0.f : warp_sum(s_kbk);
-        if (lane == 0) { sc_s[ew][VS_GMU] = sg; sc_s[ew][VS_RSUM] = sr; sc_s[ew][VS_GVAR] = sv; sc_s[ew][VS_KBK] = sk; }
+        const float sa = KIND == GPBLUR_KERNEL_RQ ? warp_sum(s_kba) : 0.f;
+        if (lane == 0) {
+          sc_s[ew][VS_GMU] = sg; sc_s[ew][VS_RSUM] = sr; sc_s[ew][VS_GVAR] = sv; sc_s[ew][VS_KBK] = sk;
+          sc_s[ew][VS_KBA] = sa;
+        }
       }
       asm volatile("bar.sync 2, 256;" ::: "memory");
-      float* vp = vecpart + (size_t)blockIdx.x * L.vec_len;
+      float* vp = vecpart + (size_t)blockIdx.x * L.vp_len;
       const float* ellv = ws_cptr<float>(a.stage, L.ell);
       float sgm = 0.f;
       for (int w = 0; w < 4; ++w) sgm += sc_s[w][VS_GMU];                 // k-half 0 warps, fixed order
@@ -1181,10 +1202,11 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
         vp[MP + d] = q;
         vp[MP + DP + d] = d < D ? ellv[d] * t1 + cen_s[d < DXW ? d : 0] * sgm : 0.f;
       }
-      if (et < VS_COUNT) {
+      if (et < VS_PART) {
         float sum = 0.f;
         if (et < 3) for (int w = 0; w < 4; ++w) sum += sc_s[w][et];
-        else if (KIND != GPBLUR_KERNEL_RBF) for (int w = 0; w < 8; ++w) sum += sc_s[w][et];   // VS_KBK: both k-halves
+        else if (et == VS_KBK ? KIND != GPBLUR_KERNEL_RBF : KIND == GPBLUR_KERNEL_RQ)
+          for (int w = 0; w < 8; ++w) sum += sc_s[w][et];   // VS_KBK / VS_KBA: both k-halves
         vp[MP + 2 * DP + et] = sum;
       }
     }
@@ -1192,6 +1214,19 @@ __global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) {
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 0) tc::tmem_dealloc(tmem_slot, TMEM_COLS);
+}
+
+template <int BQ, int BWO, int NSTB, int KIND>
+__global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_kernel(Tc2Args a) { tc2_fwd_body<BQ, BWO, NSTB, KIND>(a); }
+template <int BQ, int BWO, int NSTB>
+__global__ void __launch_bounds__(kCtaThreads, 1) tc2_fwd_rq_kernel(Tc2Args a) {
+  tc2_fwd_body<BQ, BWO, NSTB, GPBLUR_KERNEL_RQ>(a);
+}
+template <int BT, int DXW, int NSTA, int NSTB, int KIND>
+__global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_kernel(Tc2Args a) { tc2_bwd_body<BT, DXW, NSTA, NSTB, KIND>(a); }
+template <int BT, int DXW, int NSTA, int NSTB>
+__global__ void __launch_bounds__(kCtaThreads, 1) tc2_bwd_rq_kernel(Tc2Args a) {
+  tc2_bwd_body<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_RQ>(a);
 }
 
 int tc2_grid(const WsLayout& L) {
@@ -1209,8 +1244,12 @@ void set_smem(K kernel, size_t bytes) {
 template <int BQ, int BWO, int NSTB, int KIND>
 void launch_fwd_kind(const Tc2Args& a, int grid, cudaStream_t st) {
   const size_t smem = (size_t)NSTB * BWO * 256 + (size_t)(3 * a.L.MP + 3 * a.L.DP) * sizeof(float);
-  set_smem(tc2_fwd_kernel<BQ, BWO, NSTB, KIND>, smem);
-  tc2_fwd_kernel<BQ, BWO, NSTB, KIND><<<grid, kCtaThreads, smem, st>>>(a);
+  auto* kernel = [] {
+    if constexpr (KIND == GPBLUR_KERNEL_RQ) return tc2_fwd_rq_kernel<BQ, BWO, NSTB>;
+    else return tc2_fwd_kernel<BQ, BWO, NSTB, KIND>;
+  }();
+  set_smem(kernel, smem);
+  kernel<<<grid, kCtaThreads, smem, st>>>(a);
 }
 
 template <int BQ, int BWO, int NSTB>
@@ -1219,6 +1258,7 @@ int launch_fwd(const Tc2Args& a, int grid, cudaStream_t st) {
     case GPBLUR_KERNEL_MATERN12: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN12>(a, grid, st); break;
     case GPBLUR_KERNEL_MATERN32: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN32>(a, grid, st); break;
     case GPBLUR_KERNEL_MATERN52: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_MATERN52>(a, grid, st); break;
+    case GPBLUR_KERNEL_RQ: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_RQ>(a, grid, st); break;
     default: launch_fwd_kind<BQ, BWO, NSTB, GPBLUR_KERNEL_RBF>(a, grid, st);
   }
   return 0;
@@ -1229,8 +1269,12 @@ void launch_bwd_kind(const Tc2Args& a, int grid, cudaStream_t st) {
   constexpr size_t brows = BT > DXW ? BT : DXW;
   const size_t smem = (size_t)NSTB * brows * 256 +
                       (size_t)(2 * a.L.MP + 3 * DXW + TNP * (DXW + 4) + 8 * 32 * 20) * sizeof(float);
-  set_smem(tc2_bwd_kernel<BT, DXW, NSTA, NSTB, KIND>, smem);
-  tc2_bwd_kernel<BT, DXW, NSTA, NSTB, KIND><<<grid, kCtaThreads, smem, st>>>(a);
+  auto* kernel = [] {
+    if constexpr (KIND == GPBLUR_KERNEL_RQ) return tc2_bwd_rq_kernel<BT, DXW, NSTA, NSTB>;
+    else return tc2_bwd_kernel<BT, DXW, NSTA, NSTB, KIND>;
+  }();
+  set_smem(kernel, smem);
+  kernel<<<grid, kCtaThreads, smem, st>>>(a);
 }
 
 template <int BT, int DXW, int NSTA, int NSTB>
@@ -1239,6 +1283,7 @@ int launch_bwd(const Tc2Args& a, int grid, cudaStream_t st) {
     case GPBLUR_KERNEL_MATERN12: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN12>(a, grid, st); break;
     case GPBLUR_KERNEL_MATERN32: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN32>(a, grid, st); break;
     case GPBLUR_KERNEL_MATERN52: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_MATERN52>(a, grid, st); break;
+    case GPBLUR_KERNEL_RQ: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_RQ>(a, grid, st); break;
     default: launch_bwd_kind<BT, DXW, NSTA, NSTB, GPBLUR_KERNEL_RBF>(a, grid, st);
   }
   return 0;

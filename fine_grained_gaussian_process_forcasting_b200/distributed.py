@@ -37,9 +37,10 @@ class FlatGradBucket:
     accumulates straight into the bucket and the all-reduce needs no packing copy."""
 
     def __init__(self, params: Iterable[nn.Parameter], module: Optional[nn.Module] = None):
-        """`module`: if given, every single-output GP layer with a linear mean whose seven parameters are all in
-        `params` gets them laid out contiguously in the C-ABI bucket order (include/gpblur.h: Z, raw_lengthscale,
-        raw_outputscale, variational_mean, variational_stddev, weights, bias) and becomes a GRADIENT SINK: its M x M
+        """`module`: if given, every single-output GP layer with a linear mean whose parameters are all in `params`
+        gets them laid out contiguously in the C-ABI bucket order (include/gpblur.h: Z, raw_lengthscale,
+        raw_outputscale, variational_mean, variational_stddev, weights, bias, and raw_alpha for an RQKernel;
+        layer._layer_params()) and becomes a GRADIENT SINK: its M x M
         backward kernel accumulates straight into this buffer (``layer._grad_sink``) and autograd launches no
         per-parameter accumulation kernels for it."""
         self.params = list(params)
@@ -57,11 +58,11 @@ class FlatGradBucket:
                 mm = getattr(layer, "mean_module", None)
                 if layer.output_dims is not None or not isinstance(mm, LinearMean) or mm.bias is None:
                     continue
-                seven = list(layer._layer_params())
-                if all(id(p) in have and id(p) not in taken for p in seven):
-                    sinks.append((layer, seven))
-                    taken.update(id(p) for p in seven)
-            ordered = [p for _, seven in sinks for p in seven] + [p for p in self.params if id(p) not in taken]
+                lp = list(layer._layer_params())
+                if all(id(p) in have and id(p) not in taken for p in lp):
+                    sinks.append((layer, lp))
+                    taken.update(id(p) for p in lp)
+            ordered = [p for _, lp in sinks for p in lp] + [p for p in self.params if id(p) not in taken]
             self.params = ordered
         n = sum(p.numel() for p in self.params)
         self.flat = torch.zeros(n, device=dev, dtype=torch.float32)
@@ -71,9 +72,9 @@ class FlatGradBucket:
             starts[id(p)] = o
             p.grad = self.flat[o:o + p.numel()].view_as(p)
             o += p.numel()
-        for layer, seven in sinks:
-            a = starts[id(seven[0])]
-            layer._grad_sink = self.flat[a:a + sum(p.numel() for p in seven)]
+        for layer, lp in sinks:
+            a = starts[id(lp[0])]
+            layer._grad_sink = self.flat[a:a + sum(p.numel() for p in lp)]
 
     def zero(self):
         self.flat.zero_()

@@ -190,6 +190,23 @@ class MaternKernel(Kernel):
         return {0.5: "matern12", 1.5: "matern32", 2.5: "matern52"}[self.nu]
 
 
+class RQKernel(Kernel):
+    """gpytorch's RQKernel: k = (1 + d^2 / (2 alpha))^-alpha with a learnable alpha = softplus(raw_alpha), raw_alpha
+    of shape [*batch_shape, 1] (zeros: alpha = ln 2), evaluated by the same CUDA kernels as RBFKernel
+    (include/gpblur.h: GPBLUR_KERNEL_RQ)."""
+    has_lengthscale = True
+    kernel_name = "rq"
+
+    def __init__(self, alpha_constraint=None, **kwargs):
+        super().__init__(**kwargs)
+        self.register_parameter("raw_alpha", nn.Parameter(torch.zeros(*self.batch_shape, 1)))
+        self.raw_alpha_constraint = Positive() if alpha_constraint is None else alpha_constraint
+
+    @property
+    def alpha(self):
+        return self.raw_alpha_constraint.transform(self.raw_alpha)
+
+
 class ScaleKernel(Kernel):
     def __init__(self, base_kernel, outputscale_prior=None, outputscale_constraint=None, **kwargs):
         kwargs.pop("ard_num_dims", None)
@@ -204,19 +221,21 @@ class ScaleKernel(Kernel):
         return self.raw_outputscale_constraint.transform(self.raw_outputscale)
 
     def forward(self, x1, x2=None):
-        """Dense ScaleKernel(RBF | Matern) covariance by the CUDA kernel, differentiable w.r.t. the inputs and both raw
-        hyper-parameters (hand-written backward: gpblur_covariance_backward)."""
+        """Dense ScaleKernel(RBF | Matern | RQ) covariance by the CUDA kernel, differentiable w.r.t. the inputs and the
+        raw hyper-parameters (hand-written backward: gpblur_covariance_backward_alpha)."""
         x2 = x1 if x2 is None else x2
         bk = self.base_kernel
-        if not isinstance(bk, (RBFKernel, MaternKernel)) or len(self.batch_shape):
-            raise NotImplementedError("dense covariance: un-batched ScaleKernel(RBFKernel | MaternKernel) only")
+        if not isinstance(bk, _CUDA_KERNELS) or len(self.batch_shape):
+            raise NotImplementedError("dense covariance: un-batched ScaleKernel(RBFKernel | MaternKernel | RQKernel) "
+                                      "only")
         kernel = _base_kernel_name(bk)
+        raw_alpha = bk.raw_alpha if isinstance(bk, RQKernel) else None
         lead = x1.shape[:-2]
         x1f = x1.reshape(-1, x1.shape[-2], x1.shape[-1])
         x2f = x2.reshape(-1, x2.shape[-2], x2.shape[-1])
         same = x2 is x1
         outs = [ops.rbf_covariance(a, a if same else b, bk.raw_lengthscale, self.raw_outputscale, bk.ard_num_dims is not None,
-                                   kernel=kernel)
+                                   kernel=kernel, raw_alpha=raw_alpha)
                 for a, b in zip(x1f, x2f)]
         return torch.stack(outs).reshape(*lead, x1.shape[-2], x2.shape[-2])
 
@@ -225,14 +244,19 @@ def _base_kernel_name(base_kernel):
     return "rbf" if isinstance(base_kernel, RBFKernel) else base_kernel.kernel_name
 
 
+_CUDA_KERNELS = (RBFKernel, MaternKernel, RQKernel)
+
+
 def _kernel_raw_params(covar_module):
-    """(raw_lengthscale, raw_outputscale, kernel name) of a ScaleKernel(RBFKernel | MaternKernel) - anything else is
-    unsupported.  The name is what ops.svgp_predict takes as `kernel`."""
-    if not isinstance(covar_module, ScaleKernel) or not isinstance(covar_module.base_kernel, (RBFKernel, MaternKernel)):
-        raise NotImplementedError("the CUDA GP path implements ScaleKernel(RBFKernel | MaternKernel(ard_num_dims=D)) "
-                                  "(DeepGP.py:46-49); got %r" % type(covar_module).__name__)
+    """(raw_lengthscale, raw_outputscale, kernel name) of a ScaleKernel(RBFKernel | MaternKernel | RQKernel), and
+    raw_alpha after them for an RQKernel - anything else is unsupported.  The name is what ops.svgp_predict takes as
+    `kernel`."""
+    if not isinstance(covar_module, ScaleKernel) or not isinstance(covar_module.base_kernel, _CUDA_KERNELS):
+        raise NotImplementedError("the CUDA GP path implements ScaleKernel(RBFKernel | MaternKernel | "
+                                  "RQKernel(ard_num_dims=D)) (DeepGP.py:46-49); got %r" % type(covar_module).__name__)
     bk = covar_module.base_kernel
-    return bk.raw_lengthscale, covar_module.raw_outputscale, _base_kernel_name(bk)
+    return (bk.raw_lengthscale, covar_module.raw_outputscale, _base_kernel_name(bk)) + \
+        ((bk.raw_alpha,) if isinstance(bk, RQKernel) else ())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -518,11 +542,13 @@ class DeepGPLayer(ApproximateGP):
         raise NotImplementedError
 
     def _layer_params(self):
-        """Parameter tensors of the layer as the fused ops take them; a multi-output layer (output_dims = H) passes
-        its batched parameters ([H, M, D] inducing points ...) and is evaluated by ONE batched op."""
+        """Parameter tensors of the layer in the C-ABI gradient-bucket order (include/gpblur.h): Z, raw_lengthscale,
+        raw_outputscale, variational_mean, variational_stddev, weights, bias, and raw_alpha after them for an RQKernel.
+        A multi-output layer (output_dims = H) passes its batched parameters ([H, M, D] inducing points ...) and is
+        evaluated by ONE batched op."""
         vs = self.variational_strategy
         vd = vs._variational_distribution
-        raw_ell, raw_os, _ = _kernel_raw_params(self.covar_module)
+        raw_ell, raw_os, _, *alpha = _kernel_raw_params(self.covar_module)
         Z, m, s = vs.inducing_points, vd.variational_mean, vd._variational_stddev
         mm = self.mean_module
         if isinstance(mm, LinearMean):
@@ -531,18 +557,20 @@ class DeepGPLayer(ApproximateGP):
             w, b = None, mm.raw_constant
         else:
             raise NotImplementedError("mean module %r" % type(mm).__name__)
-        return Z, raw_ell, raw_os, m, s, w, b
+        return (Z, raw_ell, raw_os, m, s, w, b, *alpha)
 
-    def _kernel(self):
-        return _kernel_raw_params(self.covar_module)[2]
+    def _op_args(self):
+        """(the seven positional parameters of ops.svgp_*, keyword arguments kernel / raw_alpha)"""
+        p = self._layer_params()
+        return p[:7], {"kernel": _kernel_raw_params(self.covar_module)[2], "raw_alpha": p[7] if len(p) > 7 else None}
 
     def _stage_cache(self):
         return self._stage_caches.setdefault(None, {}) if self.share_param_stage else None
 
     def _kl_only(self):
-        _, kl, _, _ = ops.svgp_param_stage(*self._layer_params(), stage_cache=self._stage_cache(),
-                                           check=bool(check_cholesky.value()), grad_sink=self._grad_sink,
-                                           kernel=self._kernel())
+        params, kw = self._op_args()
+        _, kl, _, _ = ops.svgp_param_stage(*params, stage_cache=self._stage_cache(),
+                                           check=bool(check_cholesky.value()), grad_sink=self._grad_sink, **kw)
         return kl.sum() if kl.dim() else kl
 
     def __call__(self, inputs, are_samples=False, **kwargs):
@@ -563,12 +591,13 @@ class DeepGPLayer(ApproximateGP):
         n_pts = inputs.numel() // inputs.shape[-1]
         # GP h of a multi-output layer draws its sample with counters offset + h * n_pts + n
         seed, off, stream = self._next_counters(n_pts * (H or 1)) if self.fused_sample else (0, 0, 0)
-        mean, var, sample, kl, info = ops.svgp_predict(inputs, *self._layer_params(), seed, off, stream,
+        params, kw = self._op_args()
+        mean, var, sample, kl, info = ops.svgp_predict(inputs, *params, seed, off, stream,
                                                        want_sample=self.fused_sample,
                                                        stage_cache=self._stage_cache(),
                                                        offset_dev=self.rng_offset_dev, h_stride=self._rng_h_stride,
                                                        check=bool(check_cholesky.value()),
-                                                       grad_sink=self._grad_sink, kernel=self._kernel())
+                                                       grad_sink=self._grad_sink, **kw)
         self.last_info = info
         if H is None:
             cls = MultivariateNormal
@@ -596,11 +625,11 @@ class DeepGPLayer(ApproximateGP):
             raise RuntimeError(f"call_segments expects [N, {self.input_dims}] points, got {tuple(x_flat.shape)}")
         n_pts = x_flat.shape[0]
         seed, off, stream = self._next_counters(n_pts) if self.fused_sample else (0, 0, 0)
-        segs, kl, info = ops.svgp_predict_segments(x_flat, seg_shapes, *self._layer_params(), seed, off, stream,
+        params, kw = self._op_args()
+        segs, kl, info = ops.svgp_predict_segments(x_flat, seg_shapes, *params, seed, off, stream,
                                                    want_sample=self.fused_sample, stage_cache=self._stage_cache(),
                                                    offset_dev=self.rng_offset_dev,
-                                                   check=bool(check_cholesky.value()), grad_sink=self._grad_sink,
-                                                   kernel=self._kernel())
+                                                   check=bool(check_cholesky.value()), grad_sink=self._grad_sink, **kw)
         self.last_info = info
         vs._cache_kl(kl)
         S = num_likelihood_samples.value()

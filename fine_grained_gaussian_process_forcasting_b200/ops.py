@@ -51,13 +51,15 @@ def _f32c(t: Optional[Tensor]) -> Optional[Tensor]:
     return t.contiguous()
 
 
-def _params_struct(Z, raw_ell, raw_os, m, s, w, b) -> _cabi.SvgpParams:
+def _params_struct(Z, raw_ell, raw_os, m, s, w, b, raw_alpha=None) -> _cabi.SvgpParams:
     return _cabi.SvgpParams(Z.data_ptr(), raw_ell.data_ptr(), raw_os.data_ptr(), m.data_ptr(), s.data_ptr(),
-                            None if w is None else w.data_ptr(), b.data_ptr())
+                            None if w is None else w.data_ptr(), b.data_ptr(),
+                            None if raw_alpha is None else raw_alpha.data_ptr())
 
 
-def grad_bucket_floats(D: int, M: int) -> int:
-    return M * D + 2 * M + 2 * D + 2
+def grad_bucket_floats(D: int, M: int, kind: int = 0) -> int:
+    """Floats of the flat parameter-gradient bucket; the rational quadratic kind appends d raw_alpha."""
+    return M * D + 2 * M + 2 * D + 2 + (1 if kind == _cabi.KERNEL_KINDS["rq"] else 0)
 
 
 _WS_BYTES_CACHE = {}
@@ -133,8 +135,9 @@ def svgp_backward_raw(x, Z, raw_ell, raw_os, m, s, w, b, g_mean, g_var, g_sample
     return dx, bucket
 
 
-def split_bucket(bucket: Tensor, D: int, M: int, has_weights: bool):
-    """Views of the flat gradient bucket in parameter order (see include/gpblur.h)."""
+def split_bucket(bucket: Tensor, D: int, M: int, has_weights: bool, kernel: str = "rbf"):
+    """Views of the flat gradient bucket in parameter order (see include/gpblur.h); `kernel` "rq" appends the view of
+    d raw_alpha."""
     o = 0
     dZ = bucket[o:o + M * D].view(M, D); o += M * D
     dell = bucket[o:o + D]; o += D
@@ -142,7 +145,9 @@ def split_bucket(bucket: Tensor, D: int, M: int, has_weights: bool):
     dm = bucket[o:o + M]; o += M
     ds = bucket[o:o + M]; o += M
     dw = bucket[o:o + D] if has_weights else None; o += D
-    db = bucket[o:o + 1]
+    db = bucket[o:o + 1]; o += 1
+    if kernel == "rq":
+        return dZ, dell, dos, dm, ds, dw, db, bucket[o:o + 1]
     return dZ, dell, dos, dm, ds, dw, db
 
 
@@ -216,41 +221,45 @@ def philox_normal(seed: int, offset: int, n: int, stream_id: int = 0, device="cu
 
 
 def kernel_kind(kernel: str) -> int:
-    """Covariance function name ("rbf", "matern12", "matern32", "matern52") -> GPBLUR_KERNEL_* kind."""
+    """Covariance function name ("rbf", "matern12", "matern32", "matern52", "rq") -> GPBLUR_KERNEL_* kind."""
     kind = _cabi.KERNEL_KINDS.get(kernel)
     if kind is None:
         raise ValueError(f"unknown covariance function {kernel!r}: expected one of {sorted(_cabi.KERNEL_KINDS)}")
     return kind
 
 
-def _rbf_covariance_raw(x1, x2, raw_lengthscale, raw_outputscale, ard: bool, kind: int = 0) -> Tensor:
+def _rbf_covariance_raw(x1, x2, raw_lengthscale, raw_outputscale, ard: bool, kind: int = 0,
+                        raw_alpha: Optional[Tensor] = None) -> Tensor:
     n1, D = x1.shape
     n2 = x2.shape[0]
     out = torch.empty(n1, n2, device=x1.device, dtype=torch.float32)
     with torch.cuda.device(x1.device):
-        rc = _cabi.lib().gpblur_covariance(_ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(raw_lengthscale),
-                                           int(ard), _ptr(raw_outputscale), _ptr(out), _stream())
-    _cabi.check(rc, "gpblur_covariance")
+        rc = _cabi.lib().gpblur_covariance_alpha(_ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(raw_lengthscale),
+                                                 int(ard), _ptr(raw_outputscale), _ptr(raw_alpha), _ptr(out), _stream())
+    _cabi.check(rc, "gpblur_covariance_alpha")
     return out
 
 
 class _RbfCovFunction(torch.autograd.Function):
-    """Dense ScaleKernel(RBF | Matern) covariance with its hand-written backward (gpblur_covariance_backward):
-    gradients of the inputs, the raw lengthscale(s) and the raw outputscale."""
+    """Dense ScaleKernel(RBF | Matern | RQ) covariance with its hand-written backward
+    (gpblur_covariance_backward_alpha): gradients of the inputs, the raw lengthscale(s), the raw outputscale and (RQ)
+    raw_alpha."""
 
     @staticmethod
-    def forward(ctx, x1, x2, raw_lengthscale, raw_outputscale, ard, kind=0):
+    def forward(ctx, x1, x2, raw_lengthscale, raw_outputscale, ard, kind=0, raw_alpha=None):
         same = x2 is x1
         x1c, ellc, osc = _f32c(x1), _f32c(raw_lengthscale).reshape(-1), _f32c(raw_outputscale).reshape(-1)
         x2c = x1c if same else _f32c(x2)
-        ctx.save_for_backward(x1c, x2c, ellc, osc)
-        ctx.meta = (bool(ard), same, raw_lengthscale.shape, raw_outputscale.shape, int(kind))
-        return _rbf_covariance_raw(x1c, x2c, ellc, osc, ard, kind)
+        ac = None if raw_alpha is None else _f32c(raw_alpha).reshape(-1)
+        ctx.save_for_backward(x1c, x2c, ellc, osc, ac)
+        ctx.meta = (bool(ard), same, raw_lengthscale.shape, raw_outputscale.shape, int(kind),
+                    None if raw_alpha is None else raw_alpha.shape)
+        return _rbf_covariance_raw(x1c, x2c, ellc, osc, ard, kind, ac)
 
     @staticmethod
     def backward(ctx, g_out):
-        x1, x2, ell, os_ = ctx.saved_tensors
-        ard, same, ell_shape, os_shape, kind = ctx.meta
+        x1, x2, ell, os_, ac = ctx.saved_tensors
+        ard, same, ell_shape, os_shape, kind, a_shape = ctx.meta
         n1, D = x1.shape
         n2 = x2.shape[0]
         dev = x1.device
@@ -260,28 +269,34 @@ class _RbfCovFunction(torch.autograd.Function):
         g_x2 = torch.empty(n2, D, device=dev, dtype=torch.float32) if want_x2 else None
         g_ell = torch.empty(D if ard else 1, device=dev, dtype=torch.float32)
         g_os = torch.empty(1, device=dev, dtype=torch.float32)
+        g_a = None if ac is None else torch.empty(1, device=dev, dtype=torch.float32)
         nbytes = int(_cabi.lib().gpblur_covariance_backward_scratch_bytes(n1, n2, D, kind))
         scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
         with torch.cuda.device(dev):
-            rc = _cabi.lib().gpblur_covariance_backward(_ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(ell), int(ard),
-                                                        _ptr(os_), _ptr(_f32c(g_out)), _ptr(g_x1), _ptr(g_x2),
-                                                        _ptr(g_ell), _ptr(g_os), _ptr(scratch), nbytes, _stream())
-        _cabi.check(rc, "gpblur_covariance_backward")
+            rc = _cabi.lib().gpblur_covariance_backward_alpha(
+                _ptr(x1), _ptr(x2), n1, n2, D, kind, _ptr(ell), int(ard), _ptr(os_), _ptr(ac), _ptr(_f32c(g_out)),
+                _ptr(g_x1), _ptr(g_x2), _ptr(g_ell), _ptr(g_os), _ptr(g_a), _ptr(scratch), nbytes, _stream())
+        _cabi.check(rc, "gpblur_covariance_backward_alpha")
+        ga = None if g_a is None else g_a.reshape(a_shape)
         if same:                       # K(x, x): the one tensor is both arguments
             gx = g_x1 + g_x2 if (need[0] or need[1]) else None
-            return gx if need[0] else None, None, g_ell.reshape(ell_shape), g_os.reshape(os_shape), None, None
+            return gx if need[0] else None, None, g_ell.reshape(ell_shape), g_os.reshape(os_shape), None, None, ga
         return (g_x1 if need[0] else None, g_x2 if need[1] else None, g_ell.reshape(ell_shape), g_os.reshape(os_shape),
-                None, None)
+                None, None, ga)
 
 
 def rbf_covariance(x1: Tensor, x2: Tensor, raw_lengthscale: Tensor, raw_outputscale: Tensor, ard: bool,
-                   kernel: str = "rbf") -> Tensor:
+                   kernel: str = "rbf", raw_alpha: Optional[Tensor] = None) -> Tensor:
     """os * f(|(x1 - x2) / l|) [n1, n2] (f: exp(-d^2 / 2) for "rbf", the Matern functions of include/gpblur.h for
-    "matern12" / "matern32" / "matern52"); differentiable w.r.t. x1, x2 and both raw hyper-parameters."""
-    _need_cuda(x1, x2, raw_lengthscale, raw_outputscale)
+    "matern12" / "matern32" / "matern52", (1 + d^2 / (2 alpha))^-alpha for "rq", which needs `raw_alpha` [1]);
+    differentiable w.r.t. x1, x2 and the raw hyper-parameters."""
+    _need_cuda(x1, x2, raw_lengthscale, raw_outputscale, raw_alpha)
     if raw_lengthscale.numel() != (x1.shape[-1] if ard else 1):
         raise ValueError("rbf_covariance: raw_lengthscale must hold D values (ard) or one")
-    return _RbfCovFunction.apply(x1, x2, raw_lengthscale, raw_outputscale, bool(ard), kernel_kind(kernel))
+    kind = kernel_kind(kernel)
+    if (kernel == "rq") != (raw_alpha is not None) or (raw_alpha is not None and raw_alpha.numel() != 1):
+        raise ValueError("rbf_covariance: raw_alpha (one value) is given for kernel 'rq' and only for it")
+    return _RbfCovFunction.apply(x1, x2, raw_lengthscale, raw_outputscale, bool(ard), kind, raw_alpha)
 
 
 def debug_fetch(which: int, N: int, D: int, M: int, ws: Tensor) -> Tensor:
@@ -312,18 +327,19 @@ def debug_fetch(which: int, N: int, D: int, M: int, ws: Tensor) -> Tensor:
 # ------------------------------------------------------------------------------------------------
 # autograd
 # ------------------------------------------------------------------------------------------------
-def stage_grad_doubles(D: int, M: int) -> int:
-    return int(_cabi.lib().gpblur_svgp_stage_grad_doubles(D, M))
+def stage_grad_doubles(D: int, M: int, kind: int = 0) -> int:
+    return int(_cabi.lib().gpblur_svgp_stage_grad_doubles_kind(D, M, kind))
 
 
 def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: float = 0.0, max_ctas: int = 0,
-                    kind: int = 0):
+                    kind: int = 0, raw_alpha: Optional[Tensor] = None):
     """Once-per-parameter-update M x M stage: -> (stage uint8 [param_stage_bytes], kl [1], info [1] int32).
     `out` = preallocated (stage, kl, info) (the call then only launches on the current stream).
     `extra_jitter` is added to the diagonal of Kzz on top of the variational jitter (psd_safe_cholesky retries).
     `max_ctas` > 0 bounds the cooperative grid (stages of a multi-output layer running side by side, see _Fork).
-    `kind`: covariance function (kernel_kind); the point and backward calls on this stage must pass the same."""
-    _need_cuda(Z, raw_ell, raw_os, m, s, w, b)
+    `kind`: covariance function (kernel_kind); the point and backward calls on this stage must pass the same.
+    `raw_alpha` [1]: the rational quadratic kind's shape parameter (read for that kind only)."""
+    _need_cuda(Z, raw_ell, raw_os, m, s, w, b, raw_alpha)
     M, D = Z.shape
     dev = Z.device
     if out is None:
@@ -332,7 +348,7 @@ def param_stage_raw(Z, raw_ell, raw_os, m, s, w, b, out=None, extra_jitter: floa
         info = torch.empty(1, device=dev, dtype=torch.int32)
     else:
         stage, kl, info = out
-    p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
+    p = _params_struct(Z, raw_ell, raw_os, m, s, w, b, raw_alpha)
     with torch.cuda.device(dev):
         rc = _cabi.lib().gpblur_svgp_param_stage(C.byref(p), D, M, int(kind), float(extra_jitter), int(max_ctas),
                                                  _ptr(kl), _ptr(info), _ptr(stage), stage.numel(), _stream())
@@ -394,7 +410,7 @@ def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, of
     elif dx is None:
         dx = torch.empty(N, D, device=dev, dtype=torch.float32)
     if sgrad is None:
-        sgrad = torch.empty(stage_grad_doubles(D, M), device=dev, dtype=torch.float64)
+        sgrad = torch.empty(stage_grad_doubles(D, M, kind), device=dev, dtype=torch.float64)
     with torch.cuda.device(dev):
         rc = _cabi.lib().gpblur_svgp_point_backward(
             _ptr(stage), _ptr(x), N, D, M, int(kind), nseg, (C.c_longlong * nseg)(*starts), ptr_array(gm), ptr_array(gv),
@@ -406,14 +422,14 @@ def point_backward_raw(x: Tensor, M: int, g_mean, g_var, g_sample, var, seed, of
 
 def param_stage_backward_raw(Z, raw_ell, raw_os, m, s, w, b, sgrad: Tensor, g_kl: Optional[Tensor], stage: Tensor,
                              bucket: Optional[Tensor] = None, accumulate: bool = False, max_ctas: int = 0,
-                             kind: int = 0):
-    """Summed stage gradient (+ g_kl) -> flat parameter-gradient bucket [M*D + 2M + 2D + 2] (`accumulate`: added to
-    `bucket` instead of overwriting it)."""
-    _need_cuda(Z, sgrad, stage, g_kl)
+                             kind: int = 0, raw_alpha: Optional[Tensor] = None):
+    """Summed stage gradient (+ g_kl) -> flat parameter-gradient bucket [grad_bucket_floats(D, M, kind)]
+    (`accumulate`: added to `bucket` instead of overwriting it)."""
+    _need_cuda(Z, sgrad, stage, g_kl, raw_alpha)
     M, D = Z.shape
     if bucket is None:
-        bucket = torch.empty(grad_bucket_floats(D, M), device=Z.device, dtype=torch.float32)
-    p = _params_struct(Z, raw_ell, raw_os, m, s, w, b)
+        bucket = torch.empty(grad_bucket_floats(D, M, kind), device=Z.device, dtype=torch.float32)
+    p = _params_struct(Z, raw_ell, raw_os, m, s, w, b, raw_alpha)
     with torch.cuda.device(Z.device):
         rc = _cabi.lib().gpblur_svgp_param_stage_backward(
             C.byref(p), D, M, int(kind), _ptr(sgrad), _ptr(g_kl), _ptr(bucket), int(accumulate), int(max_ctas),
@@ -504,7 +520,7 @@ class _ParamStageFunction(torch.autograd.Function):
     side streams so that they overlap on the GPU."""
 
     @staticmethod
-    def forward(ctx, Z, raw_ell, raw_os, m, s, w, b, holder):
+    def forward(ctx, Z, raw_ell, raw_os, m, s, w, b, holder, raw_alpha=None):
         batched = Z.dim() == 3
         H = Z.shape[0] if batched else 1
         M, D = Z.shape[-2], Z.shape[-1]
@@ -515,6 +531,7 @@ class _ParamStageFunction(torch.autograd.Function):
         sc = _f32c(s).reshape(H, M)
         wc = None if w is None else _f32c(w).reshape(-1, D)           # [1, D] shared or [H, D]
         bc = _f32c(b).reshape(-1, 1)                                  # [1, 1] shared or [H, 1]
+        ac = None if raw_alpha is None else _f32c(raw_alpha).reshape(H, 1)   # rational quadratic: [H, 1]
         dev = Zc.device
         _need_cuda(Zc)
         stage = torch.empty(H, param_stage_bytes(D, M), device=dev, dtype=torch.uint8)
@@ -528,18 +545,19 @@ class _ParamStageFunction(torch.autograd.Function):
                 param_stage_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h], None if wc is None else wc[h % wc.shape[0]],
                                 bc[h % bc.shape[0]], out=(stage[h], kl[h:h + 1], info[h:h + 1]),
                                 extra_jitter=float(holder.get("extra_jitter", 0.0)), max_ctas=cap,
-                                kind=holder["kind"])
+                                kind=holder["kind"], raw_alpha=None if ac is None else ac[h])
         finally:
             fork.join()
         holder["stage"] = stage
         holder["consumed"] = False
         ctx.holder = holder
         ctx.batched = batched
-        ctx.save_for_backward(Zc, ellc, osc, mc, sc, wc, bc)
-        ctx.shapes = (Z.shape, raw_ell.shape, raw_os.shape, m.shape, s.shape, None if w is None else w.shape, b.shape)
+        ctx.save_for_backward(Zc, ellc, osc, mc, sc, wc, bc, ac)
+        ctx.shapes = (Z.shape, raw_ell.shape, raw_os.shape, m.shape, s.shape, None if w is None else w.shape, b.shape,
+                      None if raw_alpha is None else raw_alpha.shape)
         ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(info)
-        G = stage_grad_doubles(D, M)
+        G = stage_grad_doubles(D, M, holder["kind"])
         token = _zero64(dev).expand((H, G) if batched else (G,))   # carrier of the stage gradient: never written
         return token, (kl if batched else kl.reshape(())), info
 
@@ -550,17 +568,17 @@ class _ParamStageFunction(torch.autograd.Function):
 
     @staticmethod
     def _backward(ctx, g_token, g_kl, _g_info):
-        Zc, ellc, osc, mc, sc, wc, bc = ctx.saved_tensors
+        Zc, ellc, osc, mc, sc, wc, bc, ac = ctx.saved_tensors
         holder = ctx.holder
         H, M, D = Zc.shape
         dev = Zc.device
-        G = stage_grad_doubles(D, M)
+        G = stage_grad_doubles(D, M, holder["kind"])
         if g_token is None:
             sgrad = torch.zeros(H, G, device=dev, dtype=torch.float64)
         else:
             sgrad = g_token.to(torch.float64).reshape(H, G).contiguous()
         gk = None if g_kl is None else _f32c(g_kl).reshape(-1).expand(H).contiguous()
-        nb = grad_bucket_floats(D, M)
+        nb = grad_bucket_floats(D, M, holder["kind"])
         stage = holder["stage"]
         sink = holder.get("grad_sink")
         if sink is not None and H == 1 and wc is not None:
@@ -568,9 +586,9 @@ class _ParamStageFunction(torch.autograd.Function):
             # (distributed.FlatGradBucket): the kernel accumulates straight into it, autograd gets no gradient to add
             param_stage_backward_raw(Zc[0], ellc[0], osc[0], mc[0], sc[0], wc[0], bc[0], sgrad[0],
                                      None if gk is None else gk[0:1], stage[0], bucket=sink, accumulate=True,
-                                     kind=holder["kind"])
+                                     kind=holder["kind"], raw_alpha=None if ac is None else ac[0])
             holder["consumed"] = True
-            return (None,) * 8
+            return (None,) * 9
         bucket = torch.empty(H, nb, device=dev, dtype=torch.float32)
         fork = _Fork(dev, H)
         cap = _stage_cta_cap(dev, H)
@@ -580,7 +598,7 @@ class _ParamStageFunction(torch.autograd.Function):
                 param_stage_backward_raw(Zc[h], ellc[h], osc[h], mc[h], sc[h],
                                          None if wc is None else wc[h % wc.shape[0]], bc[h % bc.shape[0]], sgrad[h],
                                          None if gk is None else gk[h:h + 1], stage[h], bucket=bucket[h], max_ctas=cap,
-                                         kind=holder["kind"])
+                                         kind=holder["kind"], raw_alpha=None if ac is None else ac[h])
         finally:
             fork.join()
         holder["consumed"] = True        # the graph behind this token is gone: the next forward rebuilds the stage
@@ -591,7 +609,8 @@ class _ParamStageFunction(torch.autograd.Function):
         dm = bucket[:, o:o + M]; o += M
         ds = bucket[:, o:o + M]; o += M
         dw = bucket[:, o:o + D]; o += D
-        db = bucket[:, o:o + 1]
+        db = bucket[:, o:o + 1]; o += 1
+        da = bucket[:, o:o + 1]                                       # rational quadratic: d raw_alpha
         shp = ctx.shapes
         need = ctx.needs_input_grad
 
@@ -606,7 +625,8 @@ class _ParamStageFunction(torch.autograd.Function):
                 ds.reshape(shp[4]) if need[4] else None,
                 shared(dw, shp[5], wc.shape[0]) if (wc is not None and need[5]) else None,
                 shared(db, shp[6], bc.shape[0]) if need[6] else None,
-                None)
+                None,
+                da.reshape(shp[7]) if (ac is not None and need[8]) else None)
 
 
 class _PointFunction(torch.autograd.Function):
@@ -672,7 +692,7 @@ class _PointFunction(torch.autograd.Function):
 
         gm, gv, gs = prep(g_mean), prep(g_var), prep(g_sample)
         need = ctx.needs_input_grad
-        G = stage_grad_doubles(D, M)
+        G = stage_grad_doubles(D, M, ctx.kind)
         sgrad = torch.empty(H, G, device=dev, dtype=torch.float64)
         dx = torch.empty(H, N, D, device=dev, dtype=torch.float32) if need[0] else None
         fork = _Fork(dev, H)
@@ -691,10 +711,11 @@ class _PointFunction(torch.autograd.Function):
                 None)
 
 
-def _stage_key(Z, raw_ell, raw_os, m, s, w, b):
+def _stage_key(Z, raw_ell, raw_os, m, s, w, b, raw_alpha=None):
     key = tuple((t._version, t.data_ptr()) for t in (Z, raw_ell, raw_os, m, s, b))
-    if w is not None:
-        key += ((w._version, w.data_ptr()),)
+    for t in (w, raw_alpha):
+        if t is not None:
+            key += ((t._version, t.data_ptr()),)
     return key + (tuple(Z.shape),)
 
 
@@ -713,19 +734,23 @@ JITTER_RETRIES = (1e-6, 1e-5, 1e-4)
 def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outputscale: Tensor,
                      variational_mean: Tensor, variational_stddev: Tensor, mean_weights: Optional[Tensor],
                      mean_bias: Tensor, stage_cache: Optional[dict] = None, check: bool = False,
-                     grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
-    """-> (token, kl, info, holder).  `kernel`: covariance function ("rbf", "matern12", "matern32", "matern52"); it
-    is part of the stage-cache key and travels in `holder` to every call on the stage.  With `stage_cache` (a dict owned by the caller, one per GP layer) consecutive
+                     grad_sink: Optional[Tensor] = None, kernel: str = "rbf", raw_alpha: Optional[Tensor] = None):
+    """-> (token, kl, info, holder).  `kernel`: covariance function ("rbf", "matern12", "matern32", "matern52", "rq"); it
+    is part of the stage-cache key and travels in `holder` to every call on the stage.  `raw_alpha` ([1], or [H, 1]
+    for a multi-output layer): the shape parameter of "rq", differentiable like the other parameters; given for "rq"
+    and only for it.  With `stage_cache` (a dict owned by the caller, one per GP layer) consecutive
     calls with unchanged parameter tensors (same `_version`) share one stage - and therefore one M x M backward -
     until a backward pass has consumed it.  Parameters with a leading H (inducing points [H, M, D]) describe the H
     independent GPs of a multi-output layer: kl is [H], token [H, G]."""
     params = (inducing_points, raw_lengthscale, raw_outputscale, variational_mean, variational_stddev, mean_weights,
               mean_bias)
-    want_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in params)
     kind = kernel_kind(kernel)
+    if (kernel == "rq") != (raw_alpha is not None):
+        raise ValueError("raw_alpha is given for kernel 'rq' and only for it")
+    want_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in params + (raw_alpha,))
     key = None
     if stage_cache is not None:
-        key = _stage_key(*params) + (kind,)
+        key = _stage_key(*params, raw_alpha) + (kind,)
         ent = stage_cache.get("entry")
         if ent is not None and stage_cache.get("key") == key and not ent[3]["consumed"] \
                 and ent[0].requires_grad == want_grad:
@@ -734,7 +759,7 @@ def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outpu
     if grad_sink is not None:
         holder["grad_sink"] = grad_sink
     with torch.cuda.nvtx.range("gpblur.param_stage") if _NVTX else _null_ctx():
-        token, kl, info = _ParamStageFunction.apply(*params, holder)
+        token, kl, info = _ParamStageFunction.apply(*params, holder, raw_alpha)
     # Cholesky status (LAPACK-style info, 0 = ok).  Reading it synchronises with the device, as gpytorch's
     # psd_safe_cholesky does; it is skipped while a CUDA graph is being captured (check GraphedStep.check_info()).
     if check and not torch._C._cuda_isCurrentStreamCapturing():
@@ -745,7 +770,7 @@ def svgp_param_stage(inducing_points: Tensor, raw_lengthscale: Tensor, raw_outpu
                 holder = {"kind": kind, "extra_jitter": jit}
                 if grad_sink is not None:
                     holder["grad_sink"] = grad_sink
-                token, kl, info = _ParamStageFunction.apply(*params, holder)
+                token, kl, info = _ParamStageFunction.apply(*params, holder, raw_alpha)
                 if int(info.max().item()) == 0:
                     warnings.warn(f"Kzz + 1e-4 I is not positive definite (pivot {k}): added jitter of {jit:.1e} to the "
                                   f"diagonal", NumericalWarning)
@@ -765,16 +790,16 @@ def svgp_predict(x: Tensor, inducing_points: Tensor, raw_lengthscale: Tensor, ra
                  mean_bias: Tensor, seed: int = 0, offset: int = 0, stream_id: int = 0,
                  want_sample: bool = False, stage_cache: Optional[dict] = None,
                  offset_dev: Optional[Tensor] = None, h_stride: Optional[int] = None, check: bool = False,
-                 grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
+                 grad_sink: Optional[Tensor] = None, kernel: str = "rbf", raw_alpha: Optional[Tensor] = None):
     """x [..., D] -> (mean [...], var [...], sample [...] | None, kl [], info [1]); with inducing points [H, M, D]
     (multi-output layer) the outputs are [..., H], kl [H], info [H], and GP h draws its sample with Philox counters
     offset + h * h_stride + n (h_stride defaults to the N points of this call; batch-sharded callers pass the GLOBAL
     point count so that the counters do not depend on the number of ranks).  `stage_cache`: see svgp_param_stage.  `offset_dev`: optional int64 device scalar added to
-    `offset` when the kernels run (CUDA-graph replays draw fresh counters by bumping it between replays).  `kernel`:
-    covariance function, see svgp_param_stage."""
+    `offset` when the kernels run (CUDA-graph replays draw fresh counters by bumping it between replays).  `kernel`,
+    `raw_alpha`: covariance function, see svgp_param_stage."""
     token, kl, info, holder = svgp_param_stage(inducing_points, raw_lengthscale, raw_outputscale, variational_mean,
                                                variational_stddev, mean_weights, mean_bias, stage_cache, check=check,
-                                               grad_sink=grad_sink, kernel=kernel)
+                                               grad_sink=grad_sink, kernel=kernel, raw_alpha=raw_alpha)
     if x.numel() == 0:
         shp = tuple(x.shape[:-1]) + ((token.shape[0],) if token.dim() == 2 else ())
         e = x.new_empty(shp, dtype=torch.float32)
@@ -855,7 +880,8 @@ def svgp_predict_segments(x: Tensor, seg_shapes, inducing_points: Tensor, raw_le
                           mean_weights: Optional[Tensor], mean_bias: Tensor, seed: int = 0, offset: int = 0,
                           stream_id: int = 0, want_sample: bool = False, stage_cache: Optional[dict] = None,
                           offset_dev: Optional[Tensor] = None, check: bool = False,
-                          grad_sink: Optional[Tensor] = None, kernel: str = "rbf"):
+                          grad_sink: Optional[Tensor] = None, kernel: str = "rbf",
+                          raw_alpha: Optional[Tensor] = None):
     """svgp_predict for a single-output GP on x [N, D] = the concatenated points of several activations;
     ``seg_shapes`` (e.g. [(B, 192), (B, 24)]) are the output shapes of the segments, in order.
     -> ([(mean, var, sample | None) per segment], kl, info)."""
@@ -863,7 +889,7 @@ def svgp_predict_segments(x: Tensor, seg_shapes, inducing_points: Tensor, raw_le
         raise ValueError("svgp_predict_segments: single-output layers only")
     token, kl, info, holder = svgp_param_stage(inducing_points, raw_lengthscale, raw_outputscale, variational_mean,
                                                variational_stddev, mean_weights, mean_bias, stage_cache, check=check,
-                                               grad_sink=grad_sink, kernel=kernel)
+                                               grad_sink=grad_sink, kernel=kernel, raw_alpha=raw_alpha)
     with torch.cuda.nvtx.range("gpblur.point_forward") if _NVTX else _null_ctx():
         flat = _PointSegFunction.apply(x, token, holder, int(inducing_points.shape[-2]), int(seed), int(offset),
                                        int(stream_id), bool(want_sample), offset_dev,

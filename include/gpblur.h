@@ -42,12 +42,15 @@ extern "C" {
  *   MATERN12    f = exp(-r)                              (gpytorch MaternKernel(nu=0.5))
  *   MATERN32    f = (1 + sqrt3 r) exp(-sqrt3 r)          (nu=1.5)
  *   MATERN52    f = (1 + sqrt5 r + 5/3 r^2) exp(-sqrt5 r) (nu=2.5)
+ *   RQ          f = (1 + d2 / (2 alpha))^-alpha          (gpytorch RQKernel; d2 unclamped, alpha = softplus(raw_alpha))
+ *               df/dalpha = f (u / (1 + u) - log1p(u)), u = d2 / (2 alpha)
  * An unknown kind returns GPBLUR_EINVAL.  A parameter stage must be consumed (point forward / backward, stage backward)
  * with the kind it was built with; nothing on the device checks this. */
 #define GPBLUR_KERNEL_RBF 0
 #define GPBLUR_KERNEL_MATERN12 1
 #define GPBLUR_KERNEL_MATERN32 2
 #define GPBLUR_KERNEL_MATERN52 3
+#define GPBLUR_KERNEL_RQ 4
 
 /* Parameters of one whitened sparse variational GP layer.
  * Replaces the parameter set created by ToyDeepGPHiddenLayer.__init__
@@ -60,6 +63,8 @@ typedef struct gpblur_svgp_params {
   const float* variational_stddev; /* [M]      _variational_distribution._variational_stddev */
   const float* mean_weights;       /* [D] LinearMean.weights, or NULL for ConstantMean    */
   const float* mean_bias;          /* [1] LinearMean.bias / ConstantMean constant         */
+  const float* raw_alpha;          /* [1], read only for GPBLUR_KERNEL_RQ (NULL then: GPBLUR_EINVAL)
+                                      covar_module.base_kernel.raw_alpha                 */
 } gpblur_svgp_params;
 
 /* Number of floats in the flat parameter-gradient bucket written by gpblur_svgp_backward:
@@ -67,6 +72,8 @@ typedef struct gpblur_svgp_params {
  *     d variational_stddev (M) | d mean_weights (D) | d mean_bias (1) ]
  * This bucket is what data-parallel training all-reduces. */
 size_t gpblur_svgp_grad_bucket_floats(int D, int M);
+/* The bucket of a layer of kind `kind`: for GPBLUR_KERNEL_RQ one more trailing float, d raw_alpha. */
+size_t gpblur_svgp_grad_bucket_floats_kind(int D, int M, int kind);
 
 /* Scratch bytes for N input points.  `training` != 0 reserves room for the saved whitened
  * cross-covariance A [N, Mp] and the backward intermediates. */
@@ -111,11 +118,13 @@ int gpblur_svgp_backward(const gpblur_svgp_params* p, const float* x, long long 
  *   gpblur_svgp_point_backward       upstream grads -> dx, stage_grad (fp64)      [one per forward call]
  *   gpblur_svgp_param_stage_backward (stage, SUM of the stage_grads, g_kl) -> flat parameter-gradient bucket
  *
- * stage_grad holds gpblur_svgp_stage_grad_doubles(D, M) doubles:
- *   [ u (Mp) | colsum(W) (Mp), q (Dp), wbar (Dp), scalars (4) | S = sum g_var a a^T (Mp x Mp) | W^T X (Mp x Dp) ]
+ * stage_grad holds gpblur_svgp_stage_grad_doubles_kind(D, M, kind) doubles:
+ *   [ u (Mp) | colsum(W) (Mp), q (Dp), wbar (Dp), scalars (4) | S = sum g_var a a^T (Mp x Mp) | W^T X (Mp x Dp) |
+ *     GPBLUR_KERNEL_RQ only: sum kbar o dk/dalpha (1) ]
  * gpblur_svgp_forward / gpblur_svgp_backward above are the single-call compositions of these four (RBF, the stage
  * built in `ws`).  All four calls on one stage take the same `kind` (GPBLUR_KERNEL_*). */
-size_t gpblur_svgp_stage_grad_doubles(int D, int M);
+size_t gpblur_svgp_stage_grad_doubles(int D, int M);   /* every kind but RQ */
+size_t gpblur_svgp_stage_grad_doubles_kind(int D, int M, int kind);
 
 /* Parameters -> M x M stage in `stage` (256-byte aligned, gpblur_svgp_param_stage_bytes(D, M) bytes), kl [1], info [1].
  * `extra_jitter` >= 0 is added to the diagonal of Kzz on top of the variational jitter 1e-4.  It replaces the retry
@@ -199,9 +208,13 @@ int gpblur_rsample_backward(const float* var, const float* g_out, long long n, u
                             void* stream);
 
 /* Dense ScaleKernel covariance of kind `kind` for the exact-GP model (/root/reference/denoising_model/GPModel.py:10-13):
- * x1 [n1, D], x2 [n2, D], raw_lengthscale [D] (ard != 0) or [1] -> out [n1, n2]. */
+ * x1 [n1, D], x2 [n2, D], raw_lengthscale [D] (ard != 0) or [1] -> out [n1, n2].  gpblur_covariance_alpha also takes
+ * raw_alpha [1], read only for GPBLUR_KERNEL_RQ (NULL then: GPBLUR_EINVAL); gpblur_covariance passes NULL. */
 int gpblur_covariance(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
                       const float* raw_lengthscale, int ard, const float* raw_outputscale, float* out, void* stream);
+int gpblur_covariance_alpha(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                            const float* raw_lengthscale, int ard, const float* raw_outputscale, const float* raw_alpha,
+                            float* out, void* stream);
 
 /* Backward of gpblur_covariance (what autograd computes through the kernel evaluation when the exact GP of
  * /root/reference/denoising_model/GPModel.py:4-13 is trained): g_out [n1, n2] -> g_x1 [n1, D] (nullable), g_x2 [n2, D]
@@ -213,6 +226,12 @@ int gpblur_covariance_backward(const float* x1, const float* x2, long long n1, l
                                const float* raw_lengthscale, int ard, const float* raw_outputscale,
                                const float* g_out, float* g_x1, float* g_x2, float* g_raw_lengthscale,
                                float* g_raw_outputscale, void* scratch, size_t scratch_bytes, void* stream);
+/* The same with raw_alpha [1] and g_raw_alpha [1] (both read / written only for GPBLUR_KERNEL_RQ, which needs them). */
+int gpblur_covariance_backward_alpha(const float* x1, const float* x2, long long n1, long long n2, int D, int kind,
+                                     const float* raw_lengthscale, int ard, const float* raw_outputscale,
+                                     const float* raw_alpha, const float* g_out, float* g_x1, float* g_x2,
+                                     float* g_raw_lengthscale, float* g_raw_outputscale, float* g_raw_alpha,
+                                     void* scratch, size_t scratch_bytes, void* stream);
 
 /* Debug / test probes into the workspace of the last forward on (ws): copies device-to-device.
  * which: 0 = L (fp64 [Mp,Mp]), 1 = Linv (fp64 [Mp,Mp]), 2 = Kzz+jitter (fp64 [Mp,Mp]),

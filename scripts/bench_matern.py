@@ -1,8 +1,9 @@
-"""Step time of the GP blur with each covariance function: RBF and Matern nu = 1/2, 3/2, 5/2.
+"""Step time of the GP blur with each covariance function: RBF, Matern nu = 1/2, 3/2, 5/2 and rational quadratic.
 
 For the workloads c1 (FP32-FFMA point kernels, M = 32), c2 (two calls per step, M = 256) and c5_m256 of bench.py, the
-model of bench.make_model (exercise_init parameters) is built once per covariance function - the Matern layers take
-the same raw parameter values, only covar_module is swapped, the gpytorch idiom - and its forward + backward step is
+model of bench.make_model (exercise_init parameters) is built once per covariance function - the Matern and RQ layers
+take the same raw parameter values (RQ: raw_alpha = 0, alpha = ln 2), only covar_module is swapped, the gpytorch
+idiom - and its forward + backward step is
 captured in a CUDA graph (GraphedStep).  The kernels are then timed in rounds that alternate between them, so that a
 drift of the clocks or of the other work on the machine hits them alike.  Prints the card name and power limit, one
 JSON line per workload with the median ms per step and the ratio to RBF, and (c2) the per-stage times of the library's
@@ -23,7 +24,7 @@ sys.dont_write_bytecode = True
 
 import torch  # noqa: E402
 
-KERNELS = {"rbf": None, "matern12": 0.5, "matern32": 1.5, "matern52": 2.5}
+KERNELS = {"rbf": None, "matern12": 0.5, "matern32": 1.5, "matern52": 2.5, "rq": "rq"}
 
 
 def card():
@@ -39,9 +40,13 @@ def swap_kernel(model, nu):
     for layer in [m for m in model.modules() if isinstance(m, gpcompat.DeepGPLayer)]:
         old = layer.covar_module
         bs = old.batch_shape
-        new = gpcompat.ScaleKernel(gpcompat.MaternKernel(nu=nu, ard_num_dims=old.base_kernel.ard_num_dims,
-                                                         batch_shape=bs), batch_shape=bs)
-        new.load_state_dict(old.state_dict())        # same raw lengthscale / outputscale values
+        ard = old.base_kernel.ard_num_dims
+        base = (gpcompat.RQKernel(ard_num_dims=ard, batch_shape=bs) if nu == "rq"
+                else gpcompat.MaternKernel(nu=nu, ard_num_dims=ard, batch_shape=bs))
+        new = gpcompat.ScaleKernel(base, batch_shape=bs)
+        # same raw lengthscale / outputscale values (RQ keeps its own raw_alpha)
+        missing, unexpected = new.load_state_dict(old.state_dict(), strict=False)
+        assert not unexpected and all(k.startswith("base_kernel.raw_alpha") for k in missing), (missing, unexpected)
         layer.covar_module = new.to(old.raw_outputscale.device)
 
 
